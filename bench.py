@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the mAR-SCF flow-step hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl flowk|reference] [--workload cfg2]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl flowk|reference] [--workload cfg2] [--dump-outputs DIR]
 
 One "step" = one forward pass (z, log-det, bits/dim) of the whole flow stack over one batch of
 synthetic images.  Default workload: cfg2 = CIFAR10-shape 3x32x32, MixLogCDF coupling, L=3 K=4 C=96,
@@ -16,6 +16,10 @@ batch 64 per GPU (BASELINE.json configs[1]).  Prints ONE JSON line on rank 0.
              timed on this box's host cores on a bounded sample of the same workload
   --impl reference   the same oracle as the reference arm (the reference is Python and cannot travel
              to the GPU box; see DESIGN.md)
+  --dump-outputs DIR   after the timed steps of `value`, rank 0 writes what the last of them returned (latent z,
+             per-image bits/dim) as float32 .npy files.  Weights and images come from fixed seeds; the
+             dequantisation noise is drawn inside the CUDA graph from the seeded device generator, so it repeats
+             for the same --warmup, --steps and --depth.  The same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -365,6 +369,9 @@ def run_flowk(args):
         return ms, sampler.summary()
 
     ms_res, clocks = timed(resident_step)
+    if args.dump_outputs and rank == 0:             # before the e2e and latency legs replay the same graphs
+        last = graphed.lanes[(graphed.i - 1) % args.depth] if args.depth > 1 else graphed
+        dump_outputs(args.dump_outputs, {"z": last.static_z, "bits_per_dim": last.static_nll})
     ms_e2e, _ = timed(e2e_step)
     ms_lat, _ = timed(latency_step)
     images = batch * world * args.steps
@@ -546,6 +553,15 @@ def run_flowk(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as `<out_dir>/<name>.npy` in float32, so that two builds can be compared output for output."""
+    host = {name: t.detach().float().cpu().numpy() for name, t in arrays.items()}
+    assert sum(a.nbytes for a in host.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def time_conv_gemm_isolated(device, gb, gh, gw, cin, nn, taps, f16=True, sets=10, reps=5):
     """The dominant conditioner GEMM on its own: `sets` launches on DIFFERENT operand / output buffers (together larger
     than the 126 MB L2, so no launch finds its activations cached) captured in one CUDA graph - back-to-back launches on
@@ -674,13 +690,12 @@ def other_configs_leg(args, device):
             fn(3)
             torch.cuda.synchronize()
             s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            steps = max(5, args.steps)
             s.record()
-            fn(steps)
+            fn(args.steps)
             e.record()
             torch.cuda.synchronize()
             ms = s.elapsed_time(e)
-            res[key] = {"value": batch * steps / (ms / 1e3), "unit": "images/s", "ms_per_step": ms / steps}
+            res[key] = {"value": batch * args.steps / (ms / 1e3), "unit": "images/s", "ms_per_step": ms / args.steps}
         res["workload"] = DESCRIBE[name]
         res["batch"] = batch
         res["batches_in_flight"] = depth
@@ -848,7 +863,13 @@ def main():
     ap.add_argument("--no-inverse", action="store_true")
     ap.add_argument("--no-mar", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the latent z and the per-image bits/dim of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "flowk":
+        ap.error("--dump-outputs writes the outputs of the flowk arm")
     args.warmup = max(args.warmup, 3) if args.impl == "flowk" else args.warmup
     if args.impl == "reference":
         run_reference(args)

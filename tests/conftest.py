@@ -1,5 +1,7 @@
 """pytest plumbing: `gpu` marker, repo root on sys.path, golden-fixture loader."""
+import hashlib
 import json
+import math
 import os
 import sys
 
@@ -26,8 +28,25 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip)
 
 
+def rebuild_weight(shape, init_state, perturb_state, std):
+    """A golden weight stored as its recipe instead of its values: nn.Conv2d's default init (kaiming_uniform_, a=sqrt(5))
+    drawn from the CPU generator state `init_state`, plus make_golden.perturb()'s N(0, std^2) step drawn from
+    `perturb_state`.  This replays the draws that made the weight the reference ran with, bit for bit."""
+    gen = torch.Generator()
+    gen.set_state(init_state)
+    w = torch.empty(shape)
+    torch.nn.init.kaiming_uniform_(w, a=math.sqrt(5), generator=gen)
+    gen.set_state(perturb_state)
+    return w.add_(torch.randn(shape, generator=gen) * std)
+
+
+def sha256(t):
+    return hashlib.sha256(t.contiguous().numpy().tobytes()).hexdigest()
+
+
 class Golden(dict):
-    """arrays as torch tensors; `.meta` dict; `.sd` = state-dict sub-mapping ('sd/' keys)."""
+    """arrays as torch tensors; `.meta` dict; `.sd` = state-dict sub-mapping ('sd/' keys, plus the weights listed in
+    meta['rebuilt'], which are stored as 'rng_init/' and 'rng_perturb/' generator states and rebuilt here)."""
 
     def __init__(self, name):
         super().__init__()
@@ -35,13 +54,18 @@ class Golden(dict):
             self.meta = json.loads(bytes(f["meta"]).decode())
             self.sd = {}
             for k in f.files:
-                if k == "meta":
+                if k == "meta" or k.startswith("rng_"):
                     continue
                 t = torch.from_numpy(np.array(f[k]))
                 if k.startswith("sd/"):
                     self.sd[k[3:]] = t
                 else:
                     self[k] = t
+            for k, r in self.meta.get("rebuilt", {}).items():
+                w = rebuild_weight(r["shape"], torch.from_numpy(f["rng_init/" + k]), torch.from_numpy(f["rng_perturb/" + k]),
+                                   r["std"])
+                assert sha256(w) == r["sha256"], "%s: %s does not rebuild bit-exactly with this torch" % (name, k)
+                self.sd[k] = w
 
 
 @pytest.fixture

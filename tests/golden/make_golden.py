@@ -40,6 +40,10 @@ import flow_modules.log_dist as logistic  # noqa: E402
 
 torch.Tensor.cuda = lambda self, *a, **k: self      # see module docstring
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.dirname(HERE))
+from conftest import rebuild_weight, sha256  # noqa: E402
+
+RECIPE_MIN = 1 << 16      # weights with more elements are stored as generator states (keeps every fixture under 1 MB)
 
 
 def save(name, meta, **arrays):
@@ -54,10 +58,13 @@ def sd_arrays(module, prefix="sd/"):
     return {prefix + k: v.clone() for k, v in module.state_dict().items()}
 
 
-def perturb(module, gen, std=0.05):
-    """Move every parameter off its (partly zero / identity) init so no term is trivially 0."""
+def perturb(module, gen, std=0.05, states=None):
+    """Move every parameter off its (partly zero / identity) init so no term is trivially 0.  `states`, if given,
+    collects the generator state before each parameter's draw."""
     with torch.no_grad():
         for n, p in module.named_parameters():
+            if states is not None:
+                states[n] = gen.get_state()
             p.add_(torch.randn(p.shape, generator=gen) * std)
 
 
@@ -252,7 +259,17 @@ def gen_flownet(name, coupling, image, L, K, hidden, blocks, B, seed):
     g = torch.Generator().manual_seed(seed)
     torch.manual_seed(seed)
     np.random.seed(seed)
-    model = RefModel(image, hidden, K, L, coupling, blocks)
+    init_states = {}                  # data_ptr -> global generator state right before nn.Conv2d's default weight init
+    kaiming = nn.init.kaiming_uniform_
+
+    def recording_kaiming(t, *a, **k):
+        init_states[t.data_ptr()] = torch.get_rng_state()
+        return kaiming(t, *a, **k)
+    nn.init.kaiming_uniform_ = recording_kaiming
+    try:
+        model = RefModel(image, hidden, K, L, coupling, blocks)
+    finally:
+        nn.init.kaiming_uniform_ = kaiming
     H, W, C = image
     x = torch.rand(B, C, H, W, generator=g) - 0.5
     noise = torch.rand(B, C, H, W, generator=g)
@@ -262,7 +279,8 @@ def gen_flownet(name, coupling, image, L, K, hidden, blocks, B, seed):
     model.train()
     with torch.no_grad():
         model.flow.encode(z0, ld0)                       # ActNorm data-dependent init
-    perturb(model, g, 0.02)
+    perturb_states = {}
+    perturb(model, g, 0.02, perturb_states)
     model.eval()
     with torch.no_grad():
         z, outs, logdet = model.flow.encode(z0, ld0)
@@ -276,7 +294,19 @@ def gen_flownet(name, coupling, image, L, K, hidden, blocks, B, seed):
         arrays["z2_%d" % i] = o
     meta = {"coupling": coupling, "image_hwc": list(image), "L": L, "K": K, "hidden": hidden,
             "blocks": blocks, "B": B}
-    save(name, meta, **arrays, **sd_arrays(model))
+    sd = sd_arrays(model)
+    rebuilt = {}
+    for k, v in model.state_dict().items():
+        if v.numel() < RECIPE_MIN:
+            continue
+        init, pert = init_states[v.data_ptr()], perturb_states[k]
+        assert torch.equal(rebuild_weight(list(v.shape), init, pert, 0.02), v), k
+        rebuilt[k] = {"shape": list(v.shape), "std": 0.02, "sha256": sha256(v)}
+        arrays["rng_init/" + k], arrays["rng_perturb/" + k] = init, pert
+        del sd["sd/" + k]
+    if rebuilt:
+        meta["rebuilt"] = rebuilt
+    save(name, meta, **arrays, **sd)
 
 
 def gen_mar_prior():
