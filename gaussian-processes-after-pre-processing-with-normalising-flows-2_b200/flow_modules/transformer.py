@@ -13,6 +13,12 @@ reference's arithmetic:
   * attn = sigmoid(score / scale + offset2) + offset3 gives two 2x2 matrices, M1 for patches (0, 2) and M2 for patches
     (1, 3) (`offset` added on the diagonal); the free entries of the two patches are mixed by M (forward) or by its
     closed-form inverse (reverse); logdet +-= (log|det M1| + log|det M2|) * p * (p // 2) * C.
+
+On CUDA fp32 the layer runs on flowk kernels (csrc/patch_attention.cu): inference and sampling in one fused launch, and
+training of the forward direction through `flowk::patch_attention` (a forward launch that keeps the scores, a closed-form
+backward launch and a fixed-order batch sum of the parameter gradients); G and its weight gradients stay in torch.  The
+torch-op form below serves CPU / fp64 tensors, autograd through the reverse direction, and maps too large for the
+kernels' shared memory.
 """
 import math
 
@@ -20,7 +26,14 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from .. import _lib
+from .. import _lib, ops
+
+KERNEL_TRAINING = True     # False: train the forward direction on the torch-op form (A/B measurements, tests)
+
+
+def _fits(c, h, w, copies):
+    """Shared memory of csrc/patch_attention.cu: `copies` [C, H, W] fp32 samples (padded to 4) plus G, at most 200 KB."""
+    return (copies * ((c * h * w + 3) & ~3) + c * c) * 4 <= 200 * 1024
 
 
 def _patches(x, p):
@@ -90,8 +103,19 @@ class Transformer_attn(nn.Module):
         z = input
         b, c, h, w = z.shape
         assert h == w and w % 2 == 0, "Transformer_attn expects square maps with an even side"
-        if (z.is_cuda and z.dtype == torch.float32 and (2 * c * h * w + c * c) * 4 <= 200 * 1024 and
-                not (torch.is_grad_enabled() and (z.requires_grad or any(q.requires_grad for q in self.parameters())))):
+        tracking = torch.is_grad_enabled() and (z.requires_grad or any(q.requires_grad for q in self.parameters()))
+        if (KERNEL_TRAINING and tracking and not reverse and z.is_cuda and z.dtype == torch.float32 and
+                _fits(c, h, w, 3)):
+            # training: flowk::patch_attention (forward kernel + closed-form backward kernel); G = sum_i Wq_i^T Wk_i and
+            # prm are built with autograd, so torch turns the kernel's gradient of G into the six conv-weight gradients
+            _lib.check_device(z, "Transformer_attn")
+            g = self._bilinear()[:, :, 0, 0]
+            prm = torch.cat([t.reshape(1) for t in (self.offset, self.offset2, self.offset3, self.scale)])
+            batch_ld = torch.is_tensor(logdet) and logdet.dim() == 1 and logdet.shape[0] == b
+            ld_in = logdet.float() if batch_ld else z.new_zeros(b)
+            out, ld_out, _ = ops.patch_attention(z, g, prm, ld_in, bool(permute))
+            return out, (ld_out if batch_ld else ld_out + logdet)
+        if z.is_cuda and z.dtype == torch.float32 and (2 * c * h * w + c * c) * 4 <= 200 * 1024 and not tracking:
             # inference / sampling: one fused flowk kernel (csrc/patch_attention.cu), one read + one write of the activations
             g, prm = self._kernel_operands()
             _lib.check_device(z, "Transformer_attn")

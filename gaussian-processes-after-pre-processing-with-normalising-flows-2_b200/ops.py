@@ -373,6 +373,66 @@ mixlogcdf_coupling.register_autograd(_mix_c_backward, setup_context=_mix_c_setup
 
 
 # ------------------------------------------------------------------------------------------------
+# Transformer_attn (patch attention), forward direction for training
+# ------------------------------------------------------------------------------------------------
+@torch.library.custom_op("flowk::patch_attention", mutates_args=(), device_types="cuda")
+def patch_attention(x: Tensor, g: Tensor, prm: Tensor, ldj: Tensor, permute: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """y, ldj_out = Transformer_attn(x) with G = g [C, C], prm = {offset, offset2, offset3, scale}; `scores` [B, 8] are
+    kept for the backward pass."""
+    x = _f32c(x, "patch_attention")
+    b, c, h, w = x.shape
+    y = torch.empty_like(x)
+    out = torch.empty_like(ldj)
+    scores = x.new_empty(b, 8)
+    _lib.call("flowk_patch_attention_train_fwd", x.data_ptr(), _f32c(g, "patch_attention G").data_ptr(),
+              _f32c(prm, "patch_attention prm").data_ptr(), y.data_ptr(), _f32c(ldj, "ldj").data_ptr(), out.data_ptr(),
+              scores.data_ptr(), b, c, h, w, int(permute), _stream())
+    return y, out, scores
+
+
+@patch_attention.register_fake
+def _(x, g, prm, ldj, permute):
+    return torch.empty_like(x), torch.empty_like(ldj), x.new_empty(x.shape[0], 8)
+
+
+@torch.library.custom_op("flowk::patch_attention_bwd", mutates_args=(), device_types="cuda")
+def patch_attention_bwd(x: Tensor, g: Tensor, prm: Tensor, scores: Tensor, gy: Tensor, gldj: Tensor,
+                        permute: bool) -> Tuple[Tensor, Tensor]:
+    """gx [B, C, H, W] and partials [B, C*C + 4]: per sample the gradient of G, then of offset, offset2, offset3, scale."""
+    b, c, h, w = x.shape
+    gx = torch.empty_like(x)
+    partials = x.new_empty(b, c * c + 4)
+    _lib.call("flowk_patch_attention_bwd", x.data_ptr(), g.data_ptr(), prm.data_ptr(), scores.data_ptr(),
+              _f32c(gy, "gy").data_ptr(), _f32c(gldj, "gldj").data_ptr(), gx.data_ptr(), partials.data_ptr(),
+              b, c, h, w, int(permute), _stream())
+    return gx, partials
+
+
+@patch_attention_bwd.register_fake
+def _(x, g, prm, scores, gy, gldj, permute):
+    return torch.empty_like(x), x.new_empty(x.shape[0], x.shape[1] * x.shape[1] + 4)
+
+
+def _pa_setup(ctx, inputs, output):
+    x, g, prm, ldj, permute = inputs
+    ctx.permute = permute
+    ctx.mark_non_differentiable(output[2])
+    ctx.save_for_backward(x.contiguous(), g.contiguous(), prm.contiguous(), output[2])
+
+
+def _pa_backward(ctx, gy, gldj, gscores):
+    from .tc_autograd import channel_sum
+    x, g, prm, scores = ctx.saved_tensors
+    c = x.shape[1]
+    gx, partials = patch_attention_bwd(x, g, prm, scores, gy, gldj, ctx.permute)
+    red = channel_sum(partials, False)                     # deterministic fixed-order sum over the batch
+    return gx, red[:c * c].view(c, c), red[c * c:], gldj, None
+
+
+patch_attention.register_autograd(_pa_backward, setup_context=_pa_setup)
+
+
+# ------------------------------------------------------------------------------------------------
 # log_dist functions on explicit [B,K,...] parameter tensors
 # ------------------------------------------------------------------------------------------------
 def _mixture_call(fn: str, x: Tensor, pi: Tensor, mu: Tensor, s: Tensor) -> Tensor:

@@ -372,6 +372,21 @@ int flowk_attention_f16(const float* qkv, void* out_hi, void* out_lo, int B, int
 int flowk_patch_attention(const float* x, const float* G, const float* prm, float* y, const float* ldj_in, float* ldj_out,
                           int B, int C, int H, int W, int permute, int reverse, flowk_stream_t stream);
 
+/* `Transformer_attn` training (reference flow_modules/transformer.py:123-326 and its autograd), forward direction only.
+ * flowk_patch_attention_train_fwd is flowk_patch_attention with reverse = 0 (the same y and ldj_out, bit for bit) that also
+ * writes the raw scores [B, 8] = S_0 (row-major 2x2, patches (0, 2)), S_1 (patches (1, 3)); scores must not be NULL.
+ * flowk_patch_attention_bwd takes x, G, prm and those scores with gy [B, C, H, W] and gldj [B] (the gradient of ldj_out,
+ * which is also that of ldj_in) and writes gx [B, C, H, W] and partials [B, C*C + 4]: per sample the gradient of G
+ * (row-major) and of offset, offset2, offset3, scale; their batch sums (flowk_channel_sum over rows) are the parameter
+ * gradients.  Needs (3 C H W + C^2) * 4 <= 200 KB of shared memory; FLOWK_ERR_SHAPE otherwise.  No host synchronisation
+ * and no allocation (graph-capturable); every sum has a fixed order, so repeated calls are bit-identical. */
+int flowk_patch_attention_train_fwd(const float* x, const float* G, const float* prm, float* y, const float* ldj_in,
+                                    float* ldj_out, float* scores, int B, int C, int H, int W, int permute,
+                                    flowk_stream_t stream);
+int flowk_patch_attention_bwd(const float* x, const float* G, const float* prm, const float* scores, const float* gy,
+                              const float* gldj, float* gx, float* partials, int B, int C, int H, int W, int permute,
+                              flowk_stream_t stream);
+
 /* The same attention core on tcgen05 (csrc/attention_tc.cu): S = Q K^T and O = P V as kind::f16 MMAs with TMEM accumulators,
  * fp16 (hi, lo) operand tiles built in shared memory, softmax between them; out_f16 selects fp16 or TF32-in-fp32 output
  * pairs.  Takes HW in {128, 256} with C/heads a multiple of 8 and <= 64; FLOWK_ERR_SHAPE otherwise (use flowk_attention).
