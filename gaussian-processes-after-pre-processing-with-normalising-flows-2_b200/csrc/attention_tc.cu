@@ -312,6 +312,313 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attention_tc_kernel(const AttP
   if (threadIdx.x == 0 && failed_flag && p.status) *p.status = 1;
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// One-wave variant for head dims 24 and 32 (attention_tc_v2_kernel): 256 TMEM columns and < 110 KB of shared memory, so two
+// CTAs share an SM and the 256 (image, head) CTAs of a level-1 launch at B = 64 run in ONE wave of 2 x 148 slots; each CTA's
+// staging and softmax overlap its neighbour's MMAs.  Still one CTA per (image, head), 16 warps.  Differences to the kernel
+// above:
+//   * Q and K tiles have 64-byte SWIZZLE_64B rows (32 fp16 = dk) instead of 128-byte rows that are half zeros;
+//   * keys are processed in blocks of 128: S_b = Q_t K_b^T fills ONE 128-column TMEM region, softmax gives p = 2^(s - m_b)
+//     with the block's own row maximum m_b and row sum l_b, and P_b goes back into the same columns as packed fp16
+//     (hi: columns [0, 64), lo: [64, 128)) from where O_b = P_b V_b reads it as the A operand (TS-mode MMA); no P tile in
+//     shared memory.  The epilogue combines the blocks exactly: O = sum_b O_b 2^(m_b - m) / sum_b l_b 2^(m_b - m);
+//   * O_b has dk columns: P_hi V_hi, P_lo V_hi and P_hi V_lo accumulate into the same N = dk accumulator (the three-product
+//     scheme of the conv GEMMs);
+//   * TMEM: [0, 128) S / P, then one dk-column O_b per (query tile, key block): 128 + 4 dk <= 256.
+// Within a CTA the phases are serial (S -> softmax -> P V -> next S into the same columns); the second CTA on the SM
+// fills the gaps.
+constexpr int V2_THREADS = 512;                 // 4 threads per score row (TMEM lane), 32 keys of a 128-key block each
+constexpr int V2_ROW_B = 64;                    // bytes per SWIZZLE_64B row of Q / K
+constexpr int V2_TMEM_COLS = 256;
+constexpr int V2_QTILE_B = 2 * 128 * V2_ROW_B;  // one 128-query tile of Q: hi rows, then lo rows
+
+// byte offset of the 16-byte chunk `chunk` (0..3) of row `r` inside a K-major SWIZZLE_64B tile (512-byte 8-row atoms)
+__device__ __forceinline__ uint32_t sw64_off(int r, int chunk) {
+  return (uint32_t)(r * V2_ROW_B + ((chunk ^ ((r >> 1) & 3)) << 4));
+}
+
+// kind::f16 MMA with the A operand in tensor memory (TS mode): 128 lanes = M rows, K = 16 fp16 packed in 8 columns
+__device__ __forceinline__ void umma_f16_ts_elect(uint32_t tmem_d, uint32_t tmem_a, uint64_t desc_b, uint32_t idesc,
+                                                  uint32_t accumulate, uint32_t leader) {
+  asm volatile(
+      "{\n\t.reg .pred p, q;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "setp.ne.b32 q, %5, 0;\n\t"
+      "@q tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(leader)
+      : "memory");
+}
+// 32 consecutive columns of this thread's lane, one wait
+__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
+  uint32_t r[32];
+  asm volatile(
+      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,"
+      "%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
+      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
+        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
+        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
+      : "r"(taddr));
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
+}
+// 8 packed columns into this thread's lane (no wait: the caller waits once for all its stores)
+__device__ __forceinline__ void tmem_st8u(uint32_t taddr, const uint32_t* v) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
+               ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
+               : "memory");
+}
+
+template <int KCH, int TILES>  // KCH = dk / 8 (4), TILES = seq / 128 (1 or 2)
+__global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const AttParams p) {
+  constexpr int DK = KCH * 8, tiles = TILES, HW = 128 * TILES;
+  extern __shared__ __align__(1024) uint8_t smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
+  __shared__ uint64_t bar_s, bar_o;
+  __shared__ uint32_t tmem_slot;
+  __shared__ int failed_flag;
+  __shared__ float red_max[4][128], red_sum[4][128];
+  volatile int* failed = &failed_flag;
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int pair = blockIdx.x, b = pair / p.heads, h = pair - b * p.heads;
+  const int D = p.D, C = p.C, row_stride = 3 * C;
+  const int chunks = D >> 3;                    // 16-byte chunks of real data per row
+  constexpr int hw_shift = TILES == 2 ? 8 : 7;
+
+  if (threadIdx.x == 0) {
+    failed_flag = 0;
+    mbar_init(&bar_s, 1);
+    mbar_init(&bar_o, 1);
+    fence_barrier_init();
+  }
+  if (warp == 0) tmem_alloc(&tmem_slot, (uint32_t)V2_TMEM_COLS);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = tmem_slot;
+  const bool tracing = p.trace && blockIdx.x == 0 && threadIdx.x == 0;
+  griddep_launch();
+  griddep_wait();                               // the in_proj GEMM's rows are complete from here on
+  if (tracing) p.trace[0] = clock64();
+
+  // ---- 1. stage Q (scaled, all tiles), K and V^T as fp16 (hi, lo) operand tiles ------------------------------------------
+  uint8_t* q_t = smem + p.q_off;                // [tiles][hi | lo][128 rows][64 B], SWIZZLE_64B
+  uint8_t* k_hi = smem + p.k_off;               // [HW rows][64 B], SWIZZLE_64B
+  uint8_t* k_lo = k_hi + HW * V2_ROW_B;
+  constexpr int vt_tile = 2 * DK * ROW_B;       // one 64-key block of V^T: [DK rows of hi | DK rows of lo][128 B], SWIZZLE_128B
+  uint8_t* v_t = smem + p.v_off;
+  {
+    const float* base = p.qkv + (size_t)b * HW * row_stride + h * D;
+    const int nk = HW * KCH, total = 3 * nk;
+    constexpr int MAXI = 3;                     // loads in flight per thread (the 64-register budget of two CTAs per SM)
+    for (int i0 = threadIdx.x; i0 < total; i0 += MAXI * V2_THREADS) {
+      float4 a[MAXI], c[MAXI];
+#pragma unroll
+      for (int u = 0; u < MAXI; ++u) {
+        const int i = i0 + u * V2_THREADS;
+        a[u] = c[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (i < total) {
+          int r, ch, col;
+          if (i < nk) { r = i / KCH; ch = i % KCH; col = 2 * C; }
+          else if (i < 2 * nk) { r = (i - nk) / KCH; ch = (i - nk) % KCH; col = 0; }
+          else { r = (i - 2 * nk) & (HW - 1); ch = (i - 2 * nk) >> hw_shift; col = C; }   // V: consecutive threads -> keys
+          if (ch < chunks) {
+            const float4* g = reinterpret_cast<const float4*>(base + (size_t)r * row_stride + col + ch * 8);
+            a[u] = __ldg(g);
+            c[u] = __ldg(g + 1);
+          }
+        }
+      }
+#pragma unroll
+      for (int u = 0; u < MAXI; ++u) {
+        const int i = i0 + u * V2_THREADS;
+        if (i >= total) continue;
+        if (i < 2 * nk) {                       // Q (scaled) and K: K-major rows as they lie
+          const bool isq = i < nk;
+          const int j = isq ? i : i - nk;
+          const int r = j / KCH, ch = j % KCH;
+          const float sc = isq ? p.qscale : 1.f;
+          const float v[8] = {a[u].x * sc, a[u].y * sc, a[u].z * sc, a[u].w * sc, c[u].x * sc, c[u].y * sc, c[u].z * sc, c[u].w * sc};
+          uint4 hi, lo;
+          cvt8(v, hi, lo);
+          uint8_t* dst_hi = isq ? q_t + (r >> 7) * V2_QTILE_B : k_hi;
+          uint8_t* dst_lo = isq ? dst_hi + 128 * V2_ROW_B : k_lo;
+          const int rr = isq ? (r & 127) : r;
+          *reinterpret_cast<uint4*>(dst_hi + sw64_off(rr, ch)) = hi;
+          *reinterpret_cast<uint4*>(dst_lo + sw64_off(rr, ch)) = lo;
+        } else {                                // V^T: as in attention_tc_kernel, hi and lo rows of a block kept apart
+          const int j = i - 2 * nk, key = j & (HW - 1), ch = j >> hw_shift;
+          const float v[8] = {a[u].x, a[u].y, a[u].z, a[u].w, c[u].x, c[u].y, c[u].z, c[u].w};
+          const int kb = key >> 6, kk = key & 63;
+          uint8_t* tile = v_t + (size_t)kb * vt_tile;
+#pragma unroll
+          for (int jj = 0; jj < 8; ++jj) {
+            const int dim = ch * 8 + jj;
+            unsigned short hh, ll;
+            split_f16(v[jj], hh, ll);
+            *reinterpret_cast<unsigned short*>(tile + sw_off(dim, kk >> 3) + ((kk & 7) << 1)) = hh;
+            *reinterpret_cast<unsigned short*>(tile + sw_off(DK + dim, kk >> 3) + ((kk & 7) << 1)) = ll;
+          }
+        }
+      }
+    }
+  }
+  fence_proxy_async();                          // generic-proxy smem writes -> visible to the tensor core
+  __syncthreads();
+  if (tracing) p.trace[1] = clock64();
+
+  // ---- 2. per (query tile t, key block kb): S -> softmax -> P (TMEM) -> O_{t,kb} += P V ---------------------------------
+  const uint32_t leader = warp == 0 ? elect_one() : 0u;
+  const int lane_grp = warp & 3, quarter = warp >> 2;
+  const int row = lane_grp * 32 + lane;
+  const uint32_t lane_addr = tmem_base + ((uint32_t)(lane_grp * 32) << 16);
+  auto o_col = [&](int t, int kb) { return (uint32_t)(128 + (t * tiles + kb) * DK); };
+
+  auto issue_s = [&](int t, int kb) {           // warp 0: S = Q_t K_kb^T into columns [0, 128)
+    tc_fence_after();
+    const uint32_t idesc = make_idesc_f16(128);
+    const uint64_t dq_hi = make_smem_desc_sw64(smem_u32(q_t + t * V2_QTILE_B));
+    const uint64_t dq_lo = make_smem_desc_sw64(smem_u32(q_t + t * V2_QTILE_B + 128 * V2_ROW_B));
+    const uint64_t dk_hi = make_smem_desc_sw64(smem_u32(k_hi + kb * 128 * V2_ROW_B));
+    const uint64_t dk_lo = make_smem_desc_sw64(smem_u32(k_lo + kb * 128 * V2_ROW_B));
+#pragma unroll
+    for (int ks = 0; ks < DK / 16; ++ks) {
+      const uint64_t ko = (uint64_t)(ks * 2);  // 32 bytes per K = 16 step, in 16-byte units
+      umma_elect<true>(tmem_base, dq_hi + ko, dk_hi + ko, idesc, ks == 0 ? 0u : 1u, leader);
+      umma_elect<true>(tmem_base, dq_lo + ko, dk_hi + ko, idesc, 1u, leader);
+      umma_elect<true>(tmem_base, dq_hi + ko, dk_lo + ko, idesc, 1u, leader);
+    }
+    umma_commit_elect(&bar_s, leader);
+  };
+
+  if (warp == 0) issue_s(0, 0);
+  int it = 0;                                   // blocks done: phase of bar_s / bar_o
+#pragma unroll 1
+  for (int t = 0; t < tiles; ++t) {
+    float m0 = 0.f, m1 = 0.f, l0 = 0.f, l1 = 0.f;  // per key block: row maximum and row sum
+    for (int kb = 0; kb < tiles; ++kb, ++it) {
+      // ---- 3a. this thread's 32 scores of the row (kept in registers: P overwrites them in place) and the block maximum
+      mbar_wait(&bar_s, (uint32_t)(it & 1), failed);
+      tc_fence_after();
+      if (tracing && it == 0) p.trace[2] = clock64();
+      float s[32];
+      tmem_ld32(lane_addr + (uint32_t)(quarter * 32), s);
+      float mx = s[0];
+#pragma unroll
+      for (int i = 1; i < 32; ++i) mx = fmaxf(mx, s[i]);
+      red_max[quarter][row] = mx;
+      tc_fence_before();                        // every load of S is complete before anyone writes P over it
+      __syncthreads();
+      tc_fence_after();
+      if (tracing && it == 0) p.trace[3] = clock64();
+      mx = fmaxf(fmaxf(red_max[0][row], red_max[1][row]), fmaxf(red_max[2][row], red_max[3][row]));
+      // ---- 3b. p = 2^(s - m_b) as packed fp16 (hi, lo): keys (2i, 2i + 1) of the block in column i of each half
+      float sum = 0.f;
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {    // 16 keys -> 8 columns of P_hi and 8 of P_lo
+        uint32_t ph[8], pl[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const float e0 = ex2_fast(s[16 * half + 2 * i] - mx), e1 = ex2_fast(s[16 * half + 2 * i + 1] - mx);
+          sum += e0 + e1;
+          ph[i] = pack_h2(e0, e1);
+          float a0, a1;
+          unpack_h2(ph[i], a0, a1);
+          pl[i] = pack_h2(e0 - a0, e1 - a1);
+        }
+        tmem_st8u(lane_addr + (uint32_t)(quarter * 16 + half * 8), ph);
+        tmem_st8u(lane_addr + (uint32_t)(64 + quarter * 16 + half * 8), pl);
+      }
+      red_sum[quarter][row] = sum;
+      asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+      tc_fence_before();
+      __syncthreads();
+      if (tracing && it == 0) p.trace[4] = clock64();
+      const float l = (red_sum[0][row] + red_sum[1][row]) + (red_sum[2][row] + red_sum[3][row]);
+      if (kb == 0) { m0 = mx; l0 = l; }
+      else { m1 = mx; l1 = l; }
+
+      // ---- 4. O_{t,kb} = P_hi V_hi + P_lo V_hi + P_hi V_lo (N = dk, K = 128 keys), then the next S into the freed columns
+      if (warp == 0) {
+        tc_fence_after();
+        const uint32_t idesc = make_idesc_f16(DK);
+        const uint32_t d = tmem_base + o_col(t, kb);
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {           // K = 16 keys per step: 8 packed columns of P, 32 bytes of a V^T row
+          const int key = kb * 128 + j * 16;
+          const uint8_t* vb = v_t + (size_t)(key >> 6) * vt_tile;
+          const uint64_t ko = (uint64_t)(((key & 63) >> 4) * 2);
+          const uint64_t dv_hi = make_smem_desc(smem_u32(vb)) + ko, dv_lo = make_smem_desc(smem_u32(vb + DK * ROW_B)) + ko;
+          const uint32_t a_hi = tmem_base + (uint32_t)(j * 8), a_lo = tmem_base + (uint32_t)(64 + j * 8);
+          umma_f16_ts_elect(d, a_hi, dv_hi, idesc, j == 0 ? 0u : 1u, leader);
+          umma_f16_ts_elect(d, a_lo, dv_hi, idesc, 1u, leader);
+          umma_f16_ts_elect(d, a_hi, dv_lo, idesc, 1u, leader);
+        }
+        umma_commit_elect(&bar_o, leader);
+        const int nt = kb + 1 < tiles ? t : t + 1, nkb = kb + 1 < tiles ? kb + 1 : 0;
+        if (nt < tiles) {
+          mbar_wait(&bar_o, (uint32_t)(it & 1), failed);   // P has been read
+          issue_s(nt, nkb);
+        }
+      }
+    }
+    if (tracing && t == tiles - 1) p.trace[5] = clock64();
+
+    // ---- 5. epilogue of tile t (overlaps the next tile's first S MMAs): exact combination of the key blocks
+    mbar_wait(&bar_o, (uint32_t)((it - 1) & 1), failed);
+    tc_fence_after();
+    float w0 = 1.f, w1 = 0.f;
+    if (tiles == 2) {
+      const float m = fmaxf(m0, m1);
+      w0 = ex2_fast(m0 - m);
+      w1 = ex2_fast(m1 - m);
+    }
+    const float inv = 1.0f / (l0 * w0 + l1 * w1);
+    w0 *= inv;
+    w1 *= inv;
+    const int q0 = t * 128;
+    const size_t o0 = (size_t)(b * HW + q0 + row) * C + h * D;
+    uint8_t* stage = q_t + t * V2_QTILE_B;      // Q_t is dead (every S of tile t is done): [2 (hi, lo)][128 rows][chunks] x 16 B
+    for (int ch = quarter; ch < chunks; ch += 4) {
+      float a[8], c[8];
+      tmem_ld8(lane_addr + o_col(t, 0) + ch * 8, a);
+      if (tiles == 2) tmem_ld8(lane_addr + o_col(t, 1) + ch * 8, c);
+      else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) c[i] = 0.f;
+      }
+#pragma unroll
+      for (int i = 0; i < 8; ++i) c[i] = a[i] * w0 + c[i] * w1;
+      if (p.out_f16) {
+        uint4 hi, lo;
+        cvt8(c, hi, lo);
+        *reinterpret_cast<uint4*>(stage + ((size_t)row * chunks + ch) * 16) = hi;
+        *reinterpret_cast<uint4*>(stage + ((size_t)(128 + row) * chunks + ch) * 16) = lo;
+      } else {
+#pragma unroll
+        for (int i = 0; i < 8; i += 2) store_pair(p.out_hi, p.out_lo, o0 + ch * 8 + i, c[i], c[i + 1], 0);
+      }
+    }
+    if (p.out_f16) {
+      __syncthreads();
+      const int items = 2 * 128 * chunks;
+      for (int i = threadIdx.x; i < items; i += V2_THREADS) {
+        const int mat = i / (128 * chunks), rr = (i / chunks) % 128, ch = i % chunks;
+        const uint4 v = *reinterpret_cast<const uint4*>(stage + (size_t)i * 16);
+        unsigned short* dst = reinterpret_cast<unsigned short*>(mat ? p.out_lo : p.out_hi);
+        *reinterpret_cast<uint4*>(dst + (size_t)(b * HW + q0 + rr) * C + h * D + ch * 8) = v;
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (tracing) p.trace[6] = clock64();
+  if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)V2_TMEM_COLS);
+  if (threadIdx.x == 0 && failed_flag && p.status) *p.status = 1;
+}
+
 }  // namespace tc
 }  // namespace flowk
 
@@ -369,4 +676,99 @@ extern "C" int flowk_attention_tc(const float* qkv, void* out_hi, void* out_lo, 
   }
 #undef FLOWK_LAUNCH_ATT
   return launch_status();
+}
+
+namespace {
+// Shared-memory plan of attention_tc_v2_kernel: Q (all tiles), K, V^T; the epilogue stages its output over the dead Q tile.
+bool attention_tc_v2_plan(int HW, int C, int heads, AttParams& p, size_t& smem) {
+  if (HW != 128 && HW != 256) return false;
+  if (heads < 1 || C < 1 || C % heads) return false;
+  const int D = C / heads;
+  if (D != 24 && D != 32) return false;         // dk = 32: one 64-byte swizzle row (dk = 16 would not keep 64 registers)
+  p.HW = HW;
+  p.C = C;
+  p.heads = heads;
+  p.D = D;
+  p.dk = (D + 15) / 16 * 16;
+  p.qscale = 1.4426950408889634f / sqrtf((float)D);
+  p.q_off = 0;
+  p.k_off = (HW / 128) * V2_QTILE_B;
+  p.v_off = p.k_off + 2 * HW * V2_ROW_B;
+  smem = (size_t)p.v_off + (size_t)2 * (HW / 64) * p.dk * ROW_B + 1024;    // + alignment of the 1024-byte swizzle atoms
+  return true;
+}
+
+template <int KCH, int TILES>
+cudaError_t attention_tc_v2_prepare(size_t smem) {
+  static size_t smem_set = 0;
+  if (smem > smem_set) {
+    cudaError_t e = cudaFuncSetAttribute(attention_tc_v2_kernel<KCH, TILES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(attention_tc_v2_kernel<KCH, TILES>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                             (int)cudaSharedmemCarveoutMaxShared);
+    if (e != cudaSuccess) return e;
+    smem_set = smem;
+  }
+  return cudaSuccess;
+}
+}  // namespace
+
+// One-wave kernel (two CTAs per SM) for C / heads in {24, 32}; same contract as flowk_attention_tc otherwise.
+extern "C" int flowk_attention_tc_v2(const float* qkv, void* out_hi, void* out_lo, int out_f16, int B, int HW, int C,
+                                     int heads, int* status, long long* trace, flowk_stream_t stream) {
+  AttParams p{};
+  size_t smem = 0;
+  if (B < 0 || !attention_tc_v2_plan(HW, C, heads, p, smem)) return FLOWK_ERR_SHAPE;
+  if (B == 0) return FLOWK_OK;
+  if (!qkv || !out_hi || !out_lo) return FLOWK_ERR_ARG;
+  if ((long long)B * heads > 0x7fffffffLL) return FLOWK_ERR_SHAPE;
+  p.qkv = qkv;
+  p.out_hi = reinterpret_cast<float*>(out_hi);
+  p.out_lo = reinterpret_cast<float*>(out_lo);
+  p.out_f16 = out_f16;
+  p.status = status;
+  p.trace = trace;
+#define FLOWK_LAUNCH_ATT_V2(KCH_, TILES_)                                                                             \
+  do {                                                                                                                 \
+    FLOWK_CUDA_OK((attention_tc_v2_prepare<KCH_, TILES_>(smem)));                                                       \
+    FLOWK_CUDA_OK(launch_pdl(attention_tc_v2_kernel<KCH_, TILES_>, dim3(B * heads), dim3(V2_THREADS), smem, stream, p));  \
+  } while (0)
+  if (HW == 256) FLOWK_LAUNCH_ATT_V2(4, 2);
+  else FLOWK_LAUNCH_ATT_V2(4, 1);
+#undef FLOWK_LAUNCH_ATT_V2
+  return launch_status();
+}
+
+// CTAs of flowk_attention_tc_v2's kernel that one SM's registers, shared memory and thread slots hold at this shape; writes
+// the dynamic shared memory per CTA to *smem_bytes when it is not NULL.  FLOWK_ERR_SHAPE for shapes it does not take.
+// (cudaOccupancyMaxActiveBlocksPerMultiprocessor answers 1 for every kernel that uses tcgen05 instructions, whatever its
+// resources, so the limits are applied here from the kernel's attributes and the device's.)
+namespace {
+template <int KCH, int TILES>
+int attention_tc_v2_fit(size_t smem, int* blocks_per_sm) {
+  FLOWK_CUDA_OK((attention_tc_v2_prepare<KCH, TILES>(smem)));
+  cudaFuncAttributes fa;
+  FLOWK_CUDA_OK(cudaFuncGetAttributes(&fa, attention_tc_v2_kernel<KCH, TILES>));
+  int dev = 0, regs_sm = 0, smem_sm = 0, reserved = 0, threads_sm = 0;
+  FLOWK_CUDA_OK(cudaGetDevice(&dev));
+  FLOWK_CUDA_OK(cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, dev));
+  FLOWK_CUDA_OK(cudaDeviceGetAttribute(&smem_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev));
+  FLOWK_CUDA_OK(cudaDeviceGetAttribute(&reserved, cudaDevAttrReservedSharedMemoryPerBlock, dev));
+  FLOWK_CUDA_OK(cudaDeviceGetAttribute(&threads_sm, cudaDevAttrMaxThreadsPerMultiProcessor, dev));
+  const int warp_regs = (fa.numRegs * 32 + 255) / 256 * 256;            // registers are allocated per warp, 256 at a time
+  const int by_regs = regs_sm / (warp_regs * (V2_THREADS / 32));
+  const int by_smem = smem_sm / (int)(smem + fa.sharedSizeBytes + (size_t)reserved);
+  const int by_threads = threads_sm / V2_THREADS;
+  *blocks_per_sm = by_regs < by_smem ? (by_regs < by_threads ? by_regs : by_threads) : (by_smem < by_threads ? by_smem : by_threads);
+  return FLOWK_OK;
+}
+}  // namespace
+
+extern "C" int flowk_attention_tc_v2_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes) {
+  AttParams p{};
+  size_t smem = 0;
+  if (!attention_tc_v2_plan(HW, C, heads, p, smem)) return FLOWK_ERR_SHAPE;
+  if (!blocks_per_sm) return FLOWK_ERR_ARG;
+  if (smem_bytes) *smem_bytes = (int)smem;
+  return HW == 256 ? attention_tc_v2_fit<4, 2>(smem, blocks_per_sm) : attention_tc_v2_fit<4, 1>(smem, blocks_per_sm);
 }

@@ -130,10 +130,28 @@ def attention_tc_supported(HW, C, heads):
     return smem <= 227 * 1024
 
 
+# The one-wave tcgen05 kernel (two CTAs per SM) for the shapes it takes; FLOWK_ATTENTION_TC_V2=0 keeps them on the
+# one-CTA-per-SM kernel (A/B runs).
+ATTENTION_TC_V2 = __import__("os").environ.get("FLOWK_ATTENTION_TC_V2", "1") != "0"
+
+
+def attention_tc_v2_supported(HW, C, heads):
+    """Shapes the one-wave tcgen05 attention kernel (csrc/attention_tc.cu, attention_tc_v2_kernel) takes: seq 128 / 256 with
+    head dim 24 or 32 (one 64-byte swizzle row per Q / K row).  Other head dims (cfg4's 40 needs 96-byte rows, which
+    would not fit two CTAs per SM) stay on attention_tc_kernel."""
+    if not (ATTENTION_TC and ATTENTION_TC_V2 and heads >= 1 and C % heads == 0):
+        return False
+    return HW in (128, 256) and C // heads in (24, 32)
+
+
 def attention(qkv, B, HW, C, heads, f16=False, status=None, trace=None):
     """qkv [B*HW, 3C] (k | v | q) -> (hi, lo) [B*HW, C] of softmax(q k^T / sqrt(d)) v."""
     hi = torch.empty(B * HW, C, device=qkv.device, dtype=torch.float16 if f16 else torch.float32)
     lo = torch.empty_like(hi)
+    if attention_tc_v2_supported(HW, C, heads):
+        _lib.call("flowk_attention_tc_v2", qkv.data_ptr(), hi.data_ptr(), lo.data_ptr(), int(f16), B, HW, C, heads,
+                  _p(status), _p(trace), _stream())
+        return hi, lo
     if attention_tc_supported(HW, C, heads):
         _lib.call("flowk_attention_tc", qkv.data_ptr(), hi.data_ptr(), lo.data_ptr(), int(f16), B, HW, C, heads,
                   _p(status), _p(trace), _stream())

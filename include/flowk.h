@@ -394,6 +394,16 @@ int flowk_patch_attention_bwd(const float* x, const float* G, const float* prm, 
  * production) receives clock64 stamps of the first CTA's phases. */
 int flowk_attention_tc(const float* qkv, void* out_hi, void* out_lo, int out_f16, int B, int HW, int C, int heads,
                        int* status, long long* trace, flowk_stream_t stream);
+/* The one-wave variant (csrc/attention_tc.cu, attention_tc_v2_kernel): 256 TMEM columns and < 110 KB of shared memory per
+ * CTA, so two CTAs share an SM; keys in blocks of 128 with per-block softmax statistics combined exactly in the epilogue,
+ * P kept in tensor memory.  Same arguments, outputs and trace slots as flowk_attention_tc; takes HW in {128, 256} with
+ * C/heads in {24, 32}, FLOWK_ERR_SHAPE otherwise.
+ * flowk_attention_tc_v2_occupancy reports how many of its CTAs one SM's registers, shared memory and thread slots hold at a
+ * shape and, if smem_bytes is not NULL, the dynamic shared memory per CTA (the runtime's occupancy calculator answers 1 for
+ * any kernel that uses tcgen05 instructions). */
+int flowk_attention_tc_v2(const float* qkv, void* out_hi, void* out_lo, int out_f16, int B, int HW, int C, int heads,
+                          int* status, long long* trace, flowk_stream_t stream);
+int flowk_attention_tc_v2_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes);
 
 #ifdef __cplusplus
 }
