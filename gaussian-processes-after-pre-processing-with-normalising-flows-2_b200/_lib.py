@@ -55,6 +55,8 @@ SIGNATURES = {
     "flowk_attention_tc": ([_fp, _fp, _fp, _i, _i, _i, _i, _i, _fp, _fp, _st], _i),
     "flowk_attention_tc_v2": ([_fp, _fp, _fp, _i, _i, _i, _i, _i, _fp, _fp, _st], _i),
     "flowk_attention_tc_v2_occupancy": ([_i, _i, _i, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)], _i),
+    "flowk_attention_inproj_tc": ([_fp, _fp, _fp, _fp, _f, _fp, _fp, _i, _i, _i, _i, _fp, _fp, _st], _i),
+    "flowk_attention_inproj_tc_occupancy": ([_i, _i, _i, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)], _i),
     "flowk_attention": ([_fp, _fp, _fp, _i, _i, _i, _i, _st], _i),
     "flowk_concat_elu_fwd": ([_fp, _fp, _fp, ctypes.c_longlong, _i, ctypes.c_longlong, _st], _i),
     "flowk_concat_elu_bwd": ([_fp, _fp, _fp, _fp, ctypes.c_longlong, _i, ctypes.c_longlong, _st], _i),
@@ -121,7 +123,8 @@ DIMS = {
     "flowk_mixture_log_cdf": slice(5, 8), "flowk_mixture_log_pdf": slice(5, 8), "flowk_mixture_inv_cdf": slice(5, 8),
     "flowk_nchw_to_nhwc_hilo": slice(2, 6), "flowk_split_hilo": slice(3, 4), "flowk_attention": slice(3, 7),
     "flowk_nchw_to_nhwc_hilo_f16": slice(2, 6), "flowk_split_hilo_f16": slice(3, 4), "flowk_attention_f16": slice(3, 7),
-    "flowk_attention_tc": slice(4, 8), "flowk_attention_tc_v2": slice(4, 8), "flowk_patch_attention": slice(6, 10),
+    "flowk_attention_tc": slice(4, 8), "flowk_attention_tc_v2": slice(4, 8), "flowk_attention_inproj_tc": slice(7, 11),
+    "flowk_patch_attention": slice(6, 10),
     "flowk_patch_attention_train_fwd": slice(7, 11), "flowk_patch_attention_bwd": slice(8, 12),
     "flowk_pack_weight_f16": slice(6, 10), "flowk_fold_actnorm_invconv": slice(7, 11),
 }

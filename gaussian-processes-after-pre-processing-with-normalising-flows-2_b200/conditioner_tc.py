@@ -130,34 +130,45 @@ def mixlogcdf_nn_raw(nn_module, x_id, status=None):
         has_attn = "in_proj" in blk
         if has_attn:
             pos = nn_module.mid_convs[bi].attn._pos_enc(HW, C, dev).reshape(HW, C).contiguous()
-            qkv = buf(M, 3 * C)
-            if CHAIN and tc.chain_supported(C, 3 * C, F16):
-                # G2 + G3 in one launch: the normalised rows (+ positional encoding) go from the epilogue into swizzled
-                # shared-memory operand tiles and are multiplied by in_proj's weight in the same CTA
-                w3_hi, w3_lo, _, sc3 = blk["in_proj"]
-                tc.conv_gemm(c1_hi, c1_lo, w_hi, w_lo, B, H, W, 2 * C, 2 * C, 1, tc.PRE_GLU_RES_LN, tc.OUT_F32, bias=bias,
-                             res=x, gamma=blk["ln1"][0], beta=blk["ln1"][1], pos=pos, out_f32=x1, status=status,
-                             w2_hi=w3_hi, w2_lo=w3_lo, out2_f32=qkv, n2=3 * C, acc_scale=sc, acc_scale2=sc3)
-            else:
+            heads = blk["heads"]
+            fused = F16 and tc.attention_inproj_supported(HW, C, heads)
+            if fused:
+                # G2 writes the normalised rows (+ positional encoding) as an fp16 pair; G3 and the attention run in one
+                # launch, q, k and v never leaving the SM
                 p_hi, p_lo = obuf(M, C), obuf(M, C)
                 tc.conv_gemm(c1_hi, c1_lo, w_hi, w_lo, B, H, W, 2 * C, 2 * C, 1, tc.PRE_GLU_RES_LN,
                              tc.OUT_F32 | tc.OUT_HILO_POS, bias=bias, res=x, gamma=blk["ln1"][0], beta=blk["ln1"][1],
                              pos=pos, out_f32=x1, out_hi=p_hi, out_lo=p_lo, status=status, acc_scale=sc)
-                # G3: in_proj -> (k | v | q)
-                w_hi, w_lo, _, sc = blk["in_proj"]
-                tc.conv_gemm(p_hi, p_lo, w_hi, w_lo, B, H, W, C, 3 * C, 1, tc.PRE_BIAS, tc.OUT_F32, out_f32=qkv,
-                             status=status, acc_scale=sc)
-            heads = blk["heads"]
-            if tc.attention_supported(HW, C, heads):
-                t_hi, t_lo = tc.attention(qkv, B, HW, C, heads, F16, status=status)
-            else:                                                     # odd head sizes: library matmuls
-                _lib.library_fallback("attention core (seq %d, head dim %d)" % (HW, C // heads), qkv)
-                d = C // heads
-                t = qkv.view(B, HW, 3, heads, d)
-                k, v, q = (t[:, :, i].permute(0, 2, 1, 3) for i in range(3))
-                att = torch.softmax((q * (d ** -0.5)) @ k.transpose(-1, -2), dim=-1) @ v      # [B, heads, HW, d]
-                att = att.permute(0, 2, 1, 3).reshape(M, C).contiguous()
-                t_hi, t_lo = tc.split_rows_f16(att) if F16 else tc.split_rows(att)
+                w3_hi, w3_lo, _, sc3 = blk["in_proj"]
+                t_hi, t_lo = tc.attention_inproj(p_hi, p_lo, w3_hi, w3_lo, sc3, B, HW, C, heads, status=status)
+            else:
+                qkv = buf(M, 3 * C)
+                if CHAIN and tc.chain_supported(C, 3 * C, F16):
+                    # G2 + G3 in one launch: the normalised rows (+ positional encoding) go from the epilogue into swizzled
+                    # shared-memory operand tiles and are multiplied by in_proj's weight in the same CTA
+                    w3_hi, w3_lo, _, sc3 = blk["in_proj"]
+                    tc.conv_gemm(c1_hi, c1_lo, w_hi, w_lo, B, H, W, 2 * C, 2 * C, 1, tc.PRE_GLU_RES_LN, tc.OUT_F32, bias=bias,
+                                 res=x, gamma=blk["ln1"][0], beta=blk["ln1"][1], pos=pos, out_f32=x1, status=status,
+                                 w2_hi=w3_hi, w2_lo=w3_lo, out2_f32=qkv, n2=3 * C, acc_scale=sc, acc_scale2=sc3)
+                else:
+                    p_hi, p_lo = obuf(M, C), obuf(M, C)
+                    tc.conv_gemm(c1_hi, c1_lo, w_hi, w_lo, B, H, W, 2 * C, 2 * C, 1, tc.PRE_GLU_RES_LN,
+                                 tc.OUT_F32 | tc.OUT_HILO_POS, bias=bias, res=x, gamma=blk["ln1"][0], beta=blk["ln1"][1],
+                                 pos=pos, out_f32=x1, out_hi=p_hi, out_lo=p_lo, status=status, acc_scale=sc)
+                    # G3: in_proj -> (k | v | q)
+                    w_hi, w_lo, _, sc = blk["in_proj"]
+                    tc.conv_gemm(p_hi, p_lo, w_hi, w_lo, B, H, W, C, 3 * C, 1, tc.PRE_BIAS, tc.OUT_F32, out_f32=qkv,
+                                 status=status, acc_scale=sc)
+                if tc.attention_supported(HW, C, heads):
+                    t_hi, t_lo = tc.attention(qkv, B, HW, C, heads, F16, status=status)
+                else:                                                     # odd head sizes: library matmuls
+                    _lib.library_fallback("attention core (seq %d, head dim %d)" % (HW, C // heads), qkv)
+                    d = C // heads
+                    t = qkv.view(B, HW, 3, heads, d)
+                    k, v, q = (t[:, :, i].permute(0, 2, 1, 3) for i in range(3))
+                    att = torch.softmax((q * (d ** -0.5)) @ k.transpose(-1, -2), dim=-1) @ v      # [B, heads, HW, d]
+                    att = att.permute(0, 2, 1, 3).reshape(M, C).contiguous()
+                    t_hi, t_lo = tc.split_rows_f16(att) if F16 else tc.split_rows(att)
             # G4: attention gate -> GLU + x1 -> LayerNorm
             w_hi, w_lo, bias, sc = blk["attn_gate"]
             x2 = buf(M, C)

@@ -59,6 +59,8 @@ struct AttParams {
   int dk;                   // D rounded up to 16: contraction length of S and MMA N of O
   float qscale;             // log2(e) / sqrt(D)
   int q_off, k_off, v_off, p_off, o_off;   // byte offsets of the tile groups in dynamic shared memory
+  float acc_scale;          // fused in_proj (attention_tc_v2_kernel<.., true>): undoes the weights' power-of-two pre-scaling
+  int kslices;              // fused in_proj: 32-channel K slices of the projection, ceil(C / 32)
   int* status;
   long long* trace;         // optional device [8]: clock64 stamps of CTA (0,0) (profiling), NULL in production
 };
@@ -327,10 +329,24 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) attention_tc_kernel(const AttP
 //   * TMEM: [0, 128) S / P, then one dk-column O_b per (query tile, key block): 128 + 4 dk <= 256.
 // Within a CTA the phases are serial (S -> softmax -> P V -> next S into the same columns); the second CTA on the SM
 // fills the gaps.
+//
+// INPROJ = true (flowk_attention_inproj_tc) computes q, k, v in the CTA instead of reading the in_proj GEMM's fp32 rows:
+//   * the input is the gate GEMM's normalised rows + positional encoding as an fp16 (hi, lo) pair [B*HW, C], and the in_proj
+//     weight operand [3C, ceil64(C)] (k | v | q rows, pre-scaled like every fp16 weight operand, undone by acc_scale);
+//   * warp 0 streams K slices of 32 channels through two stages: the image's HW rows of P (hi, lo) and this head's three
+//     32-row groups of weight rows (k at h D, v at C + h D, q at 2C + h D; rows past D belong to the next head or are
+//     zero-filled past 3C, their output columns are never read), all SWIZZLE_64B TMA boxes;
+//   * per query tile, [k | v | q] = P W^T (N = 96, the three-product split) lands in TMEM columns [96 t, 96 t + 96);
+//   * the drain turns those columns into the Q (pre-scaled), K and V^T operand tiles the staging loop writes in the
+//     INPROJ = false kernel, over the stage buffers (every projection MMA has retired by then) and before the first S.
 constexpr int V2_THREADS = 512;                 // 4 threads per score row (TMEM lane), 32 keys of a 128-key block each
 constexpr int V2_ROW_B = 64;                    // bytes per SWIZZLE_64B row of Q / K
 constexpr int V2_TMEM_COLS = 256;
 constexpr int V2_QTILE_B = 2 * 128 * V2_ROW_B;  // one 128-query tile of Q: hi rows, then lo rows
+constexpr int PJ_N = 96;                        // projection MMA N: k, v, q groups of 32 columns
+constexpr int PJ_W_B = PJ_N * V2_ROW_B;         // one K slice of the head's weight rows (hi or lo)
+// one stage of the projection: [P_hi: HW rows | P_lo: HW rows | W_hi: 96 rows | W_lo: 96 rows] x 64 B
+__host__ __device__ constexpr int pj_stage_bytes(int HW) { return 2 * HW * V2_ROW_B + 2 * PJ_W_B; }
 
 // byte offset of the 16-byte chunk `chunk` (0..3) of row `r` inside a K-major SWIZZLE_64B tile (512-byte 8-row atoms)
 __device__ __forceinline__ uint32_t sw64_off(int r, int chunk) {
@@ -347,6 +363,12 @@ __device__ __forceinline__ void umma_f16_ts_elect(uint32_t tmem_d, uint32_t tmem
       "@q tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
       ::"r"(tmem_d), "r"(tmem_a), "l"(desc_b), "r"(idesc), "r"(accumulate), "r"(leader)
       : "memory");
+}
+// blockIdx.x, read anew at every use (the compiler may not keep values derived from it live across the kernel)
+__device__ __forceinline__ int cta_index() {
+  int r;
+  asm volatile("mov.u32 %0, %%ctaid.x;" : "=r"(r));
+  return r;
 }
 // 32 consecutive columns of this thread's lane, one wait
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float* v) {
@@ -370,12 +392,19 @@ __device__ __forceinline__ void tmem_st8u(uint32_t taddr, const uint32_t* v) {
                : "memory");
 }
 
-template <int KCH, int TILES>  // KCH = dk / 8 (4), TILES = seq / 128 (1 or 2)
-__global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const AttParams p) {
+// INPROJ: the maps of the P pair (boxes of 32 channels x HW rows) and of the in_proj weight pair (32 channels x 32 rows);
+// unused otherwise.
+template <int KCH, int TILES, bool INPROJ>  // KCH = dk / 8 (4), TILES = seq / 128 (1 or 2)
+__global__ void __launch_bounds__(V2_THREADS, 2)
+attention_tc_v2_kernel(const AttParams p, const __grid_constant__ CUtensorMap map_p_hi,
+                       const __grid_constant__ CUtensorMap map_p_lo, const __grid_constant__ CUtensorMap map_w_hi,
+                       const __grid_constant__ CUtensorMap map_w_lo) {
   constexpr int DK = KCH * 8, tiles = TILES, HW = 128 * TILES;
+  constexpr int TR = INPROJ ? 1 : 0;            // trace slot 1 is the projection's when INPROJ; the later stamps move up one
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   __shared__ uint64_t bar_s, bar_o;
+  __shared__ uint64_t bar_full[2], bar_empty[2], bar_proj;   // INPROJ: projection stages and the last projection MMA
   __shared__ uint32_t tmem_slot;
   __shared__ int failed_flag;
   __shared__ float red_max[4][128], red_sum[4][128];
@@ -391,6 +420,13 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
     failed_flag = 0;
     mbar_init(&bar_s, 1);
     mbar_init(&bar_o, 1);
+    if (INPROJ) {
+      mbar_init(&bar_full[0], 1);
+      mbar_init(&bar_full[1], 1);
+      mbar_init(&bar_empty[0], 1);
+      mbar_init(&bar_empty[1], 1);
+      mbar_init(&bar_proj, 1);
+    }
     fence_barrier_init();
   }
   if (warp == 0) tmem_alloc(&tmem_slot, (uint32_t)V2_TMEM_COLS);
@@ -399,8 +435,14 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
   const bool tracing = p.trace && blockIdx.x == 0 && threadIdx.x == 0;
+  if (INPROJ && threadIdx.x == 0) {
+    prefetch_tmap(&map_p_hi);
+    prefetch_tmap(&map_p_lo);
+    prefetch_tmap(&map_w_hi);
+    prefetch_tmap(&map_w_lo);
+  }
   griddep_launch();
-  griddep_wait();                               // the in_proj GEMM's rows are complete from here on
+  griddep_wait();                               // the producing GEMM's rows are complete from here on
   if (tracing) p.trace[0] = clock64();
 
   // ---- 1. stage Q (scaled, all tiles), K and V^T as fp16 (hi, lo) operand tiles ------------------------------------------
@@ -409,7 +451,111 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
   uint8_t* k_lo = k_hi + HW * V2_ROW_B;
   constexpr int vt_tile = 2 * DK * ROW_B;       // one 64-key block of V^T: [DK rows of hi | DK rows of lo][128 B], SWIZZLE_128B
   uint8_t* v_t = smem + p.v_off;
-  {
+  // V^T: rows = head dims, contraction (keys) along the 128-byte rows, 64 keys per block; dims [8 ch, 8 ch + 8) of `key`
+  auto store_vt = [&](int key, int ch, const float* v) {
+    const int kb = key >> 6, kk = key & 63;
+    uint8_t* tile = v_t + (size_t)kb * vt_tile;
+#pragma unroll
+    for (int jj = 0; jj < 8; ++jj) {
+      const int dim = ch * 8 + jj;
+      unsigned short hh, ll;
+      split_f16(v[jj], hh, ll);
+      *reinterpret_cast<unsigned short*>(tile + sw_off(dim, kk >> 3) + ((kk & 7) << 1)) = hh;
+      *reinterpret_cast<unsigned short*>(tile + sw_off(DK + dim, kk >> 3) + ((kk & 7) << 1)) = ll;
+    }
+  };
+  if constexpr (INPROJ) {
+    // ---- 1a. [k | v | q]_t = P_t W_h^T for both query tiles, K slices of 32 channels through two stages (warp 0) ----------
+    constexpr int STAGE_B = pj_stage_bytes(HW);
+    const int nsl = p.kslices;
+    const uint32_t leader = warp == 0 ? elect_one() : 0u;
+    auto load_slice = [&](int ks) {             // elected lane of warp 0
+      uint8_t* st = smem + (ks & 1) * STAGE_B;
+      uint64_t* bar = &bar_full[ks & 1];
+      mbar_expect_tx(bar, (uint32_t)STAGE_B);
+      tma_load_2d(st, &map_p_hi, bar, ks * 32, b * HW);
+      tma_load_2d(st + HW * V2_ROW_B, &map_p_lo, bar, ks * 32, b * HW);
+#pragma unroll
+      for (int g = 0; g < 3; ++g) {
+        tma_load_2d(st + 2 * HW * V2_ROW_B + g * 32 * V2_ROW_B, &map_w_hi, bar, ks * 32, g * C + h * D);
+        tma_load_2d(st + 2 * HW * V2_ROW_B + PJ_W_B + g * 32 * V2_ROW_B, &map_w_lo, bar, ks * 32, g * C + h * D);
+      }
+    };
+    if (warp == 0) {
+      if (leader) {
+        load_slice(0);
+        if (nsl > 1) load_slice(1);
+      }
+      const uint32_t idesc = make_idesc_f16(PJ_N);
+      for (int ks = 0; ks < nsl; ++ks) {
+        mbar_wait(&bar_full[ks & 1], (uint32_t)((ks >> 1) & 1), failed);
+        tc_fence_after();
+        const uint8_t* st = smem + (ks & 1) * STAGE_B;
+        const uint64_t dw_hi = make_smem_desc_sw64(smem_u32(st + 2 * HW * V2_ROW_B));
+        const uint64_t dw_lo = make_smem_desc_sw64(smem_u32(st + 2 * HW * V2_ROW_B + PJ_W_B));
+#pragma unroll
+        for (int t = 0; t < tiles; ++t) {
+          const uint64_t dp_hi = make_smem_desc_sw64(smem_u32(st + t * 128 * V2_ROW_B));
+          const uint64_t dp_lo = make_smem_desc_sw64(smem_u32(st + (HW + t * 128) * V2_ROW_B));
+          const uint32_t d = tmem_base + (uint32_t)(t * PJ_N);
+#pragma unroll
+          for (int k = 0; k < 2; ++k) {         // K = 16 per MMA: two per 64-byte row
+            const uint64_t ko = (uint64_t)(k * 2);
+            umma_elect<true>(d, dp_hi + ko, dw_hi + ko, idesc, (ks | k) == 0 ? 0u : 1u, leader);
+            umma_elect<true>(d, dp_lo + ko, dw_hi + ko, idesc, 1u, leader);
+            umma_elect<true>(d, dp_hi + ko, dw_lo + ko, idesc, 1u, leader);
+          }
+        }
+        umma_commit_elect(&bar_empty[ks & 1], leader);
+        if (ks >= 1 && ks + 1 < nsl) {          // the other stage held slice ks - 1: refill it once its MMAs have read it
+          mbar_wait(&bar_empty[(ks + 1) & 1], (uint32_t)(((ks - 1) >> 1) & 1), failed);
+          if (leader) load_slice(ks + 1);
+        }
+      }
+      umma_commit_elect(&bar_proj, leader);
+    }
+    mbar_wait(&bar_proj, 0, failed);            // every projection MMA has retired: the stage buffers are free
+    tc_fence_after();
+    if (tracing) p.trace[1] = clock64();
+    // ---- 1b. drain: thread (row, quarter) takes 16-byte chunk `quarter` of the row's k, v and q; dims >= D are zero
+    const int lane_grp = warp & 3, ch = warp >> 2;
+    const int row = lane_grp * 32 + lane;
+    const uint32_t lane_addr = tmem_base + ((uint32_t)(lane_grp * 32) << 16);
+    const float sc = p.acc_scale;
+#pragma unroll 1
+    for (int t = 0; t < tiles; ++t) {
+      const uint32_t col = lane_addr + (uint32_t)(t * PJ_N + ch * 8);
+      const int key = t * 128 + row;
+      float v[8];
+      uint4 hi, lo;
+      if (ch < chunks) {
+        tmem_ld8(col, v);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] *= sc;
+      } else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] = 0.f;
+      }
+      cvt8(v, hi, lo);
+      *reinterpret_cast<uint4*>(k_hi + sw64_off(key, ch)) = hi;
+      *reinterpret_cast<uint4*>(k_lo + sw64_off(key, ch)) = lo;
+      if (ch < chunks) {
+        tmem_ld8(col + 64, v);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] = v[i] * sc * p.qscale;
+      }
+      cvt8(v, hi, lo);
+      *reinterpret_cast<uint4*>(q_t + t * V2_QTILE_B + sw64_off(row, ch)) = hi;
+      *reinterpret_cast<uint4*>(q_t + t * V2_QTILE_B + 128 * V2_ROW_B + sw64_off(row, ch)) = lo;
+      if (ch < chunks) {
+        tmem_ld8(col + 32, v);
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] *= sc;
+      }
+      store_vt(key, ch, v);
+    }
+    tc_fence_before();                          // the drain's loads are complete before S overwrites those columns
+  } else {
     const float* base = p.qkv + (size_t)b * HW * row_stride + h * D;
     const int nk = HW * KCH, total = 3 * nk;
     constexpr int MAXI = 3;                     // loads in flight per thread (the 64-register budget of two CTAs per SM)
@@ -451,23 +597,14 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
         } else {                                // V^T: as in attention_tc_kernel, hi and lo rows of a block kept apart
           const int j = i - 2 * nk, key = j & (HW - 1), ch = j >> hw_shift;
           const float v[8] = {a[u].x, a[u].y, a[u].z, a[u].w, c[u].x, c[u].y, c[u].z, c[u].w};
-          const int kb = key >> 6, kk = key & 63;
-          uint8_t* tile = v_t + (size_t)kb * vt_tile;
-#pragma unroll
-          for (int jj = 0; jj < 8; ++jj) {
-            const int dim = ch * 8 + jj;
-            unsigned short hh, ll;
-            split_f16(v[jj], hh, ll);
-            *reinterpret_cast<unsigned short*>(tile + sw_off(dim, kk >> 3) + ((kk & 7) << 1)) = hh;
-            *reinterpret_cast<unsigned short*>(tile + sw_off(DK + dim, kk >> 3) + ((kk & 7) << 1)) = ll;
-          }
+          store_vt(key, ch, v);
         }
       }
     }
   }
   fence_proxy_async();                          // generic-proxy smem writes -> visible to the tensor core
   __syncthreads();
-  if (tracing) p.trace[1] = clock64();
+  if (tracing) p.trace[TR + 1] = clock64();
 
   // ---- 2. per (query tile t, key block kb): S -> softmax -> P (TMEM) -> O_{t,kb} += P V ---------------------------------
   const uint32_t leader = warp == 0 ? elect_one() : 0u;
@@ -502,7 +639,7 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
       // ---- 3a. this thread's 32 scores of the row (kept in registers: P overwrites them in place) and the block maximum
       mbar_wait(&bar_s, (uint32_t)(it & 1), failed);
       tc_fence_after();
-      if (tracing && it == 0) p.trace[2] = clock64();
+      if (tracing && it == 0) p.trace[TR + 2] = clock64();
       float s[32];
       tmem_ld32(lane_addr + (uint32_t)(quarter * 32), s);
       float mx = s[0];
@@ -512,7 +649,7 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
       tc_fence_before();                        // every load of S is complete before anyone writes P over it
       __syncthreads();
       tc_fence_after();
-      if (tracing && it == 0) p.trace[3] = clock64();
+      if (tracing && it == 0) p.trace[TR + 3] = clock64();
       mx = fmaxf(fmaxf(red_max[0][row], red_max[1][row]), fmaxf(red_max[2][row], red_max[3][row]));
       // ---- 3b. p = 2^(s - m_b) as packed fp16 (hi, lo): keys (2i, 2i + 1) of the block in column i of each half
       float sum = 0.f;
@@ -535,7 +672,7 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
       asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
       tc_fence_before();
       __syncthreads();
-      if (tracing && it == 0) p.trace[4] = clock64();
+      if (tracing && it == 0) p.trace[TR + 4] = clock64();
       const float l = (red_sum[0][row] + red_sum[1][row]) + (red_sum[2][row] + red_sum[3][row]);
       if (kb == 0) { m0 = mx; l0 = l; }
       else { m1 = mx; l1 = l; }
@@ -564,7 +701,7 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
         }
       }
     }
-    if (tracing && t == tiles - 1) p.trace[5] = clock64();
+    if (tracing && t == tiles - 1) p.trace[TR + 5] = clock64();
 
     // ---- 5. epilogue of tile t (overlaps the next tile's first S MMAs): exact combination of the key blocks
     mbar_wait(&bar_o, (uint32_t)((it - 1) & 1), failed);
@@ -579,7 +716,10 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
     w0 *= inv;
     w1 *= inv;
     const int q0 = t * 128;
-    const size_t o0 = (size_t)(b * HW + q0 + row) * C + h * D;
+    // the output offset of this (image, head) from a fresh read of the CTA index: keeping the image index in a register
+    // from the prologue to here costs the fused in_proj variant a spill under its 64-register budget
+    const size_t out0 = (size_t)(cta_index() / p.heads) * HW * C + (size_t)(cta_index() % p.heads) * D;
+    const size_t o0 = out0 + (size_t)(q0 + row) * C;
     uint8_t* stage = q_t + t * V2_QTILE_B;      // Q_t is dead (every S of tile t is done): [2 (hi, lo)][128 rows][chunks] x 16 B
     for (int ch = quarter; ch < chunks; ch += 4) {
       float a[8], c[8];
@@ -608,13 +748,13 @@ __global__ void __launch_bounds__(V2_THREADS, 2) attention_tc_v2_kernel(const At
         const int mat = i / (128 * chunks), rr = (i / chunks) % 128, ch = i % chunks;
         const uint4 v = *reinterpret_cast<const uint4*>(stage + (size_t)i * 16);
         unsigned short* dst = reinterpret_cast<unsigned short*>(mat ? p.out_lo : p.out_hi);
-        *reinterpret_cast<uint4*>(dst + (size_t)(b * HW + q0 + rr) * C + h * D + ch * 8) = v;
+        *reinterpret_cast<uint4*>(dst + out0 + (size_t)(q0 + rr) * C + ch * 8) = v;
       }
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (tracing) p.trace[6] = clock64();
+  if (tracing) p.trace[TR + 6] = clock64();
   if (warp == 0) tmem_dealloc(tmem_base, (uint32_t)V2_TMEM_COLS);
   if (threadIdx.x == 0 && failed_flag && p.status) *p.status = 1;
 }
@@ -680,7 +820,8 @@ extern "C" int flowk_attention_tc(const float* qkv, void* out_hi, void* out_lo, 
 
 namespace {
 // Shared-memory plan of attention_tc_v2_kernel: Q (all tiles), K, V^T; the epilogue stages its output over the dead Q tile.
-bool attention_tc_v2_plan(int HW, int C, int heads, AttParams& p, size_t& smem) {
+// With the fused in_proj, the two projection stages lie over the same region first.
+bool attention_tc_v2_plan(int HW, int C, int heads, bool inproj, AttParams& p, size_t& smem) {
   if (HW != 128 && HW != 256) return false;
   if (heads < 1 || C < 1 || C % heads) return false;
   const int D = C / heads;
@@ -694,22 +835,52 @@ bool attention_tc_v2_plan(int HW, int C, int heads, AttParams& p, size_t& smem) 
   p.q_off = 0;
   p.k_off = (HW / 128) * V2_QTILE_B;
   p.v_off = p.k_off + 2 * HW * V2_ROW_B;
-  smem = (size_t)p.v_off + (size_t)2 * (HW / 64) * p.dk * ROW_B + 1024;    // + alignment of the 1024-byte swizzle atoms
+  p.kslices = (C + 31) / 32;
+  size_t bytes = (size_t)p.v_off + (size_t)2 * (HW / 64) * p.dk * ROW_B;
+  if (inproj && (size_t)2 * pj_stage_bytes(HW) > bytes) bytes = (size_t)2 * pj_stage_bytes(HW);
+  smem = bytes + 1024;                          // + alignment of the 1024-byte swizzle atoms
   return true;
 }
 
-template <int KCH, int TILES>
+template <int KCH, int TILES, bool INPROJ>
 cudaError_t attention_tc_v2_prepare(size_t smem) {
   static size_t smem_set = 0;
   if (smem > smem_set) {
-    cudaError_t e = cudaFuncSetAttribute(attention_tc_v2_kernel<KCH, TILES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(attention_tc_v2_kernel<KCH, TILES, INPROJ>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(attention_tc_v2_kernel<KCH, TILES>, cudaFuncAttributePreferredSharedMemoryCarveout,
+    e = cudaFuncSetAttribute(attention_tc_v2_kernel<KCH, TILES, INPROJ>, cudaFuncAttributePreferredSharedMemoryCarveout,
                              (int)cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return e;
     smem_set = smem;
   }
   return cudaSuccess;
+}
+
+template <bool INPROJ>
+int attention_tc_v2_launch(const AttParams& p, int B, size_t smem, const CUtensorMap* maps, cudaStream_t stream) {
+#define FLOWK_LAUNCH_ATT_V2(KCH_, TILES_)                                                                             \
+  do {                                                                                                                 \
+    FLOWK_CUDA_OK((attention_tc_v2_prepare<KCH_, TILES_, INPROJ>(smem)));                                               \
+    FLOWK_CUDA_OK(launch_pdl(attention_tc_v2_kernel<KCH_, TILES_, INPROJ>, dim3(B * p.heads), dim3(V2_THREADS), smem,    \
+                             stream, p, maps[0], maps[1], maps[2], maps[3]));                                          \
+  } while (0)
+  if (p.HW == 256) FLOWK_LAUNCH_ATT_V2(4, 2);
+  else FLOWK_LAUNCH_ATT_V2(4, 1);
+#undef FLOWK_LAUNCH_ATT_V2
+  return launch_status();
+}
+
+// K-major fp16 matrix [rows, cols] -> 2-D map with boxes of 32 columns (one 64-byte swizzle row) x box_rows rows
+bool make_map_sw64(CUtensorMap* map, const void* base, long long rows, long long cols, int box_rows) {
+  if (!encode_fn()) return false;
+  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
+  cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
+  cuuint32_t box[2] = {32u, (cuuint32_t)box_rows};
+  cuuint32_t estr[2] = {1, 1};
+  return encode_fn()(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 }  // namespace
 
@@ -718,7 +889,7 @@ extern "C" int flowk_attention_tc_v2(const float* qkv, void* out_hi, void* out_l
                                      int heads, int* status, long long* trace, flowk_stream_t stream) {
   AttParams p{};
   size_t smem = 0;
-  if (B < 0 || !attention_tc_v2_plan(HW, C, heads, p, smem)) return FLOWK_ERR_SHAPE;
+  if (B < 0 || !attention_tc_v2_plan(HW, C, heads, false, p, smem)) return FLOWK_ERR_SHAPE;
   if (B == 0) return FLOWK_OK;
   if (!qkv || !out_hi || !out_lo) return FLOWK_ERR_ARG;
   if ((long long)B * heads > 0x7fffffffLL) return FLOWK_ERR_SHAPE;
@@ -728,27 +899,46 @@ extern "C" int flowk_attention_tc_v2(const float* qkv, void* out_hi, void* out_l
   p.out_f16 = out_f16;
   p.status = status;
   p.trace = trace;
-#define FLOWK_LAUNCH_ATT_V2(KCH_, TILES_)                                                                             \
-  do {                                                                                                                 \
-    FLOWK_CUDA_OK((attention_tc_v2_prepare<KCH_, TILES_>(smem)));                                                       \
-    FLOWK_CUDA_OK(launch_pdl(attention_tc_v2_kernel<KCH_, TILES_>, dim3(B * heads), dim3(V2_THREADS), smem, stream, p));  \
-  } while (0)
-  if (HW == 256) FLOWK_LAUNCH_ATT_V2(4, 2);
-  else FLOWK_LAUNCH_ATT_V2(4, 1);
-#undef FLOWK_LAUNCH_ATT_V2
-  return launch_status();
+  const CUtensorMap unused[4] = {};
+  return attention_tc_v2_launch<false>(p, B, smem, unused, stream);
 }
 
-// CTAs of flowk_attention_tc_v2's kernel that one SM's registers, shared memory and thread slots hold at this shape; writes
-// the dynamic shared memory per CTA to *smem_bytes when it is not NULL.  FLOWK_ERR_SHAPE for shapes it does not take.
-// (cudaOccupancyMaxActiveBlocksPerMultiprocessor answers 1 for every kernel that uses tcgen05 instructions, whatever its
-// resources, so the limits are applied here from the kernel's attributes and the device's.)
+// The one-wave kernel with the in_proj GEMM fused in front (attention_tc_v2_kernel<.., true>): p_hi / p_lo [B*HW, C] fp16
+// normalised rows + positional encoding, w_hi / w_lo the in_proj weight operand [3C, ceil64(C)] fp16 (k | v | q rows).
+extern "C" int flowk_attention_inproj_tc(const void* p_hi, const void* p_lo, const void* w_hi, const void* w_lo,
+                                         float acc_scale, void* out_hi, void* out_lo, int B, int HW, int C, int heads,
+                                         int* status, long long* trace, flowk_stream_t stream) {
+  AttParams p{};
+  size_t smem = 0;
+  if (B < 0 || !attention_tc_v2_plan(HW, C, heads, true, p, smem)) return FLOWK_ERR_SHAPE;
+  if (B == 0) return FLOWK_OK;
+  if (!p_hi || !p_lo || !w_hi || !w_lo || !out_hi || !out_lo || !(acc_scale > 0.f)) return FLOWK_ERR_ARG;
+  if (!aligned16(p_hi) || !aligned16(p_lo) || !aligned16(w_hi) || !aligned16(w_lo)) return FLOWK_ERR_ALIGN;
+  if ((long long)B * HW > 0x7fffffffLL) return FLOWK_ERR_SHAPE;
+  p.out_hi = reinterpret_cast<float*>(out_hi);
+  p.out_lo = reinterpret_cast<float*>(out_lo);
+  p.out_f16 = 1;
+  p.acc_scale = acc_scale;
+  p.status = status;
+  p.trace = trace;
+  const long long rows = (long long)B * HW, kw = (C + 63) / 64 * 64;
+  CUtensorMap maps[4];
+  if (!make_map_sw64(&maps[0], p_hi, rows, C, HW) || !make_map_sw64(&maps[1], p_lo, rows, C, HW) ||
+      !make_map_sw64(&maps[2], w_hi, 3LL * C, kw, 32) || !make_map_sw64(&maps[3], w_lo, 3LL * C, kw, 32))
+    return FLOWK_ERR_ARG;
+  return attention_tc_v2_launch<true>(p, B, smem, maps, stream);
+}
+
+// CTAs of flowk_attention_tc_v2's (or flowk_attention_inproj_tc's) kernel that one SM's registers, shared memory and thread
+// slots hold at this shape; writes the dynamic shared memory per CTA to *smem_bytes when it is not NULL.  FLOWK_ERR_SHAPE
+// for shapes it does not take.  (cudaOccupancyMaxActiveBlocksPerMultiprocessor answers 1 for every kernel that uses tcgen05
+// instructions, whatever its resources, so the limits are applied here from the kernel's attributes and the device's.)
 namespace {
-template <int KCH, int TILES>
+template <int KCH, int TILES, bool INPROJ>
 int attention_tc_v2_fit(size_t smem, int* blocks_per_sm) {
-  FLOWK_CUDA_OK((attention_tc_v2_prepare<KCH, TILES>(smem)));
+  FLOWK_CUDA_OK((attention_tc_v2_prepare<KCH, TILES, INPROJ>(smem)));
   cudaFuncAttributes fa;
-  FLOWK_CUDA_OK(cudaFuncGetAttributes(&fa, attention_tc_v2_kernel<KCH, TILES>));
+  FLOWK_CUDA_OK(cudaFuncGetAttributes(&fa, attention_tc_v2_kernel<KCH, TILES, INPROJ>));
   int dev = 0, regs_sm = 0, smem_sm = 0, reserved = 0, threads_sm = 0;
   FLOWK_CUDA_OK(cudaGetDevice(&dev));
   FLOWK_CUDA_OK(cudaDeviceGetAttribute(&regs_sm, cudaDevAttrMaxRegistersPerMultiprocessor, dev));
@@ -762,13 +952,22 @@ int attention_tc_v2_fit(size_t smem, int* blocks_per_sm) {
   *blocks_per_sm = by_regs < by_smem ? (by_regs < by_threads ? by_regs : by_threads) : (by_smem < by_threads ? by_smem : by_threads);
   return FLOWK_OK;
 }
+
+template <bool INPROJ>
+int attention_tc_v2_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes) {
+  AttParams p{};
+  size_t smem = 0;
+  if (!attention_tc_v2_plan(HW, C, heads, INPROJ, p, smem)) return FLOWK_ERR_SHAPE;
+  if (!blocks_per_sm) return FLOWK_ERR_ARG;
+  if (smem_bytes) *smem_bytes = (int)smem;
+  return HW == 256 ? attention_tc_v2_fit<4, 2, INPROJ>(smem, blocks_per_sm) : attention_tc_v2_fit<4, 1, INPROJ>(smem, blocks_per_sm);
+}
 }  // namespace
 
 extern "C" int flowk_attention_tc_v2_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes) {
-  AttParams p{};
-  size_t smem = 0;
-  if (!attention_tc_v2_plan(HW, C, heads, p, smem)) return FLOWK_ERR_SHAPE;
-  if (!blocks_per_sm) return FLOWK_ERR_ARG;
-  if (smem_bytes) *smem_bytes = (int)smem;
-  return HW == 256 ? attention_tc_v2_fit<4, 2>(smem, blocks_per_sm) : attention_tc_v2_fit<4, 1>(smem, blocks_per_sm);
+  return attention_tc_v2_occupancy<false>(HW, C, heads, blocks_per_sm, smem_bytes);
+}
+
+extern "C" int flowk_attention_inproj_tc_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes) {
+  return attention_tc_v2_occupancy<true>(HW, C, heads, blocks_per_sm, smem_bytes);
 }

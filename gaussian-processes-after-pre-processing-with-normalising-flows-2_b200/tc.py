@@ -161,6 +161,33 @@ def attention(qkv, B, HW, C, heads, f16=False, status=None, trace=None):
     return hi, lo
 
 
+# q, k, v computed inside the one-wave kernel from the gate GEMM's normalised rows (flowk_attention_inproj_tc) instead of
+# a chained in_proj GEMM writing them as fp32 rows; FLOWK_ATTENTION_INPROJ=0 keeps the in_proj GEMM (A/B runs).
+ATTENTION_INPROJ = __import__("os").environ.get("FLOWK_ATTENTION_INPROJ", "1") != "0"
+
+
+def attention_inproj_supported(HW, C, heads):
+    """Shapes the fused in_proj + attention kernel takes: those of the one-wave kernel it extends."""
+    return ATTENTION_INPROJ and attention_tc_v2_supported(HW, C, heads)
+
+
+def attention_inproj(p_hi, p_lo, w_hi, w_lo, acc_scale, B, HW, C, heads, status=None, trace=None):
+    """p_hi / p_lo [B*HW, C] fp16 rows in_proj multiplies, (w_hi, w_lo, acc_scale) its fp16 weight operand [3C, ceil64(C)]
+    (conv_weight_operand_f16) -> fp16 (hi, lo) [B*HW, C] of softmax(q k^T / sqrt(d)) v with (k | v | q) = rows W^T."""
+    assert p_hi.dtype == p_lo.dtype == w_hi.dtype == w_lo.dtype == torch.float16
+    # the kernel's tensor maps are built from B, HW and C: the tensors must have exactly these layouts
+    assert p_hi.shape == p_lo.shape == (B * HW, C) and p_hi.is_contiguous() and p_lo.is_contiguous(), \
+        "p_hi / p_lo must be contiguous [B*HW, C]"
+    assert w_hi.shape == w_lo.shape == (3 * C, (C + 63) // 64 * 64) and w_hi.is_contiguous() and w_lo.is_contiguous(), \
+        "w_hi / w_lo must be the contiguous in_proj operand [3C, ceil64(C)]"
+    _lib.check_device(p_hi, "attention_inproj")
+    hi = torch.empty(B * HW, C, device=p_hi.device, dtype=torch.float16)
+    lo = torch.empty_like(hi)
+    _lib.call("flowk_attention_inproj_tc", p_hi.data_ptr(), p_lo.data_ptr(), w_hi.data_ptr(), w_lo.data_ptr(),
+              float(acc_scale), hi.data_ptr(), lo.data_ptr(), B, HW, C, heads, _p(status), _p(trace), _stream())
+    return hi, lo
+
+
 def attention_supported(HW, C, heads):
     if attention_tc_supported(HW, C, heads):
         return True

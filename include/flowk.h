@@ -404,6 +404,18 @@ int flowk_attention_tc(const float* qkv, void* out_hi, void* out_lo, int out_f16
 int flowk_attention_tc_v2(const float* qkv, void* out_hi, void* out_lo, int out_f16, int B, int HW, int C, int heads,
                           int* status, long long* trace, flowk_stream_t stream);
 int flowk_attention_tc_v2_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes);
+/* The one-wave kernel with the in_proj GEMM fused in front: instead of the fp32 in_proj rows it takes the rows that GEMM
+ * would multiply, p_hi / p_lo [B*HW, C] fp16 (the normalised rows + positional encoding, as flowk_conv_gemm's
+ * OUT_HILO_POS writes them), and the in_proj weight operand w_hi / w_lo [3C, ceil64(C)] fp16 with (k | v | q) rows as
+ * flowk_pack_weight_f16 packs a 1x1 weight, whose pre-scaling acc_scale undoes.  q, k and v are computed per (image, head)
+ * on the tensor cores and never leave the SM.  Output: fp16 (hi, lo) pairs [B*HW, C].  Same shapes as flowk_attention_tc_v2
+ * (FLOWK_ERR_SHAPE otherwise); FLOWK_ERR_ALIGN unless the four inputs are 16-byte aligned.  `trace` slots: 0 start,
+ * 1 projection done, 2..7 as slots 1..6 of flowk_attention_tc.  flowk_attention_inproj_tc_occupancy: as
+ * flowk_attention_tc_v2_occupancy, for this kernel. */
+int flowk_attention_inproj_tc(const void* p_hi, const void* p_lo, const void* w_hi, const void* w_lo, float acc_scale,
+                              void* out_hi, void* out_lo, int B, int HW, int C, int heads, int* status, long long* trace,
+                              flowk_stream_t stream);
+int flowk_attention_inproj_tc_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes);
 
 #ifdef __cplusplus
 }
