@@ -82,6 +82,7 @@ SIGNATURES = {
     "flowk_attention_dropout_mask": ([_fp, ctypes.c_uint, ctypes.c_float, _i, _i, _fp, _st], _i),
     "flowk_adamax_step": ([_fp, _i, _fp, ctypes.c_float, ctypes.c_float, ctypes.c_float, _st], _i),
     "flowk_glu_bwd": ([_fp, _fp, _fp, ctypes.c_longlong, _i, ctypes.c_longlong, _st], _i),
+    "flowk_mar_step": ([ctypes.c_void_p, _st], _i),
 }
 
 
@@ -94,6 +95,15 @@ class ConvGemmArgs(ctypes.Structure):
                [(n, ctypes.c_void_p) for n in ("w2_hi", "w2_lo", "out2_f32")] + [("N2", ctypes.c_int)] + \
                [("splitk_ws", ctypes.c_void_p), ("operand_format", ctypes.c_int), ("acc_scale", ctypes.c_float),
                 ("dilation", ctypes.c_int), ("acc_scale2", ctypes.c_float), ("acc_scale_ptr", ctypes.c_void_p)]
+
+
+class MarStepArgs(ctypes.Structure):
+    """Mirror of `flowk_mar_step_args` (include/flowk.h)."""
+    _fields_ = [(n, ctypes.c_void_p) for n in ("a_hi", "a_lo", "w_hi", "w_lo", "bias", "dst0_hi", "dst0_lo", "dst1_hi",
+                                                "dst1_lo", "c", "noise", "z")] + \
+               [("z_stride", ctypes.c_longlong), ("status", ctypes.c_void_p)] + \
+               [(n, ctypes.c_int) for n in ("mode", "B", "H", "W", "Cin", "taps", "dilation", "hid", "dst0_pitch",
+                                            "dst0_col", "dst1_pitch", "dst1_col")] + [("acc_scale", ctypes.c_float)]
 
 
 class WnJob(ctypes.Structure):
@@ -109,6 +119,7 @@ class AdamaxChunk(ctypes.Structure):
 
 OPERAND_TF32, OPERAND_F16 = 0, 1
 PRE_BIAS, PRE_GLU_RES_LN, PRE_LSTM = 0, 1, 2
+MAR_EMBED, MAR_LSTM, MAR_SAMPLE = 0, 1, 2
 PACK_PLAIN, PACK_WEIGHT_NORM, PACK_EXP_GAIN = 0, 1, 2
 OUT_F32, OUT_HILO, OUT_HILO_POS, OUT_HILO_CELU, OUT_NCHW, OUT_HILO_RELU = 1, 2, 4, 8, 16, 32
 

@@ -44,6 +44,8 @@ __device__ __forceinline__ float sigmoid_fast(float x) { return __fdividef(1.f, 
 // kernel parameters (device view)
 // --------------------------------------------------------------------------------------------------
 enum { PRE_BIAS = 0, PRE_GLU_RES_LN = 1, PRE_LSTM = 2 };
+// one step of mAR ancestral sampling (flowk_mar_step): internal epilogues only, reached through that entry point
+enum { PRE_MAR_EMBED = 3, PRE_MAR_LSTM = 4, PRE_MAR_SAMPLE = 5 };
 enum { OUT_F32 = 1, OUT_HILO = 2, OUT_HILO_POS = 4, OUT_HILO_CELU = 8, OUT_NCHW = 16, OUT_HILO_RELU = 32 };
 
 struct Params {
@@ -78,6 +80,14 @@ struct Params {
                                    // out_f32 + z*M*N (no bias) and flowk's split-K reduce kernel finishes the layer
   int* status;                     // set to 1 if a barrier wait timed out
   long long* trace;                // optional [16] clock64 stamps of CTA (0,0): setup, first full, last mma, epi start, epi end
+  // PRE_MAR_*: up to two fp16-pair destinations, each with its own row pitch and first column (fp16 elements)
+  void* dst_hi[2];
+  void* dst_lo[2];
+  int dst_pitch[2], dst_col[2];
+  float* cell;                     // PRE_MAR_LSTM: c [M, hid], updated in place
+  const float* noise;              // PRE_MAR_SAMPLE: [M] standard-normal draws
+  float* z;                        // PRE_MAR_SAMPLE: z[b * z_stride + hw]
+  long long z_stride;
 };
 
 // NV: 128-column groups per lane in the LayerNorm epilogue (1: C <= 128, 2: C <= 256); PAIR: the CTA-pair (cta_group::2)
@@ -556,6 +566,74 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap map_a_hi, const __grid_cons
           *reinterpret_cast<float4*>(co + 4) = make_float4(cn[4], cn[5], cn[6], cn[7]);
           store_hilo4<F16>(p.out_hi, p.out_lo, (size_t)m * hid + j, hn);
           store_hilo4<F16>(p.out_hi, p.out_lo, (size_t)m * hid + j + 4, hn + 4);
+        }
+      }
+    } else if (PRE == PRE_MAR_EMBED || PRE == PRE_MAR_LSTM) {
+      // One thread per row; the four warps of a TMEM lane group take interleaved 8-column slices.  EMBED: y = D + bias
+      // (conv_embed).  LSTM: D holds the gates of W_ih x_t + W_hh h_{t-1} (one GEMM over the [x | h] rows), bias =
+      // b_ih + b_hh; c is updated in place (only this thread reads or writes its row).  The result (y, or h_t) goes as an
+      // fp16 pair to dst 0 and, when given, dst 1.  TMEM loads are warp-uniform; rows past M only skip their memory accesses.
+      const int m = slab_row0 + lane;
+      const bool row_ok = m < p.M;
+      const int hid = PRE == PRE_MAR_LSTM ? p.N >> 2 : p.N;
+      for (int j = sub * 8; j < hid; j += 32) {
+        __syncwarp();
+        float hn[8];
+        if (PRE == PRE_MAR_EMBED) {
+          tmem_ld8(trow + j, hn);
+#pragma unroll
+          for (int i = 0; i < 8; ++i) hn[i] = fmaf(hn[i], sc, __ldg(p.bias + j + i));
+        } else {
+          float acc[4][8];
+#pragma unroll
+          for (int gte = 0; gte < 4; ++gte) {
+            tmem_ld8(trow + gte * hid + j, acc[gte]);
+#pragma unroll
+            for (int i = 0; i < 8; ++i) acc[gte][i] = fmaf(acc[gte][i], sc, __ldg(p.bias + gte * hid + j + i));
+          }
+          if (row_ok) {
+            float* cp = p.cell + (size_t)m * hid + j;
+            const float4 c0 = *reinterpret_cast<const float4*>(cp), c1 = *reinterpret_cast<const float4*>(cp + 4);
+            const float cv[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
+            float cn[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {            // the accurate forms of the PRE_LSTM cell above
+              const float ig = 1.f / (1.f + expf(-acc[0][i])), fg = 1.f / (1.f + expf(-acc[1][i]));
+              const float gg = tanhf(acc[2][i]), og = 1.f / (1.f + expf(-acc[3][i]));
+              cn[i] = fg * cv[i] + ig * gg;
+              hn[i] = og * tanhf(cn[i]);
+            }
+            *reinterpret_cast<float4*>(cp) = make_float4(cn[0], cn[1], cn[2], cn[3]);
+            *reinterpret_cast<float4*>(cp + 4) = make_float4(cn[4], cn[5], cn[6], cn[7]);
+          }
+        }
+        if (row_ok) {
+#pragma unroll
+          for (int d = 0; d < 2; ++d) {
+            if (!p.dst_hi[d]) continue;
+            const size_t o = (size_t)m * p.dst_pitch[d] + p.dst_col[d] + j;
+            store_hilo4_f16(reinterpret_cast<float*>(p.dst_hi[d]), reinterpret_cast<float*>(p.dst_lo[d]), o, hn);
+            store_hilo4_f16(reinterpret_cast<float*>(p.dst_hi[d]), reinterpret_cast<float*>(p.dst_lo[d]), o + 4, hn + 4);
+          }
+        }
+      }
+    } else if (PRE == PRE_MAR_SAMPLE) {
+      // conv_out1 over [x | h] with weights [0 | W_out]: columns (mean, log-std) of channel t, never stored.  The sample
+      // noise * exp(logs) + mean (corr_prior.py:96-101, same operation order, accurate expf) goes to z[b, t, hw] and, as an
+      // fp16 pair, to column dst_col of dst 0 (the next step's input rows).
+      if (sub == 0) {
+        float v[8];
+        tmem_ld8(trow, v);
+        const int m = slab_row0 + lane;
+        if (m < p.M) {
+          const float mean = fmaf(v[0], sc, __ldg(p.bias)), logs = fmaf(v[1], sc, __ldg(p.bias + 1));
+          const float s = __fadd_rn(__fmul_rn(__ldg(p.noise + m), expf(logs)), mean);
+          p.z[(size_t)(m / p.HW) * p.z_stride + m % p.HW] = s;
+          unsigned short h, l;
+          split_f16(s, h, l);
+          const size_t o = (size_t)m * p.dst_pitch[0] + p.dst_col[0];
+          reinterpret_cast<unsigned short*>(p.dst_hi[0])[o] = h;
+          reinterpret_cast<unsigned short*>(p.dst_lo[0])[o] = l;
         }
       }
     } else {
@@ -1268,6 +1346,105 @@ static int conv_gemm_impl(const flowk_conv_gemm_args* a, flowk_stream_t stream, 
                              a->out_mask == OUT_F32 ? a->out_f32 : (float*)nullptr,
                              a->out_mask == OUT_NCHW ? a->out_nchw : (float*)nullptr, p.M, N, p.HW, p.ksplit));
   }
+  return launch_status();
+}
+
+// A destination (hi, lo, pitch, column) of `width` fp16 elements per row; 8-byte stores need pitch and column % 4.
+static int check_mar_dst(const void* hi, const void* lo, int pitch, int col, int width) {
+  if (!hi || !lo) return FLOWK_ERR_ARG;
+  if (pitch < 1 || col < 0 || col + width > pitch || (width > 1 && (pitch % 4 || col % 4))) return FLOWK_ERR_SHAPE;
+  return FLOWK_OK;
+}
+
+extern "C" int flowk_mar_step(const flowk_mar_step_args* a, flowk_stream_t stream) {
+  if (!a) return FLOWK_ERR_ARG;
+  const int mode = a->mode;
+  if (mode != FLOWK_MAR_EMBED && mode != FLOWK_MAR_LSTM && mode != FLOWK_MAR_SAMPLE) return FLOWK_ERR_ARG;
+  if (!a->a_hi || !a->a_lo || !a->w_hi || !a->w_lo || !a->bias) return FLOWK_ERR_ARG;
+  if (mode == FLOWK_MAR_LSTM && !a->c) return FLOWK_ERR_ARG;
+  if (mode == FLOWK_MAR_SAMPLE && (!a->noise || !a->z)) return FLOWK_ERR_ARG;
+  if (a->taps != 1 && a->taps != 9 && a->taps != 25) return FLOWK_ERR_ARG;
+  if (!(a->acc_scale > 0.f)) return FLOWK_ERR_ARG;
+  const int B = a->B, H = a->H, W = a->W, Cin = a->Cin, hid = a->hid;
+  if (B < 1 || H < 1 || W < 1 || Cin < 8 || Cin % 8) return FLOWK_ERR_SHAPE;
+  if (hid < 8 || hid % 8 || 4 * hid > 256) return FLOWK_ERR_SHAPE;
+  const int width = mode == FLOWK_MAR_SAMPLE ? 1 : hid;
+  int st = check_mar_dst(a->dst0_hi, a->dst0_lo, a->dst0_pitch, a->dst0_col, width);
+  if (st != FLOWK_OK) return st;
+  const bool dst1 = mode == FLOWK_MAR_LSTM && (a->dst1_hi || a->dst1_lo);
+  if (dst1 && (st = check_mar_dst(a->dst1_hi, a->dst1_lo, a->dst1_pitch, a->dst1_col, width)) != FLOWK_OK) return st;
+  if (mode == FLOWK_MAR_SAMPLE && a->z_stride < (long long)H * W) return FLOWK_ERR_SHAPE;
+  if (W > BLOCK_M || BLOCK_M % W) return FLOWK_ERR_SHAPE;
+  if (H * W >= BLOCK_M ? (H * W) % BLOCK_M != 0 : BLOCK_M % (H * W) != 0) return FLOWK_ERR_SHAPE;
+  if (!encode_fn()) return FLOWK_ERR_ARG;
+
+  const int N = mode == FLOWK_MAR_LSTM ? 4 * hid : mode == FLOWK_MAR_EMBED ? hid : 2;
+  constexpr int bk = 64;                                       // fp16 channels per k-block
+  Params p{};
+  p.M = B * H * W;
+  p.N = N;
+  p.HW = H * W;
+  p.W = W;
+  p.H = H;
+  p.taps = a->taps;
+  p.ksz = a->taps == 25 ? 5 : a->taps == 9 ? 3 : 1;
+  p.dil = a->dilation > 0 ? a->dilation : 1;
+  p.kblocks_per_tap = (Cin + bk - 1) / bk;
+  p.wt = W;
+  p.ht = H * W >= BLOCK_M ? BLOCK_M / W : H;
+  p.bt = H * W >= BLOCK_M ? 1 : BLOCK_M / (H * W);
+  p.n_chunk = (N + 15) / 16 * 16;                              // weight rows past N are zero-filled by TMA
+  p.n_chunks = 1;
+  p.ksplit = 1;
+  p.pre = PRE_MAR_EMBED + mode;
+  p.bias = a->bias;
+  p.acc_scale = a->acc_scale;
+  p.status = a->status;
+  p.dst_hi[0] = a->dst0_hi;
+  p.dst_lo[0] = a->dst0_lo;
+  p.dst_pitch[0] = a->dst0_pitch;
+  p.dst_col[0] = a->dst0_col;
+  if (dst1) {
+    p.dst_hi[1] = a->dst1_hi;
+    p.dst_lo[1] = a->dst1_lo;
+    p.dst_pitch[1] = a->dst1_pitch;
+    p.dst_col[1] = a->dst1_col;
+  }
+  p.cell = a->c;
+  p.noise = a->noise;
+  p.z = a->z;
+  p.z_stride = a->z_stride;
+  p.tmem_cols = p.n_chunk <= 32 ? 32 : p.n_chunk <= 64 ? 64 : p.n_chunk <= 128 ? 128 : 256;
+  const int stage_bytes = 2 * A_TILE_BYTES + 2 * p.n_chunk * ROW_BYTES;
+  int stages = (220 * 1024 - 2048) / stage_bytes;
+  if (stages > 6) stages = 6;
+  p.stages = stages;
+  p.bar_offset = stages * stage_bytes;                         // these epilogues stage nothing in shared memory
+  const size_t smem_bytes = (size_t)p.bar_offset + 1024 + 256;
+
+  alignas(64) CUtensorMap ma_hi, ma_lo, mw_hi, mw_lo;
+  const int Ktot = p.taps * p.kblocks_per_tap * bk;
+  if (!make_map_act(&ma_hi, (const float*)a->a_hi, B, H, W, Cin, p.bt, p.ht, p.wt, 2) ||
+      !make_map_act(&ma_lo, (const float*)a->a_lo, B, H, W, Cin, p.bt, p.ht, p.wt, 2) ||
+      !make_map_w(&mw_hi, (const float*)a->w_hi, N, Ktot, p.n_chunk, 2) ||
+      !make_map_w(&mw_lo, (const float*)a->w_lo, N, Ktot, p.n_chunk, 2))
+    return FLOWK_ERR_ARG;
+  const dim3 grid((p.M + BLOCK_M - 1) / BLOCK_M, 1, 1);
+#define FLOWK_LAUNCH_MAR(PRE_)                                                                                          \
+  do {                                                                                                                  \
+    static size_t smem_set = 0;                                                                                         \
+    if (smem_bytes > smem_set) {                                                                                        \
+      FLOWK_CUDA_OK(cudaFuncSetAttribute(conv_gemm_kernel<PRE_, 1, true, false>,                                        \
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));                \
+      smem_set = smem_bytes;                                                                                            \
+    }                                                                                                                   \
+    FLOWK_CUDA_OK(launch_pdl_cluster(conv_gemm_kernel<PRE_, 1, true, false>, grid, dim3(NUM_THREADS), smem_bytes,       \
+                                     stream, 1, ma_hi, ma_lo, mw_hi, mw_lo, mw_hi, mw_lo, p));                          \
+  } while (0)
+  if (mode == FLOWK_MAR_EMBED) FLOWK_LAUNCH_MAR(PRE_MAR_EMBED);
+  else if (mode == FLOWK_MAR_LSTM) FLOWK_LAUNCH_MAR(PRE_MAR_LSTM);
+  else FLOWK_LAUNCH_MAR(PRE_MAR_SAMPLE);
+#undef FLOWK_LAUNCH_MAR
   return launch_status();
 }
 

@@ -75,13 +75,26 @@ class GraphedSampler:
     the final level and for every factored-out half are drawn from N(0, eps_std^2) IN the captured graph (fresh samples
     at every replay), pushed through `FlowNet.decode_latents`, NaNs replaced by -0.5 and the result clamped to the data
     range [-0.5, 0.5].  `run(out)` replays on this instance's stream and optionally copies the images to pinned host
-    memory."""
+    memory.
 
-    def __init__(self, model, batch, image_hwc, eps_std=1.0, warmup=2):
+    With the mAR channel prior (`MarScfFlow(..., prior="mar")`) the latents depend on the decoded images' upper halves, so
+    the graph runs the interleaved decode instead (`FlowNet.decode` with this instance's prior): sample the last level, decode
+    it, and at every split sample z2 given the decoded z1.  Each level has its own `mar_prior.cuda_path.AncestralSampler`
+    (own buffers, so instances replay concurrently) whose standard-normal noise `normal_` redraws in the graph.  That
+    prior has no temperature (corr_prior.py:96-101), so eps_std != 1 raises ValueError.  `noise[level - 1]` is the
+    [nc, B*H*W] noise buffer of a level, which the caller fills when `draw_noise=False`; `latents[level]` = (z1 or None,
+    z2) of the last replay."""
+
+    def __init__(self, model, batch, image_hwc, eps_std=1.0, warmup=2, draw_noise=True):
+        from .mar_prior import ChannelPriorMultiScale
         flow = model.flow
         dev = next(model.parameters()).device
         h, w, c = image_hwc
         self.model, self.eps_std = model, float(eps_std)
+        self.mar = isinstance(flow.c_prior, ChannelPriorMultiScale)
+        if self.mar and self.eps_std != 1.0:
+            raise ValueError("the mAR channel prior has no temperature: eps_std must be 1.0, got %g" % self.eps_std)
+        self.draw_noise = draw_noise
         self.stream = torch.cuda.Stream()
         self.stream.wait_stream(torch.cuda.current_stream())
         shapes = []                                  # factored-out halves, in split order, then the final latent
@@ -91,8 +104,14 @@ class GraphedSampler:
                 c //= 2
                 shapes.append((batch, c, h, w))
         with torch.cuda.stream(self.stream), torch.no_grad():
-            self.z = torch.empty(batch, c, h, w, device=dev)
-            self.z2s = [torch.empty(s, device=dev) for s in shapes]
+            if self.mar:
+                from .mar_prior import cuda_path
+                self.samplers = [cuda_path.AncestralSampler(p, batch, dev) for p in flow.c_prior.prior_list]
+                self.noise = [s.noise for s in self.samplers]
+                self.latents = {}
+            else:
+                self.z = torch.empty(batch, c, h, w, device=dev)
+                self.z2s = [torch.empty(s, device=dev) for s in shapes]
             for _ in range(warmup):
                 self._sample(flow)
         torch.cuda.current_stream().wait_stream(self.stream)
@@ -103,10 +122,21 @@ class GraphedSampler:
             self.images = self._sample(flow)
         self.flowk_launches = _lib.LAUNCHES - before
 
+    def _mar_prior(self, z, level, reverse=True, **kw):
+        sampler = self.samplers[level - 1]
+        if self.draw_noise:
+            sampler.noise.normal_()
+        z2 = sampler.sample(z)
+        self.latents[level] = (z, z2)
+        return z2
+
     def _sample(self, flow):
-        for t in [self.z] + self.z2s:
-            t.normal_(0.0, self.eps_std)
-        x = flow.decode_latents(self.z, self.z2s)
+        if self.mar:
+            x = flow.decode(None, prior=self._mar_prior)
+        else:
+            for t in [self.z] + self.z2s:
+                t.normal_(0.0, self.eps_std)
+            x = flow.decode_latents(self.z, self.z2s)
         x = torch.where(torch.isnan(x), torch.full_like(x, -0.5), x)
         return torch.clamp(x, -0.5, 0.5)
 

@@ -4,8 +4,9 @@ embedding of the half that continues through the flow).  Plugs into `flowk.marsc
 like the reference's `c_prior(z, level, reverse=...)`.
 
 On CUDA tensors with autograd off (evaluation, sampling) the networks run on the flowk tensor-core kernels
-(`mar_prior/cuda_path.py`: every conv a tcgen05 implicit GEMM, the LSTM cell fused into the recurrent GEMM's epilogue);
-training (autograd) and CPU tensors use the torch layers below."""
+(`mar_prior/cuda_path.py`: every conv a tcgen05 implicit GEMM, the LSTM cell fused into the recurrent GEMM's epilogue;
+sampling through `AncestralSampler`, 2 + num_layers launches per channel); training (autograd) and CPU tensors use the
+torch layers below."""
 import numpy as np
 import torch
 import torch.nn as nn
@@ -58,7 +59,7 @@ class ChannelPriorUniScale(nn.Module):
         if z1_embd is not None:
             lstm_input = torch.cat([lstm_input, z1_embd], dim=2)
         if fast:
-            out, _ = cuda_path.run_sequence(self.prior_lstm, lstm_input)
+            out = cuda_path.run_sequence(self.prior_lstm, lstm_input)
         else:
             out, _ = self.prior_lstm(lstm_input, None)
         return torch.sum(self.likelihood(out[:, :, 0:1], out[:, :, 1:2], z2), dim=(1, 2, 3, 4))
@@ -67,9 +68,14 @@ class ChannelPriorUniScale(nn.Module):
         with torch.no_grad():
             fast = cuda_path.usable(self, z1 if z1 is not None else
                                     torch.empty(1, 1, self.height, self.width, device=device or next(self.parameters()).device))
+            if fast:
+                b = z1.size(0) if z1 is not None else batch_size or self.batch_size
+                sampler = cuda_path.sampler_for(self, b, z1.device if z1 is not None else device or next(self.parameters()).device)
+                # the reference's host-side draws (corr_prior.py:96-101), one per channel in its order, copied once
+                noise = torch.stack([torch.randn(b, 1, 1, self.height, self.width) for _ in range(self.nc)])
+                return sampler.sample(z1, noise)
             if z1 is not None:
-                emb = cuda_path.z1_embedding(self.z1_cond_network, z1) if fast else self.z1_cond_network(z1)
-                z1_embd = emb.unsqueeze(1)
+                z1_embd = self.z1_cond_network(z1).unsqueeze(1)
                 b, device = z1.size(0), z1.device
                 lstm_input = torch.cat([z1.new_zeros(b, 1, 1, self.height, self.width), z1_embd], dim=2)
             else:
@@ -79,10 +85,7 @@ class ChannelPriorUniScale(nn.Module):
                 lstm_input = torch.zeros(b, 1, 1, self.height, self.width, device=device)
             hidden, chans = None, []
             for _ in range(self.nc):
-                if fast:
-                    out, hidden = cuda_path.run_sequence(self.prior_lstm, lstm_input, hidden)
-                else:
-                    out, hidden = self.prior_lstm(lstm_input, None, hidden)
+                out, hidden = self.prior_lstm(lstm_input, None, hidden)
                 mean, logs = out[:, :, 0:1], out[:, :, 1:2]
                 sample = torch.randn(mean.size()).to(device) * torch.exp(logs) + mean       # corr_prior.py:96-101
                 chans.append(sample)

@@ -16,6 +16,10 @@ pairs (fp32-accurate two-term split, csrc/tc_gemm.cu):
     z1_cond_network         5 x 5 conv, ReLU (epilogue), 5 x 5 conv
 
 so one likelihood evaluation of a level is 3 + L (T + 1) launches and nothing but the T-step recurrence is sequential.
+
+Ancestral sampling (`AncestralSampler`) runs the same networks one channel at a time with `flowk_mar_step`: conv_embed,
+one launch per LSTM layer (input-to-hidden and hidden-to-hidden convolutions as ONE GEMM over the rows [x_t | h_{t-1}]),
+and conv_out1 with the Gaussian sample drawn in its epilogue - 2 + L launches per channel and no host work in between.
 """
 import torch
 
@@ -78,9 +82,8 @@ def _conv(a_hi, a_lo, prepared, images, h, w, cin, n, pre, mask, dilation=1, **k
                  **kw)
 
 
-def run_sequence(enc, x, state=None):
-    """ConvSeqEncoder.forward on the flowk kernels.  x [B, T, Cin, H, W]; `state` = per-layer [(h_hi, h_lo), c] from a
-    previous call (ancestral sampling feeds one step at a time) or None.  Returns (out [B, T, 2, H, W], state)."""
+def run_sequence(enc, x):
+    """ConvSeqEncoder.forward on the flowk kernels from a zero state: x [B, T, Cin, H, W] -> out [B, T, 2, H, W]."""
     B, T, cin, H, W = x.shape
     HW, E = H * W, enc.embed_ch
     rows, step_rows = T * B * HW, B * HW
@@ -100,27 +103,21 @@ def run_sequence(enc, x, state=None):
     a_hi, a_lo = tc.nchw_to_nhwc_hilo(x_tb, cpad, True)
     x_hi, x_lo = f16(rows, E), f16(rows, E)
     _conv(a_hi, a_lo, ops["embed"], T * B, H, W, cpad, E, tc.PRE_BIAS, tc.OUT_HILO, out_hi=x_hi, out_lo=x_lo)
-    new_state = []
     for layer, (ih, hh) in enumerate(ops["layers"]):
         gi = f32(T, step_rows, 4 * E)                                                # input-to-hidden gates, all steps
         _conv(x_hi, x_lo, ih, T * B, H, W, E, 4 * E, tc.PRE_BIAS, tc.OUT_F32, dilation=lstm.dilation, out_f32=gi)
         h_hi, h_lo = f16(T, step_rows, E), f16(T, step_rows, E)
-        if state is None:
-            hp_hi = hp_lo = torch.zeros(step_rows, E, device=dev, dtype=torch.float16)
-            c_prev = torch.zeros(step_rows, E, device=dev, dtype=torch.float32)
-        else:
-            (hp_hi, hp_lo), c_prev = state[layer]
+        hp_hi = hp_lo = torch.zeros(step_rows, E, device=dev, dtype=torch.float16)
+        c_prev = torch.zeros(step_rows, E, device=dev, dtype=torch.float32)
         for t in range(T):                                                           # the recurrence: one launch per step
             c_next = f32(step_rows, E)
             _conv(hp_hi, hp_lo, hh, B, H, W, E, 4 * E, tc.PRE_LSTM, 0, dilation=lstm.dilation, res=gi[t], gamma=c_prev,
                   out_f32=c_next, out_hi=h_hi[t], out_lo=h_lo[t])
             hp_hi, hp_lo, c_prev = h_hi[t], h_lo[t], c_next
-        new_state.append(((hp_hi, hp_lo), c_prev))
         x_hi, x_lo = h_hi.view(rows, E), h_lo.view(rows, E)
     out = f32(rows, 4)
     _conv(x_hi, x_lo, ops["out"], T * B, H, W, E, 4, tc.PRE_BIAS, tc.OUT_F32, out_f32=out)
-    out = out.view(T, B, H, W, 4)[..., :enc.out_ch].permute(1, 0, 4, 2, 3).contiguous()
-    return out, new_state
+    return out.view(T, B, H, W, 4)[..., :enc.out_ch].permute(1, 0, 4, 2, 3).contiguous()
 
 
 def z1_embedding(net, z1):
@@ -142,3 +139,101 @@ def z1_embedding(net, z1):
     out = torch.empty(B * H * W, n_out, device=dev, dtype=torch.float32)
     _conv(h_hi, h_lo, ops[1], B, H, W, mid, n_out, tc.PRE_BIAS, tc.OUT_F32, out_f32=out)
     return out.view(B, H, W, n_out).permute(0, 3, 1, 2).contiguous()
+
+
+def _sampling_operands(enc):
+    """Weights of one sampling step: conv_embed; per layer [W_ih | W_hh] (one GEMM over the [x | h] rows) with b_ih + b_hh;
+    conv_out1 as [0 | W_out], so that it reads the same rows (under fp16's 64-channel k-blocks that costs no extra MMA)."""
+    lstm = enc.lstm
+    w_out = enc.conv_out1.weight.detach()
+    ops = {"embed": _prep(enc.conv_embed.weight, enc.conv_embed.bias),
+           "out": _prep(torch.cat([torch.zeros_like(w_out), w_out], 1), enc.conv_out1.bias, pad_out=4), "layers": []}
+    for layer in range(lstm.num_layers):
+        w_ih, w_hh = getattr(lstm, "weight_ih_l%d" % layer), getattr(lstm, "weight_hh_l%d" % layer)
+        b_ih, b_hh = getattr(lstm, "bias_ih_l%d" % layer), getattr(lstm, "bias_hh_l%d" % layer)
+        ops["layers"].append(_prep(torch.cat([w_ih.detach(), w_hh.detach()], 1), b_ih.detach() + b_hh.detach()))
+    return ops
+
+
+class AncestralSampler:
+    """Ancestral sampling of one level of the channel prior (ChannelPriorUniScale.get_sample, corr_prior.py:66-101) for a
+    fixed batch size and device.  All buffers are allocated and zeroed here, once:
+
+        S      fp16 pair [B*HW, 8]            step input [previous channel's sample | z1 embedding | 0]
+        A      fp16 pairs [L][2][B*HW, 2 hid]  per layer and step parity, rows [x_t | h_{t-1}]
+        c      fp32 [L][B*HW, hid]             cell states
+        noise  fp32 [nc, B*HW]                 the standard-normal draw of every channel
+
+    Channel t (parity p = t % 2) is 2 + L flowk_mar_step launches, none of which writes a buffer it reads (the 3x3 / 5x5
+    taps read rows of other CTAs): EMBED S -> x of A_0[p]; LSTM l reads A_l[p], writes h to A_l[1-p] and to x of A_{l+1}[p];
+    SAMPLE reads A_{L-1}[1-p] and writes z[:, t] and column 0 of S.  SAMPLE multiplies the stale x half of its rows by zero
+    weights, which is why the buffers start zeroed (uninitialised fp16 can hold NaN, and 0 * NaN = NaN).  The per-channel
+    loop makes no allocation, no host synchronisation and no ATen call, so `sample` can be captured in a CUDA graph."""
+
+    def __init__(self, prior, batch, device):
+        enc = prior.prior_lstm
+        self.prior, self.enc = prior, enc
+        self.B, self.H, self.W, self.nc = batch, prior.height, prior.width, prior.nc
+        self.hid, self.layers = enc.embed_ch, enc.lstm.num_layers
+        self.M = batch * self.H * self.W
+        f16 = dict(device=device, dtype=torch.float16)
+        self.S = torch.zeros(2, self.M, 8, **f16)
+        self.A = torch.zeros(self.layers, 2, 2, self.M, 2 * self.hid, **f16)
+        self.c = torch.zeros(self.layers, self.M, self.hid, device=device)
+        self.noise = torch.zeros(self.nc, self.M, device=device)
+        self._cache = enc.__dict__.setdefault("_flowk_sample_cache", _Cache())
+
+    def _steps(self, ops, z):
+        """The launch arguments of an even and an odd channel (SAMPLE's noise / z pointers are set per channel)."""
+        B, H, W, hid, L = self.B, self.H, self.W, self.hid, self.layers
+        S = (self.S[0], self.S[1])
+
+        def rows(layer, parity, col):
+            return (self.A[layer, parity, 0], self.A[layer, parity, 1], 2 * hid, col)
+
+        steps = []
+        for p in (0, 1):
+            (ew, eb, etaps), (ow, ob, otaps) = ops["embed"], ops["out"]
+            seq = [tc.mar_step_args(_lib.MAR_EMBED, S, ew, eb, B, H, W, etaps, hid, rows(0, p, 0))]
+            for layer, (lw, lb, ltaps) in enumerate(ops["layers"]):
+                seq.append(tc.mar_step_args(_lib.MAR_LSTM, rows(layer, p, 0)[:2], lw, lb, B, H, W, ltaps, hid,
+                                            rows(layer, 1 - p, hid), dilation=self.enc.lstm.dilation,
+                                            dst1=rows(layer + 1, p, 0) if layer + 1 < L else None, c=self.c[layer]))
+            seq.append(tc.mar_step_args(_lib.MAR_SAMPLE, rows(L - 1, 1 - p, 0)[:2], ow, ob, B, H, W, otaps, hid,
+                                        S + (8, 0), noise=self.noise, z=z, z_stride=self.nc * H * W))
+            steps.append(seq)
+        return steps
+
+    def sample(self, z1=None, noise=None):
+        """z2 [B, nc, H, W] given z1 (the half that continues through the flow; None at the last level).  `noise`
+        [nc, B, ..., H, W] (any device) is copied into the noise buffer first; None samples with what it holds."""
+        B, H, W = self.B, self.H, self.W
+        ops = self._cache.get(list(self.enc.parameters()), lambda: _sampling_operands(self.enc))
+        if noise is not None:
+            self.noise.copy_(noise.reshape(self.nc, self.M))
+        if z1 is None:
+            self.S.zero_()
+        else:
+            emb = z1_embedding(self.prior.z1_cond_network, z1)
+            tc.nchw_to_nhwc_hilo(torch.cat([emb.new_zeros(B, 1, H, W), emb], 1), 8, True, out=(self.S[0], self.S[1]))
+        self.A.zero_()                                   # h_{-1} = 0, c_{-1} = 0
+        self.c.zero_()
+        z2 = torch.empty(B, self.nc, H, W, device=self.noise.device)
+        steps = self._steps(ops, z2)
+        noise0, z0 = self.noise.data_ptr(), z2.data_ptr()
+        for t in range(self.nc):
+            seq = steps[t % 2]
+            seq[-1].noise = noise0 + 4 * t * self.M
+            seq[-1].z = z0 + 4 * t * H * W
+            for args in seq:
+                tc.mar_step(args)
+        return z2
+
+
+def sampler_for(prior, batch, device):
+    """The AncestralSampler eager sampling uses for (prior, batch size, device)."""
+    samplers = prior.__dict__.setdefault("_flowk_samplers", {})
+    key = (batch, str(torch.device(device)))
+    if key not in samplers:
+        samplers[key] = AncestralSampler(prior, batch, device)
+    return samplers[key]

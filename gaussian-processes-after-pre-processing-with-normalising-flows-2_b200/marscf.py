@@ -226,19 +226,23 @@ class FlowNet(nn.Module):
             i -= 1
         return (z, ldj) if with_logdet else z
 
-    def decode(self, z, eps_std=None):
+    def decode(self, z, eps_std=None, prior=None):
+        """Sample (marscf_main.py:167-175): the last level's latent, then at every split z2 given the decoded z1.
+        `prior` (default: self.c_prior) takes the same calls as c_prior, e.g. one whose samples come from a CUDA graph's
+        device-side noise."""
+        prior = self.c_prior if prior is None else prior
         if z is None:
-            z = self.c_prior(None, self.L, reverse=True, eps_std=eps_std, batch_size=self.batch_size,
-                             device=next(self.parameters()).device)
+            z = prior(None, self.L, reverse=True, eps_std=eps_std, batch_size=self.batch_size,
+                      device=next(self.parameters()).device)
         else:
-            z = self.c_prior(z, self.L, reverse=True, eps_std=eps_std)
+            z = prior(z, self.L, reverse=True, eps_std=eps_std)
         layers = list(self.layers)
         i = len(layers) - 1
         while i >= 0:
             layer = layers[i]
             prev = layers[i - 1] if i > 0 else None
             if isinstance(layer, Split2dMsC):
-                z2 = self.c_prior(z, layer.level, reverse=True, eps_std=eps_std)
+                z2 = prior(z, layer.level, reverse=True, eps_std=eps_std)
                 z, _ = layer((z, z2), logdet=0, reverse=True)
             elif (self.fuse_squeeze and isinstance(layer, FlowStep) and isinstance(prev, SqueezeLayer)
                   and prev.factor == 2):

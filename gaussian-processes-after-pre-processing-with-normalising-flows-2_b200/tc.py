@@ -99,15 +99,40 @@ def conv_gemm(a_hi, a_lo, w_hi, w_lo, B, H, W, Cin, N, taps, pre, out_mask, bias
     _lib.call("flowk_conv_gemm", ctypes.addressof(args), _stream(), meta=(B, H, W, Cin, N, taps, pre))
 
 
-def nchw_to_nhwc_hilo(x, c_pad, f16=False):
-    """x: NCHW view whose (C,H,W) block is contiguous (e.g. a channel slice) -> ([B*HW, c_pad] hi, lo)."""
+def nchw_to_nhwc_hilo(x, c_pad, f16=False, out=None):
+    """x: NCHW view whose (C,H,W) block is contiguous (e.g. a channel slice) -> ([B*HW, c_pad] hi, lo), written into
+    `out` = (hi, lo) when given."""
     b, c, h, w = x.shape
     assert x.stride(3) == 1 and x.stride(2) == w and x.stride(1) == h * w, "channel slice of a contiguous NCHW tensor"
-    hi = torch.empty(b * h * w, c_pad, device=x.device, dtype=torch.float16 if f16 else torch.float32)
-    lo = torch.empty_like(hi)
+    if out is None:
+        hi = torch.empty(b * h * w, c_pad, device=x.device, dtype=torch.float16 if f16 else torch.float32)
+        lo = torch.empty_like(hi)
+    else:
+        hi, lo = out
+        assert hi.shape == lo.shape == (b * h * w, c_pad) and hi.is_contiguous() and lo.is_contiguous()
+        assert hi.dtype == lo.dtype == (torch.float16 if f16 else torch.float32)
     _lib.call("flowk_nchw_to_nhwc_hilo_f16" if f16 else "flowk_nchw_to_nhwc_hilo", x.data_ptr(), x.stride(0), b, c, h * w,
               c_pad, hi.data_ptr(), lo.data_ptr(), _stream())
     return hi, lo
+
+
+def mar_step_args(mode, a, w, bias, B, H, W, taps, hid, dst0, dilation=1, dst1=None, c=None, noise=None, z=None,
+                  z_stride=0, status=None):
+    """flowk_mar_step_args for one step of mAR ancestral sampling (include/flowk.h).  a = (hi, lo) fp16 rows [B*H*W, Cin];
+    w = (w_hi, w_lo, acc_scale) from conv_weight_operand_f16; dst0 / dst1 = (hi, lo, pitch, column) with hi / lo the fp16
+    row arrays; noise / z are fp32 tensors whose data pointers are the first element the step reads / writes.  The
+    struct holds raw pointers: the tensors must outlive every launch made with it."""
+    assert a[0].dtype == a[1].dtype == w[0].dtype == w[1].dtype == torch.float16
+    _lib.check_device(a[0], "mar_step")
+    d1 = dst1 or (None, None, 0, 0)
+    return _lib.MarStepArgs(_p(a[0]), _p(a[1]), _p(w[0]), _p(w[1]), _p(bias), _p(dst0[0]), _p(dst0[1]), _p(d1[0]),
+                            _p(d1[1]), _p(c), _p(noise), _p(z), int(z_stride), _p(status), int(mode), B, H, W,
+                            a[0].shape[1], taps, int(dilation), hid, dst0[2], dst0[3], d1[2], d1[3], float(w[2]))
+
+
+def mar_step(args):
+    """Enqueue flowk_mar_step(args) on the current stream."""
+    _lib.call("flowk_mar_step", ctypes.addressof(args), _stream(), meta=(args.mode, args.B, args.H, args.W, args.hid))
 
 
 def split_rows(x):

@@ -197,6 +197,46 @@ int flowk_conv_gemm(const flowk_conv_gemm_args* args, flowk_stream_t stream);
 /* Slices flowk_conv_gemm would use for `args` if args->splitk_ws were non-null (1 = no split-K); no pointer is read. */
 int flowk_conv_gemm_splitk_slices(const flowk_conv_gemm_args* args);
 
+/* ---- one step of ancestral sampling from the mAR channel prior (mar_prior/corr_prior.py:66-101) -------------------------
+ * The implicit GEMM of flowk_conv_gemm (FLOWK_OPERAND_F16 only: a_* / w_* / dst*_ are fp16 arrays, weights
+ * [N, taps * ceil64(Cin)] from flowk_pack_weight_f16 with acc_scale = 1 / their pre-scaling) with one of three epilogues.
+ * Every activation row is [B*H*W, Cin] NHWC; hid = the ConvLSTM width (hid % 8 == 0, 4 hid <= 256).  A destination d is
+ * the fp16 pair dst<d>_hi / dst<d>_lo written at row m, columns [dst<d>_col, dst<d>_col + width) of rows dst<d>_pitch
+ * elements long.  `mode` selects:
+ *   FLOWK_MAR_EMBED   N = hid: y = D + bias (conv_embed on the step input [prev sample | z1 embedding | 0]), width hid, to
+ *                     dst 0
+ *   FLOWK_MAR_LSTM    N = 4 hid gate columns [i | f | g | o] of one ConvLSTM layer from ONE GEMM over the rows [x_t | h_{t-1}]
+ *                     (Cin = 2 hid) with weights [W_ih | W_hh] per tap and bias = b_ih + b_hh (functional.py:30-52):
+ *                     c [B*H*W, hid] (fp32, c_{t-1} in, c_t out, in place), h_t = sig(o) tanh(c_t), width hid, to dst 0
+ *                     and, when dst1_hi is non-NULL, to dst 1
+ *   FLOWK_MAR_SAMPLE  N = 2 columns (mean, log-std) of conv_out1 (weights [0 | W_out] over [x | h] rows), never stored:
+ *                     s = noise[m] * exp(log-std) + mean (fp32, accurate exp) to z[b * z_stride + hw] and, width 1, to dst 0
+ * A launch must not write rows it reads (neighbouring taps belong to other CTAs): callers ping-pong buffers by step parity.
+ * Returns FLOWK_ERR_ARG for a pointer the mode needs that is NULL (dst 1 is optional) or a bad mode / taps / acc_scale,
+ * FLOWK_ERR_SHAPE for a bad hid, Cin, destination (column + width beyond the pitch, pitch or column not a multiple of 4)
+ * or z_stride < H*W, or maps that do not tile into 128-row blocks (W | 128, and H*W | 128 or 128 | H*W) - before any launch. */
+enum { FLOWK_MAR_EMBED = 0, FLOWK_MAR_LSTM = 1, FLOWK_MAR_SAMPLE = 2 };
+typedef struct flowk_mar_step_args {
+  const void* a_hi;       /* activation pair [B*H*W, Cin] */
+  const void* a_lo;
+  const void* w_hi;       /* weight pair [N, taps * ceil64(Cin)] */
+  const void* w_lo;
+  const float* bias;      /* [N] */
+  void* dst0_hi;
+  void* dst0_lo;
+  void* dst1_hi;          /* FLOWK_MAR_LSTM only, optional */
+  void* dst1_lo;
+  float* c;               /* FLOWK_MAR_LSTM: cell state [B*H*W, hid] */
+  const float* noise;     /* FLOWK_MAR_SAMPLE: [B*H*W] */
+  float* z;               /* FLOWK_MAR_SAMPLE: z[b * z_stride + hw] (the caller points it at the channel) */
+  long long z_stride;
+  int* status;            /* device int, may be NULL: set to 1 if an internal barrier wait timed out */
+  int mode, B, H, W, Cin, taps, dilation, hid;   /* taps 1, 9 or 25; dilation 0 or 1 = dense */
+  int dst0_pitch, dst0_col, dst1_pitch, dst1_col;
+  float acc_scale;
+} flowk_mar_step_args;
+int flowk_mar_step(const flowk_mar_step_args* args, flowk_stream_t stream);
+
 /* x[b, ch, p] (NCHW, `batch_stride` floats between samples, ch < C) -> NHWC hi/lo [B*HW, C_pad], zero-padded channels. */
 int flowk_nchw_to_nhwc_hilo(const float* x, long long batch_stride, int B, int C, int HW, int C_pad,
                             float* hi, float* lo, flowk_stream_t stream);
