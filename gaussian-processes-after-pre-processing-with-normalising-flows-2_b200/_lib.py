@@ -83,6 +83,10 @@ SIGNATURES = {
     "flowk_adamax_step": ([_fp, _i, _fp, ctypes.c_float, ctypes.c_float, ctypes.c_float, _st], _i),
     "flowk_glu_bwd": ([_fp, _fp, _fp, ctypes.c_longlong, _i, ctypes.c_longlong, _st], _i),
     "flowk_mar_step": ([ctypes.c_void_p, _st], _i),
+    "flowk_conv_wgrad_nhwc_splits": ([_i] * 7 + [ctypes.POINTER(ctypes.c_int)], _i),
+    "flowk_conv_wgrad_nhwc": ([_fp] * 4 + [_i] * 7 + [_st], _i),
+    "flowk_lstm_cell_bwd": ([_fp] * 11 + [ctypes.c_longlong, _i, _st], _i),
+    "flowk_f16_pair_to_f32": ([_fp] * 3 + [ctypes.c_longlong, _i, _i, _st], _i),
 }
 
 
@@ -138,6 +142,7 @@ DIMS = {
     "flowk_patch_attention": slice(6, 10),
     "flowk_patch_attention_train_fwd": slice(7, 11), "flowk_patch_attention_bwd": slice(8, 12),
     "flowk_pack_weight_f16": slice(6, 10), "flowk_fold_actnorm_invconv": slice(7, 11),
+    "flowk_conv_wgrad_nhwc": slice(4, 11), "flowk_lstm_cell_bwd": slice(11, 13), "flowk_f16_pair_to_f32": slice(3, 6),
 }
 
 

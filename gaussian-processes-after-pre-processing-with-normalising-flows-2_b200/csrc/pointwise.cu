@@ -3,6 +3,7 @@
 //   glu(x)        = x[:, :C] * sigmoid(x[:, C:])    flow_modules/mixlogcdf_nn.py:149-151,257-258
 // Tensors are viewed as [outer, channels, inner]: inner = H*W for the NCHW convolutional branch (split along dim 1),
 // inner = 1 for the NHWC attention branch (split along the last dim).  HBM-bound: 12 B / 12 B per input element.
+#include <cuda_fp16.h>
 #include "common.cuh"
 
 namespace flowk {
@@ -872,5 +873,95 @@ extern "C" int flowk_std_normal_logp(const float* z, long long sample_stride, co
   if (B == 0) return FLOWK_OK;
   if (!z || !out) return FLOWK_ERR_ARG;
   flowk::std_normal_logp_kernel<<<B, 256, 0, stream>>>(z, sample_stride, in, out, n);
+  return flowk::launch_status();
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// ConvLSTM cell backward of one time step (the cell of mar_prior/convolutional_rnn/functional.py:30-52, forward in the
+// PRE_LSTM epilogue of csrc/tc_gemm.cu).  Rows [M, 4 hid] of gate pre-activations a = gi + hh ([i | f | g | o], hh the
+// recomputed hidden-to-hidden term with b_hh), cell states c_{t-1}, c_t [M, hid]; dh = dh_a (+ dh_b), the gradient of h_t
+// from the layer above and from step t+1; dc_next = dL/dc_t arriving from step t+1 (already multiplied by f_{t+1}):
+//   dc = dh o tanh'(c_t) + dc_next      do = dh tanh(c_t) o'      di = dc g i'      df = dc c_{t-1} f'      dg = dc i tanh'(g)
+// -> dgates [M, 4 hid] fp32 and as the TF32 (hi, lo) pair the input-gradient GEMM reads, and dc_prev = dc f (dL/dc_{t-1}).
+// Sigmoid' = s(a) s(-a) and tanh' = 4e / (1 + e)^2 with e = exp(-2|x|) keep their relative accuracy in saturated gates.
+// One thread per (row, unit): the four gates of a unit are independent of every other unit.  dc_prev may alias dc_next.
+namespace flowk {
+
+__device__ __forceinline__ float sigm(float a) { return 1.f / (1.f + expf(-a)); }
+__device__ __forceinline__ float dtanh_of(float x) {
+  const float e = expf(-2.f * fabsf(x));
+  return 4.f * e / ((1.f + e) * (1.f + e));
+}
+__device__ __forceinline__ void tf32_pair(float v, float& hi, float& lo) {
+  hi = __uint_as_float((__float_as_uint(v) + 0x1000u) & 0xffffe000u);
+  lo = __uint_as_float((__float_as_uint(v - hi) + 0x1000u) & 0xffffe000u);
+}
+
+__global__ void __launch_bounds__(256) lstm_cell_bwd_kernel(const float* __restrict__ gi, const float* __restrict__ hh,
+                                                            const float* __restrict__ c_prev, const float* __restrict__ c,
+                                                            const float* __restrict__ dh_a, const float* __restrict__ dh_b,
+                                                            const float* dc_next, float* __restrict__ dgates,
+                                                            float* __restrict__ dg_hi, float* __restrict__ dg_lo,
+                                                            float* dc_prev, long long total, int hid) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const long long m = e / hid;
+    const int j = (int)(e - m * hid);
+    const size_t g0 = (size_t)m * 4 * hid + j;
+    float a[4];
+#pragma unroll
+    for (int q = 0; q < 4; ++q) a[q] = __ldg(hh + g0 + (size_t)q * hid) + __ldg(gi + g0 + (size_t)q * hid);
+    const float ig = sigm(a[0]), fg = sigm(a[1]), gg = tanhf(a[2]), og = sigm(a[3]);
+    const float ct = __ldg(c + e), cp = __ldg(c_prev + e);
+    const float dh = __ldg(dh_a + e) + (dh_b ? __ldg(dh_b + e) : 0.f);
+    const float dc = dh * og * dtanh_of(ct) + (dc_next ? dc_next[e] : 0.f);
+    float d[4];
+    d[0] = dc * gg * (ig * sigm(-a[0]));
+    d[1] = dc * cp * (fg * sigm(-a[1]));
+    d[2] = dc * ig * dtanh_of(a[2]);
+    d[3] = dh * tanhf(ct) * (og * sigm(-a[3]));
+    dc_prev[e] = dc * fg;
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const size_t o = g0 + (size_t)q * hid;
+      float h, l;
+      tf32_pair(d[q], h, l);
+      dgates[o] = d[q];
+      dg_hi[o] = h;
+      dg_lo[o] = l;
+    }
+  }
+}
+
+// fp16 (hi, lo) operand rows [M, C] -> fp32 rows [M, C_out] = hi + lo, columns C..C_out-1 zero (the weight-gradient
+// kernels read fp32 containers with whole 32-channel blocks)
+__global__ void __launch_bounds__(256) f16_pair_to_f32_kernel(const __half* __restrict__ hi, const __half* __restrict__ lo,
+                                                              float* __restrict__ out, long long total, int C, int C_out) {
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const long long m = e / C_out;
+    const int c = (int)(e - m * C_out);
+    out[e] = c < C ? __half2float(hi[(size_t)m * C + c]) + __half2float(lo[(size_t)m * C + c]) : 0.f;
+  }
+}
+
+}  // namespace flowk
+
+extern "C" int flowk_lstm_cell_bwd(const float* gi, const float* hh, const float* c_prev, const float* c, const float* dh,
+                                   const float* dh_rec, const float* dc_next, float* dgates, float* dg_hi, float* dg_lo,
+                                   float* dc_prev, long long M, int hid, flowk_stream_t stream) {
+  if (M < 0 || hid < 1) return FLOWK_ERR_SHAPE;
+  if (M == 0) return FLOWK_OK;
+  if (!gi || !hh || !c_prev || !c || !dh || !dgates || !dg_hi || !dg_lo || !dc_prev) return FLOWK_ERR_ARG;
+  flowk::lstm_cell_bwd_kernel<<<grid_for(M * hid), 256, 0, stream>>>(gi, hh, c_prev, c, dh, dh_rec, dc_next, dgates, dg_hi,
+                                                                      dg_lo, dc_prev, M * hid, hid);
+  return flowk::launch_status();
+}
+
+extern "C" int flowk_f16_pair_to_f32(const void* hi, const void* lo, float* out, long long M, int C, int C_out,
+                                     flowk_stream_t stream) {
+  if (M < 0 || C < 1 || C_out < C) return FLOWK_ERR_SHAPE;
+  if (M == 0) return FLOWK_OK;
+  if (!hi || !lo || !out) return FLOWK_ERR_ARG;
+  flowk::f16_pair_to_f32_kernel<<<grid_for(M * C_out), 256, 0, stream>>>(
+      reinterpret_cast<const __half*>(hi), reinterpret_cast<const __half*>(lo), out, M * C_out, C, C_out);
   return flowk::launch_status();
 }

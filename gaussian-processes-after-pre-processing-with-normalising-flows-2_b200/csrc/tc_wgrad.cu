@@ -9,6 +9,11 @@
 // A column shift dx = +-1 cannot be a TMA coordinate (the innermost coordinate must be 16-byte aligned: measured,
 // profiles/dbg/tma_box_probe.cu), so the caller passes two column-shifted copies of x (flowk_shift_columns, zero at
 // the image border) and the tap picks its tensor map.
+// NHWC rows (flowk_conv_wgrad_nhwc: the mAR prior's time-major [T*B*H*W, C] tensors, 3x3 / 5x5 taps at any dilation)
+// need no copies: a k-block is a 5-D box (32 channels, bw columns, bh rows, bb images; bw * bh * bb = 32 pixels) whose
+// W / H start coordinates carry the tap's (dx, dy) * dilation - the innermost dimension is the channel block, so every
+// shift is aligned - and the TMA unit zero-fills pixels outside the image ("same" padding).  Per 32-channel block the
+// tile is the [32 pixels x 128 B] MN-major tile of the row-major (Linear) mode, read with the same descriptors.
 // No operand is pre-split in HBM: tcgen05 kind::tf32 ignores the 13 low mantissa bits of its fp32 containers
 // (measured, profiles/trunc_probe.py), so the raw tile IS `hi`, and eight converter warps build
 // lo = rna(x - trunc(x)) into a second tile (same swizzled offsets, pure elementwise) while the previous k-block's
@@ -34,6 +39,8 @@ struct WgradParams {
   int shift_a;                    // 1: the A side is x (carries the tap shift), 0: the B side is
   int rows;                       // 1: row-major operands [M, C] (Linear layers): MN-major tiles of [32 rows x 32 channels]
                                   //    blocks, 3-D TMA boxes (32 ch, 32 rows, blocks), transposed UMMA descriptors
+                                  // 2: NHWC rows [NB*H*W, C] of a k x k (dilated) convolution: the same tiles, fetched as
+                                  //    5-D boxes (32 ch, bw, bh, bb, blocks) whose W / H coordinates carry the tap shift
   int g_tile_bytes;               // shared-memory bytes reserved for the A tile (its real rows, rounded to 8)
   int kblk;                       // pixels per k-block: 32 (128-byte swizzle rows) or 16 (64-byte rows, H*W == 16 maps)
   int W;                          // image width: a row shift is W pixels
@@ -43,6 +50,8 @@ struct WgradParams {
   int stages, stage_bytes, tmem_cols;
   float* partial;                 // [splits][taps][N][Cin]
   int* status;
+  int ksz, dil;                   // rows == 2: taps = ksz * ksz, tap (ky, kx) reads pixel + ((ky, kx) - ksz / 2) * dil
+  int bw, bh, bb, kpi_w, kpi_h;   // rows == 2: k-block box (bw x bh pixels x bb images = 32), boxes per image row / column
 };
 
 __global__ void __launch_bounds__(WG_THREADS, 1)
@@ -100,7 +109,15 @@ conv_wgrad_kernel(const __grid_constant__ CUtensorMap map_g, const __grid_consta
         uint8_t* st = smem + (size_t)s * p.stage_bytes;
         mbar_expect_tx(&full_raw[s], (uint32_t)(g_bytes + x_bytes));
         const CUtensorMap* mx = dx < 0 ? &map_xm : dx > 0 ? &map_xp : &map_x;
-        if (p.rows) {                 // k-block = rows [32 kb, 32 kb + 32); A side = map_g when !shift_a
+        if (p.rows == 2) {            // k-block = a (bw, bh, bb) box of pixels; out-of-image taps are zero-filled by TMA
+          const int sy = (tap / p.ksz - p.ksz / 2) * p.dil, sx = (tap % p.ksz - p.ksz / 2) * p.dil;
+          const int r = kb / p.kpi_w, w0 = (kb - r * p.kpi_w) * p.bw;
+          const int h0 = (r % p.kpi_h) * p.bh, b0 = (r / p.kpi_h) * p.bb;
+          const int ay = p.shift_a ? sy : 0, ax = p.shift_a ? sx : 0;
+          tma_load_5d(st, p.shift_a ? &map_x : &map_g, &full_raw[s], 0, w0 + ax, h0 + ay, b0, mt * (BLOCK_M / 32));
+          tma_load_5d(st + x_off, p.shift_a ? &map_g : &map_x, &full_raw[s], 0, w0 + sx - ax, h0 + sy - ay, b0,
+                      ct * (p.c_tile / 32));
+        } else if (p.rows) {          // k-block = rows [32 kb, 32 kb + 32); A side = map_g when !shift_a
           tma_load_3d(st, p.shift_a ? &map_x : &map_g, &full_raw[s], 0, kb * BLOCK_K, mt * (BLOCK_M / 32));
           tma_load_3d(st + x_off, p.shift_a ? &map_g : &map_x, &full_raw[s], 0, kb * BLOCK_K, ct * (p.c_tile / 32));
         } else if (p.shift_a) {
@@ -430,5 +447,101 @@ extern "C" int flowk_conv_wgrad(const float* x, const float* x_left, const float
   }
   FLOWK_CUDA_OK(launch_pdl(conv_wgrad_kernel, dim3(pl.m_tiles * taps * pl.c_tiles, pl.splits), dim3(WG_THREADS), smem,
                            stream, mg, mx, mxm, mxp, p));
+  return FLOWK_OK;
+}
+
+// NHWC rows [NB, H, W, C] (C % 32 == 0) viewed by TMA as dims (32, W, H, NB, C/32); box (32 channels, bw, bh, bb, blocks):
+// per 32-channel block a [32 pixels x 128 B] tile laid out (and swizzled) exactly like make_map_rows' [32 rows x 128 B]
+static bool make_map_nhwc(CUtensorMap* map, const float* base, int NB, int H, int W, int C, int bw, int bh, int bb,
+                          int blocks) {
+  cuuint64_t dims[5] = {32, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)NB, (cuuint64_t)(C / 32)};
+  cuuint64_t strides[4] = {(cuuint64_t)C * 4, (cuuint64_t)W * C * 4, (cuuint64_t)H * W * C * 4, 128};
+  cuuint32_t box[5] = {32, (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bb, (cuuint32_t)blocks};
+  cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+  return encode_fn() && encode_fn()(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 5, const_cast<float*>(base), dims, strides, box,
+                                    estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B,
+                                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
+struct NhwcBox {
+  int bw, bh, bb;
+};
+
+// The plan of plan_linear_wgrad over M = NB*H*W rows, with the split-K count re-balanced over taps x tiles CTAs and the
+// k-block box: bw = min(W, 32) columns, bh rows, bb images (bw * bh * bb = 32; every box lies in whole images).
+static WgradPlan plan_nhwc_wgrad(int NB, int H, int W, int Cin, int N, int taps, int dil, NhwcBox* box) {
+  WgradPlan none = {};
+  if (NB < 1 || H < 1 || W < 1 || dil < 1 || (taps != 1 && taps != 9 && taps != 25)) return none;
+  if (W <= 32 ? 32 % W : W % 32) return none;
+  const int bw = W < 32 ? W : 32, bh = H < 32 / bw ? H : 32 / bw;
+  if (H % bh || 32 % (bw * bh)) return none;
+  const int bb = 32 / (bw * bh);
+  if (NB % bb || (long long)NB * H * W > 0x7fffffffLL) return none;
+  WgradPlan pl = plan_linear_wgrad((long long)NB * H * W, Cin, N);
+  if (!pl.ok) return pl;
+  const long long total_kb = (long long)NB * H * W / BLOCK_K;
+  const int tiles = pl.m_tiles * taps * pl.c_tiles;
+  long long s = (148 + tiles / 2) / tiles;
+  if (s > total_kb / 4) s = total_kb / 4;
+  if (s > 64) s = 64;
+  if (s < 1) s = 1;
+  pl.splits = (int)s;
+  if (box) *box = NhwcBox{bw, bh, bb};
+  return pl;
+}
+
+extern "C" int flowk_conv_wgrad_nhwc_splits(int NB, int H, int W, int Cin, int N, int taps, int dilation, int* transposed) {
+  const WgradPlan pl = plan_nhwc_wgrad(NB, H, W, Cin, N, taps, dilation, nullptr);
+  if (transposed) *transposed = pl.ok ? pl.swap : 0;
+  return pl.ok ? pl.splits : 0;
+}
+
+extern "C" int flowk_conv_wgrad_nhwc(const float* x, const float* gy, float* partial, int* status, int NB, int H, int W,
+                                     int Cin, int N, int taps, int dilation, flowk_stream_t stream) {
+  NhwcBox bx;
+  const WgradPlan pl = plan_nhwc_wgrad(NB, H, W, Cin, N, taps, dilation, &bx);
+  if (!pl.ok) return FLOWK_ERR_SHAPE;
+  if (!x || !gy || !partial) return FLOWK_ERR_ARG;
+  if (!aligned16(x) || !aligned16(gy) || !aligned16(partial)) return FLOWK_ERR_ALIGN;
+  WgradParams p = {};
+  p.N = pl.a_ch;
+  p.Cin = pl.b_ch;
+  p.shift_a = pl.swap;
+  p.rows = 2;
+  p.kblk = BLOCK_K;
+  p.g_tile_bytes = pl.g_tile_bytes;
+  p.taps = taps;
+  p.ksz = taps == 25 ? 5 : taps == 9 ? 3 : 1;
+  p.dil = dilation;
+  p.W = W;
+  p.bw = bx.bw;
+  p.bh = bx.bh;
+  p.bb = bx.bb;
+  p.kpi_w = W / bx.bw;
+  p.kpi_h = H / bx.bh;
+  p.total_kb = (int)((long long)NB * H * W / BLOCK_K);
+  p.kb_per_image = p.total_kb;
+  const int a_blocks = pl.g_tile_bytes / 4096, b_blocks = (pl.b_ch < pl.c_tile ? pl.b_ch : pl.c_tile) / 32;
+  p.g_rows = a_blocks * 32;
+  p.x_rows = b_blocks * 32;
+  p.c_tile = pl.c_tile;
+  p.c_tiles = pl.c_tiles;
+  p.m_tiles = pl.m_tiles;
+  p.stages = pl.stages;
+  p.stage_bytes = pl.stage_bytes;
+  p.tmem_cols = pl.tmem_cols;
+  p.partial = partial;
+  p.status = status;
+  CUtensorMap mg, mx;
+  if (!make_map_nhwc(&mg, gy, NB, H, W, N, bx.bw, bx.bh, bx.bb, pl.swap ? b_blocks : a_blocks) ||
+      !make_map_nhwc(&mx, x, NB, H, W, Cin, bx.bw, bx.bh, bx.bb, pl.swap ? a_blocks : b_blocks))
+    return FLOWK_ERR_ARG;
+  const size_t smem = (size_t)pl.stages * pl.stage_bytes + 1024 + (BLOCK_M * 128 - pl.g_tile_bytes);
+  if (smem > g_wgrad_smem_attr) {
+    FLOWK_CUDA_OK(cudaFuncSetAttribute(conv_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    g_wgrad_smem_attr = smem;
+  }
+  FLOWK_CUDA_OK(launch_pdl(conv_wgrad_kernel, dim3(pl.m_tiles * taps * pl.c_tiles, pl.splits), dim3(WG_THREADS), smem, stream,
+                           mg, mx, mx, mx, p));
   return FLOWK_OK;
 }

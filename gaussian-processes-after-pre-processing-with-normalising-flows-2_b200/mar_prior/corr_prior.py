@@ -5,8 +5,9 @@ like the reference's `c_prior(z, level, reverse=...)`.
 
 On CUDA tensors with autograd off (evaluation, sampling) the networks run on the flowk tensor-core kernels
 (`mar_prior/cuda_path.py`: every conv a tcgen05 implicit GEMM, the LSTM cell fused into the recurrent GEMM's epilogue;
-sampling through `AncestralSampler`, 2 + num_layers launches per channel); training (autograd) and CPU tensors use the
-torch layers below."""
+sampling through `AncestralSampler`, 2 + num_layers launches per channel).  Training (autograd on, dp_rate = 0 or eval
+mode) runs on them too, with backward through time on flowk kernels (`cuda_path.run_sequence_train`); training with
+channel dropout, shapes the kernels do not take and CPU tensors use the torch layers below."""
 import numpy as np
 import torch
 import torch.nn as nn
@@ -46,10 +47,18 @@ class ChannelPriorUniScale(nn.Module):
         return -0.5 * (logs * 2. + ((z - mean) ** 2) / torch.exp(logs * 2.) + self.Log2PI)
 
     def get_likelihood(self, z):
-        fast = cuda_path.usable(self, z[1] if isinstance(z, (tuple, list)) else z) and not (self.training and self.dp_rate > 0)
+        zz = z[1] if isinstance(z, (tuple, list)) else z
+        no_dropout = not (self.training and self.dp_rate > 0)
+        fast = cuda_path.usable(self, zz) and no_dropout
+        train = not fast and no_dropout and cuda_path.trainable(self, zz)
         if isinstance(z, (tuple, list)):
             z1, z2 = z
-            emb = cuda_path.z1_embedding(self.z1_cond_network, z1) if fast else self.z1_cond_network(z1)
+            if fast:
+                emb = cuda_path.z1_embedding(self.z1_cond_network, z1)
+            elif train:
+                emb = cuda_path.z1_embedding_train(self.z1_cond_network, z1)
+            else:
+                emb = self.z1_cond_network(z1)
             z1_embd = emb.unsqueeze(1).repeat(1, z2.size(1), 1, 1, 1)
         else:
             z1_embd, z2 = None, z
@@ -60,6 +69,8 @@ class ChannelPriorUniScale(nn.Module):
             lstm_input = torch.cat([lstm_input, z1_embd], dim=2)
         if fast:
             out = cuda_path.run_sequence(self.prior_lstm, lstm_input)
+        elif train:
+            out = cuda_path.run_sequence_train(self.prior_lstm, lstm_input)
         else:
             out, _ = self.prior_lstm(lstm_input, None)
         return torch.sum(self.likelihood(out[:, :, 0:1], out[:, :, 1:2], z2), dim=(1, 2, 3, 4))

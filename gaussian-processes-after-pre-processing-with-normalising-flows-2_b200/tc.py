@@ -37,12 +37,14 @@ def conv_weight_operand(w, cin_pad=None):
     return split_hilo(wk.reshape(n, kh * kw * cin_pad))
 
 
-def conv_weight_operand_f16(w, gain=None, mode=_lib.PACK_PLAIN, factor=1.0, bias=None):
+def conv_weight_operand_f16(w, gain=None, mode=_lib.PACK_PLAIN, factor=1.0, bias=None, device_scale=False):
     """[N, Cin, kh, kw] conv weight (or [N, Cin] linear weight) -> fp16 (hi, lo) pair [N, taps * ceil64(Cin)] in (tap, c)
     order for FLOWK_OPERAND_F16, pre-scaled by a power of two s so that max|w s| lies in [2^14, 2^15): the lo part then
     keeps its 11 bits clear of fp16's subnormal range.  `gain` / `mode` fuse a per-output-channel factor (weight norm, or an
     ActNorm's exp(factor * logs) with `bias` scaled alike) - see flowk_pack_weight_f16.  Two launches per weight.
-    Returns (hi, lo, 1 / s[, bias * gain]); 1 / s goes to conv_gemm(acc_scale=)."""
+    Returns (hi, lo, 1 / s[, bias * gain]); 1 / s goes to conv_gemm(acc_scale=).  With `device_scale` 1 / s stays on the
+    device as a 1-element tensor for conv_gemm(acc_scale=1, acc_scale_ptr=): no host read, so the packing can be captured
+    in a CUDA graph and re-run at every replay."""
     if w.dim() == 2:
         w = w[:, :, None, None]
     n, cin, kh, kw = w.shape
@@ -59,6 +61,9 @@ def conv_weight_operand_f16(w, gain=None, mode=_lib.PACK_PLAIN, factor=1.0, bias
     assert g is None or g.numel() == n
     _lib.call("flowk_pack_weight_f16", w.data_ptr(), _p(g), int(mode), float(factor), _p(b_in), _p(b_out), n, cin, taps,
               cin_pad, hi.data_ptr(), lo.data_ptr(), ws.data_ptr(), _stream())
+    if device_scale:
+        assert bias is None
+        return hi, lo, ws[n + 1:]
     acc_scale = float(ws[n + 1])                       # (host sync: cached per weight version)
     return (hi, lo, acc_scale) if bias is None else (hi, lo, acc_scale, b_out)
 

@@ -361,6 +361,24 @@ int flowk_linear_wgrad_splits(long long M, int K, int N, int* transposed);
 int flowk_linear_wgrad(const float* x, const float* gy, float* partial, int* status, long long M, int K, int N,
                        flowk_stream_t stream);
 int flowk_shift_columns(const float* x, float* x_left, float* x_right, long long total, int W, flowk_stream_t stream);
+/* Same for a stride-1 "same" convolution over NHWC rows x [NB*H*W, Cin], gy [NB*H*W, N] (Cin % 32 == 0, N % 32 == 0;
+ * the mAR prior's time-major tensors, NB = T*B images), taps = 1, 9 or 25 at any dilation:
+ *   partial[s][t][n][c] = sum over the s-th slice of (image, pixel) of gy[., n, p] * x[., c, p + (ky, kx - k/2) * dilation]
+ * with out-of-image pixels zero.  No shifted copies: the tap shift is a TMA coordinate.  Shapes: W | 32 or 32 | W, and the
+ * 32-pixel k-block (min(W, 32) columns x bh rows x bb images) must tile the maps (NB % bb == 0).  Replaces the weight
+ * gradients of F.conv2d in the ConvLSTM prior (mar_prior/lstm.py:33-35, 73-74; corr_prior.py:26-28). */
+int flowk_conv_wgrad_nhwc_splits(int NB, int H, int W, int Cin, int N, int taps, int dilation, int* transposed);
+int flowk_conv_wgrad_nhwc(const float* x, const float* gy, float* partial, int* status, int NB, int H, int W, int Cin, int N,
+                          int taps, int dilation, flowk_stream_t stream);
+/* Backward of one ConvLSTM cell step (mar_prior/convolutional_rnn/functional.py:30-52), one thread per (row, unit):
+ * gi, hh [M, 4 hid] (gate pre-activations = gi + hh, order i, f, g, o), c_prev, c [M, hid], dh [M, hid] plus the optional
+ * recurrent dh_rec and dc_next (dL/dc_t from step t+1, already times f_{t+1}) -> dgates [M, 4 hid] fp32 and as the TF32
+ * (hi, lo) operand pair, dc_prev = dL/dc_{t-1} (may alias dc_next). */
+int flowk_lstm_cell_bwd(const float* gi, const float* hh, const float* c_prev, const float* c, const float* dh,
+                        const float* dh_rec, const float* dc_next, float* dgates, float* dg_hi, float* dg_lo, float* dc_prev,
+                        long long M, int hid, flowk_stream_t stream);
+/* fp16 (hi, lo) operand rows [M, C] -> fp32 rows out [M, C_out] = hi + lo, columns >= C zero (C_out >= C). */
+int flowk_f16_pair_to_f32(const void* hi, const void* lo, float* out, long long M, int C, int C_out, flowk_stream_t stream);
 int flowk_weight_norm_bwd_partials(const float* v, const float* g, const float* norm, const float* partial, float* gv,
                                    float* gg, int N, int cin, int taps, int splits, int transposed,
                                    flowk_stream_t stream);
