@@ -232,3 +232,50 @@ def chain_supported(C, n2, f16=False):
     slab = ((4 * 32 * (C + 4) * 4 + 1023) // 1024) * 1024
     kblocks = (C + 63) // 64 if f16 else C // 32
     return slab + kblocks * 32768 + 2 * n2 * 128 + 2048 <= 227 * 1024
+
+
+# The attention half of a ConvAttnBlock (gate, LayerNorm, in_proj, attention, attention gate) as one launch where a 128-row
+# tile holds whole images (flowk_block_tail_tc); FLOWK_BLOCK_TAIL=0 keeps the chained gate, attention and gate launches
+# (A/B runs).
+BLOCK_TAIL = __import__("os").environ.get("FLOWK_BLOCK_TAIL", "1") != "0"
+
+
+def block_tail_supported(HW, C, heads, M):
+    """Shapes the conditioner routes to flowk_block_tail_tc: whole images per 128-row tile, head dims 24 / 32, the gate and
+    in_proj accumulators side by side in the 512 TMEM columns (5C <= 512), and at least two tiles.  A single-tile batch
+    (B = 2 at 8x8) keeps the three-launch route, as the conditioner's route test (tests/test_attention_inproj_fused.py)
+    specifies; the kernel takes that shape too and is not slower there (profiles/r8_block_tail_probe.txt)."""
+    if not (BLOCK_TAIL and heads >= 1 and C % heads == 0):
+        return False
+    return (HW <= 128 and 128 % HW == 0 and M % 128 == 0 and M >= 256 and C % 32 == 0 and 5 * C <= 512
+            and C // heads in (24, 32))
+
+
+def block_tail(c1_hi, c1_lo, gate, bias_g, x, ln1, pos, in_proj, attn_gate, bias_a, ln2, B, HW, C, heads, celu,
+               status=None, trace=None):
+    """c1_hi / c1_lo [B*HW, 2C] fp16 rows the block's gate multiplies, x [B*HW, C] the block input; gate / in_proj /
+    attn_gate = (w_hi, w_lo, acc_scale) fp16 weight operands (conv_weight_operand_f16), ln1 / ln2 = (gamma, beta), pos
+    [HW, C] -> (x2 [B*HW, C] fp32, out_hi, out_lo): concat_elu(x2) as an fp16 pair [B*HW, 2C] when `celu`, else x2 as a
+    pair [B*HW, C]."""
+    M = B * HW
+    # the kernel's tensor maps are built from B, HW and C: the tensors must have exactly these layouts
+    assert c1_hi.dtype == c1_lo.dtype == torch.float16 and c1_hi.shape == c1_lo.shape == (M, 2 * C)
+    assert c1_hi.is_contiguous() and c1_lo.is_contiguous()
+    for (w_hi, w_lo, _), rows, k in ((gate, 2 * C, 2 * C), (in_proj, 3 * C, C), (attn_gate, 2 * C, C)):
+        assert w_hi.dtype == w_lo.dtype == torch.float16 and w_hi.shape == w_lo.shape == (rows, (k + 63) // 64 * 64)
+        assert w_hi.is_contiguous() and w_lo.is_contiguous()
+    for t, shape in ((x, (M, C)), (pos, (HW, C)), (bias_g, (2 * C,)), (bias_a, (2 * C,)), (ln1[0], (C,)), (ln1[1], (C,)),
+                     (ln2[0], (C,)), (ln2[1], (C,))):
+        assert t.dtype == torch.float32 and tuple(t.shape) == shape and t.is_contiguous()
+    _lib.check_device(c1_hi, "block_tail")
+    x2 = torch.empty(M, C, device=x.device, dtype=torch.float32)
+    width = 2 * C if celu else C
+    hi = torch.empty(M, width, device=x.device, dtype=torch.float16)
+    lo = torch.empty_like(hi)
+    _lib.call("flowk_block_tail_tc", c1_hi.data_ptr(), c1_lo.data_ptr(), gate[0].data_ptr(), gate[1].data_ptr(),
+              float(gate[2]), bias_g.data_ptr(), x.data_ptr(), ln1[0].data_ptr(), ln1[1].data_ptr(), pos.data_ptr(),
+              in_proj[0].data_ptr(), in_proj[1].data_ptr(), float(in_proj[2]), attn_gate[0].data_ptr(),
+              attn_gate[1].data_ptr(), float(attn_gate[2]), bias_a.data_ptr(), ln2[0].data_ptr(), ln2[1].data_ptr(),
+              x2.data_ptr(), hi.data_ptr(), lo.data_ptr(), int(bool(celu)), B, HW, C, heads, _p(status), _p(trace),
+              _stream())
+    return x2, hi, lo

@@ -474,6 +474,25 @@ int flowk_attention_inproj_tc(const void* p_hi, const void* p_lo, const void* w_
                               void* out_hi, void* out_lo, int B, int HW, int C, int heads, int* status, long long* trace,
                               flowk_stream_t stream);
 int flowk_attention_inproj_tc_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes);
+/* The attention half of a ConvAttnBlock in one launch (csrc/block_tail_tc.cu), for feature maps whose images fit whole into
+ * a 128-row tile: gate GEMM -> GLU + bias + x -> LayerNorm(gamma1, beta1) = x1; in_proj of x1 + pos; softmax attention per
+ * image and head; attention-gate GEMM -> GLU + bias + x1 -> LayerNorm(gamma2, beta2) = x2.  x1, q, k, v and the attention
+ * output never leave the SM.  Inputs: c1_hi / c1_lo [B*HW, 2C] fp16 (the concat-ELU rows the gate multiplies), the fp16
+ * weight operands as flowk_pack_weight_f16 packs 1x1 weights (gate [2C, ceil64(2C)], in_proj [3C, ceil64(C)] with
+ * (k | v | q) rows, attention gate [2C, ceil64(C)]) with their acc_scale factors, fp32 biases [2C], x [B*HW, C],
+ * LayerNorm parameters [C] and the positional encoding pos [HW, C].  Outputs: x2 [B*HW, C] fp32 and out_hi / out_lo fp16,
+ * [B*HW, 2C] concat_elu(x2) when celu != 0, else [B*HW, C] x2.  Takes HW <= 128 with 128 % HW == 0, B*HW % 128 == 0,
+ * C a multiple of 32 with 5C <= 512 and C/heads in {24, 32}; FLOWK_ERR_SHAPE otherwise, FLOWK_ERR_ARG for a NULL input or
+ * output or a non-positive scale, FLOWK_ERR_ALIGN unless every pointer is 16-byte aligned.  `status` (device int, may be
+ * NULL) is set to 1 if an internal barrier wait timed out; `trace` (device long long[8], NULL in production) receives
+ * clock64 stamps of the first CTA: 0 start, 1 gate accumulator, 2 in_proj operand written, 3 in_proj accumulator, 4 first
+ * head's S, 5 attention done, 6 attention-gate accumulator, 7 end. */
+int flowk_block_tail_tc(const void* c1_hi, const void* c1_lo, const void* wg_hi, const void* wg_lo, float sc_g,
+                        const float* bias_g, const float* x, const float* gamma1, const float* beta1, const float* pos,
+                        const void* wi_hi, const void* wi_lo, float sc_i, const void* wa_hi, const void* wa_lo, float sc_a,
+                        const float* bias_a, const float* gamma2, const float* beta2, float* x2, void* out_hi,
+                        void* out_lo, int celu, int B, int HW, int C, int heads, int* status, long long* trace,
+                        flowk_stream_t stream);
 
 #ifdef __cplusplus
 }
