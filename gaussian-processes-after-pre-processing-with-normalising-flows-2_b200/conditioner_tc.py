@@ -10,7 +10,8 @@ in_conv -> 10 x ConvAttnBlock -> out_conv) as a chain of `flowk_conv_gemm` launc
                 G4 gate     attention output    -> LayerNorm(GLU + x1)         = x2, concat_elu(x2) (fp32 + operand)
 
 Every nonlinearity lives in a GEMM epilogue, so a block is 4 GEMM launches + attention; where a 128-row tile holds whole
-images (8x8 and 4x4 maps), G2 to G4 and the attention are one launch (tc.block_tail).  Weight-normalised,
+images (8x8 and 4x4 maps), G2 to G4 and the attention are one launch (tc.block_tail), and at 16x16 from B = 8 one launch of
+two-CTA clusters, one per image (tc.block_tail_pair).  Weight-normalised,
 re-laid-out, hi/lo-split weights are cached per parameter version.
 """
 import os
@@ -128,14 +129,16 @@ def mixlogcdf_nn_raw(nn_module, x_id, status=None):
         # G2: gate 1x1 -> GLU + x -> LayerNorm
         w_hi, w_lo, bias, sc = blk["gate"]
         has_attn = "in_proj" in blk
-        if has_attn and F16 and tc.block_tail_supported(HW, C, blk["heads"], M):
-            # G2, G3, the attention and G4 in one launch: x1, q, k, v and the attention output stay on chip
+        pair = has_attn and F16 and tc.block_tail_pair_supported(HW, C, blk["heads"], B)
+        if has_attn and F16 and (pair or tc.block_tail_supported(HW, C, blk["heads"], M)):
+            # G2, G3, the attention and G4 in one launch: x1, q, k, v and the attention output stay on chip (at 16x16 in a
+            # cluster of two CTAs per image)
             pos = nn_module.mid_convs[bi].attn._pos_enc(HW, C, dev).reshape(HW, C).contiguous()
             w3_hi, w3_lo, _, sc3 = blk["in_proj"]
             w4_hi, w4_lo, bias4, sc4 = blk["attn_gate"]
             x, nxt_hi, nxt_lo = tc.block_tail(c1_hi, c1_lo, (w_hi, w_lo, sc), bias, x, blk["ln1"], pos, (w3_hi, w3_lo, sc3),
                                               (w4_hi, w4_lo, sc4), bias4, blk["ln2"], B, HW, C, blk["heads"], not last,
-                                              status=status)
+                                              status=status, pair=pair)
             continue
         x1 = buf(M, C)
         if has_attn:

@@ -23,6 +23,21 @@
 //      written out row-contiguously.
 // Same numerics as the three launches it replaces: the two-term fp16 split with three products per GEMM, the chained gate's
 // GLU / LayerNorm epilogue and the one-wave attention kernel's softmax (csrc/tc_gemm.cu, csrc/attention_tc.cu).
+//
+// PAIR = true (flowk_block_tail_pair_tc): 16x16 maps, where an image's 256 rows span two tiles.  A cluster of two CTAs per
+// image, rank r owning image rows [128 r, 128 r + 128); phases 1-3, 5 and 6 are the per-CTA ones above (the positional
+// encoding rows offset by 128 r, no mask: all 256 keys of the image are valid).  Phase 4, per head:
+//   * after its drain a CTA also sends the head's K pair and V^T (32 KB, one cp.async.bulk shared::cta -> shared::cluster)
+//     into the peer's "remote" buffer, completing on the peer's rfull barrier;
+//   * S and P V run over two 128-key blocks, the CTA's own keys first (the first S never waits for the peer), then the
+//     peer's from the remote buffer; each block keeps its row maximum m_b and sum l_b, and the epilogue combines them
+//     exactly: O = sum_b O_b 2^(m_b - m) / sum_b l_b 2^(m_b - m) (the one-wave attention kernel's split-key softmax);
+//   * once the P V that read the remote buffer has retired, the CTA arrives on the peer's pempty barrier; a CTA waits
+//     there before its next drain (so its bulk copy of the previous head has been read) and before sending a head.
+//   TMEM: S [s, s + 128) and O_0, O_1 (32 columns each) after it, over the drained gate accumulator at C = 96.  Shared
+//   memory: the remote buffer lies over the ring stage the attention gate's second weight slice goes to; the producer
+//   loads that slice only after the last P V has retired (rfree barrier), the first slice goes to the other stage.
+//   All tcgen05 instructions stay cta_group::1.
 #include <cuda.h>
 #include "common.cuh"
 #include "umma.cuh"
@@ -37,6 +52,7 @@ constexpr int BT_SLICE = 128 * V2_ROW_B;        // one 32-channel slice of a 128
 constexpr int BT_DK = 32;                       // head dim padded to the MMA's K = 16 granule (one 64-byte row)
 constexpr int BT_VT_B = 2 * BT_DK * ROW_B;      // one 64-key block of V^T: [32 rows of hi | 32 rows of lo][128 B]
 constexpr int BT_QKV_B = 4 * BT_SLICE + 2 * BT_VT_B;   // one head's Q pair, K pair and V^T: 48 KB
+constexpr int BT_REM_B = 2 * BT_SLICE + 2 * BT_VT_B;   // PAIR: the peer's K pair and V^T of one head: 32 KB
 
 // elu(x) = x > 0 ? x : e^x - 1 and the logistic sigmoid, as the GEMM epilogues of csrc/tc_gemm.cu compute them
 __device__ __forceinline__ float bt_elu(float x) { return x > 0.f ? x : ex2_fast(x * kLog2e) - 1.f; }
@@ -61,13 +77,14 @@ struct BlockTailParams {
   int n_ip;                 // in_proj MMA N: 3C in one MMA, or two of 3C / 2 when 3C > 256
   int s_col;                // TMEM column of S / P; O follows at s_col + 128
   int qkv_off, r2_off, ring_off, stage_b, slab_off;   // shared-memory carve (bytes)
+  int rem_off, rem_alias;   // PAIR: the remote K / V^T buffer, and whether it lies over a ring stage
   int* status;
   long long* trace;         // optional device [8]: clock64 stamps of CTA 0 (profiling), NULL in production
 };
 
 __device__ __forceinline__ void bt_sync() { asm volatile("bar.sync 1, %0;" ::"n"(32 * BT_WARPS) : "memory"); }
 
-template <int NKB>          // C = 32 NKB channels
+template <int NKB, bool PAIR>   // C = 32 NKB channels; PAIR: two-CTA clusters over 256-row images
 __global__ void __launch_bounds__(BT_THREADS, 1)
 block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMap map_c1_hi,
                      const __grid_constant__ CUtensorMap map_c1_lo, const __grid_constant__ CUtensorMap map_wg_hi,
@@ -81,9 +98,11 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   __shared__ uint64_t bar_a, bar_full[2], bar_empty[2], bar_g, bar_i, bar_s, bar_o, bar_ag;
+  __shared__ uint64_t bar_rfull, bar_pempty, bar_rfree;   // PAIR: remote buffer filled / peer's buffer free / ring stage free
   __shared__ uint32_t tmem_slot;
   __shared__ int failed_flag;
   __shared__ float red[2][4][128];              // per-row partials of the four threads that share a row
+  __shared__ float own_ml[PAIR ? 2 : 1][128];   // PAIR: the own key block's row maximum and sum, per row
   volatile int* failed = &failed_flag;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -100,6 +119,9 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
     mbar_init(&bar_s, 1);
     mbar_init(&bar_o, 1);
     mbar_init(&bar_ag, 1);
+    mbar_init(&bar_rfull, 1);
+    mbar_init(&bar_pempty, 1);
+    mbar_init(&bar_rfree, 1);
     fence_barrier_init();
   }
   if (warp == 0) tmem_alloc(&tmem_slot, 512u);
@@ -116,6 +138,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
+  if (PAIR) cluster_sync_all();                 // the peer's barriers are initialised before anything signals them
   const uint32_t tmem = tmem_slot;
   const bool tracing = p.trace && blockIdx.x == 0 && threadIdx.x == 0;
   griddep_launch();
@@ -133,6 +156,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
       for (int g = 0; g < NSL; ++g) {
         const int st = g & 1;
         mbar_wait(&bar_empty[st], (uint32_t)(((g >> 1) & 1) ^ 1), failed);
+        if (PAIR && g == NG + NKB + 1 && p.rem_alias) mbar_wait(&bar_rfree, 0, failed);  // the remote buffer's stage
         uint8_t* w = smem + p.ring_off + st * p.stage_b;
         if (g < NG || g >= NG + NKB) {          // gate / attention gate: 2C rows, one box each
           const bool gate = g < NG;
@@ -263,7 +287,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
       float v[NKB][8];
       const float psum = glu(v, p.bias_g, p.sc_g, slab, PITCH);   // x1 then replaces x in the slab, row by row
       layer_norm(v, psum, p.gamma1, p.beta1);
-      const float* pr = p.pos + (size_t)(row % p.HW) * C;   // 128 % HW == 0: tile row r is position r % HW
+      const float* pr = p.pos + (size_t)((tile * 128 + row) % p.HW) * C;   // the row's position in its image
 #pragma unroll
       for (int i = 0; i < NKB; ++i) {
         const int j = i * 32 + quarter * 8;
@@ -288,6 +312,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
     if (warp == 0) gemm(NG, NKB, r1, 3 * C, 3 * C / p.n_ip, (uint32_t)(2 * C), &bar_i);
     mbar_wait(&bar_i, 0, failed);
     tc_fence_after();
+    if (PAIR && threadIdx.x == 0) mbar_arrive_cluster(mapa_rank(&bar_pempty, cluster_ctarank() ^ 1u));   // in_proj has read the ring stage
     if (tracing) p.trace[3] = clock64();
 
     // ---- 4. attention, one head at a time ----------------------------------------------------------------------------------
@@ -296,12 +321,15 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
       uint8_t* k_t = q_t + 2 * BT_SLICE;
       uint8_t* v_t = q_t + 4 * BT_SLICE;        // 2 blocks of 64 keys, SWIZZLE_128B
       const int D = p.D, chunks = D >> 3;
-      const uint32_t ip = (uint32_t)(2 * C), sc_col = (uint32_t)p.s_col, o_col = sc_col + 128u;
-      const int klo = row / p.HW * p.HW, khi = klo + p.HW;  // the keys of this row's image
+      const uint32_t ip = (uint32_t)(2 * C), sc_col = (uint32_t)p.s_col, o_col = sc_col + 128u;  // PAIR: O_1 at o_col + 32
+      const int klo = PAIR ? 0 : row / p.HW * p.HW, khi = PAIR ? 128 : klo + p.HW;  // the keys of this row's image
       const int k0 = quarter * 32;
       const bool live = k0 < khi && k0 + 32 > klo;          // warp-uniform: a warp's 32 rows meet the same quarters
+      uint8_t* rem = smem + p.rem_off;          // PAIR: the peer's K pair and V^T of the head, laid out as k_t, v_t
+      constexpr int NB = PAIR ? 2 : 1;          // key blocks per head: own keys, then (PAIR) the peer's
 #pragma unroll 1
       for (int h = 0; h < p.heads; ++h) {
+        if (PAIR) mbar_wait(&bar_pempty, (uint32_t)(h & 1), failed);   // the peer is done with our previous head's copy
         // 4a. drain: thread (row, quarter) takes dims [8 quarter, 8 quarter + 8) of the head's k, v and q; dims >= D are zero
         {
           const uint32_t col = lane_addr + ip + (uint32_t)(h * D + quarter * 8);
@@ -347,13 +375,18 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
         fence_proxy_async();
         tc_fence_before();
         bt_sync();
+        if (PAIR && warp == 1 && lane == 0) {   // K pair and V^T (contiguous from k_t) -> the peer's remote buffer
+          mbar_expect_tx(&bar_rfull, (uint32_t)BT_REM_B);   // ... and the peer's into ours
+          const uint32_t peer = cluster_ctarank() ^ 1u;
+          bulk_copy_to_peer(mapa_rank(rem, peer), k_t, (uint32_t)BT_REM_B, mapa_rank(&bar_rfull, peer));
+        }
 
-        // 4b. S = Q K^T into TMEM [s_col, s_col + 128)
-        if (warp == 0) {
+        // 4b. S = Q K^T into TMEM [s_col, s_col + 128) (warp 0; `kt` = the key block's K pair)
+        auto issue_s = [&](const uint8_t* kt) {
           tc_fence_after();
           const uint32_t idesc = make_idesc_f16(128);
           const uint64_t dq_hi = make_smem_desc_sw64(smem_u32(q_t)), dq_lo = make_smem_desc_sw64(smem_u32(q_t + BT_SLICE));
-          const uint64_t dk_hi = make_smem_desc_sw64(smem_u32(k_t)), dk_lo = make_smem_desc_sw64(smem_u32(k_t + BT_SLICE));
+          const uint64_t dk_hi = make_smem_desc_sw64(smem_u32(kt)), dk_lo = make_smem_desc_sw64(smem_u32(kt + BT_SLICE));
 #pragma unroll
           for (int ks = 0; ks < BT_DK / 16; ++ks) {
             const uint64_t ko = (uint64_t)(ks * 2);
@@ -362,83 +395,117 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
             umma_elect<true>(tmem + sc_col, dq_hi + ko, dk_lo + ko, idesc, 1u, leader);
           }
           umma_commit_elect(&bar_s, leader);
-        }
-        mbar_wait(&bar_s, (uint32_t)(h & 1), failed);
-        tc_fence_after();
-        if (tracing && h == 0) p.trace[4] = clock64();
-
-        // 4c. masked row maximum over this thread's 32 keys
-        float s[32];
-        float mx = -INFINITY;
-        if (live) {
-          tmem_ld32(lane_addr + sc_col + (uint32_t)k0, s);
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            const int key = k0 + i;
-            s[i] = (key >= klo && key < khi) ? s[i] : -INFINITY;
-            mx = fmaxf(mx, s[i]);
-          }
-        }
-        red[0][quarter][row] = mx;
-        tc_fence_before();                      // every load of S is complete before anyone writes P over it
-        bt_sync();
-        tc_fence_after();
-        mx = fmaxf(fmaxf(red[0][0][row], red[0][1][row]), fmaxf(red[0][2][row], red[0][3][row]));
-
-        // 4d. p = 2^(s - max) (0 for other images' keys) as packed fp16 (hi, lo): keys (2i, 2i + 1) in column i of each half
-        float sum = 0.f;
-#pragma unroll
-        for (int half = 0; half < 2; ++half) {
-          uint32_t ph[8], pl[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            float e0 = 0.f, e1 = 0.f;
-            if (live) {
-              e0 = ex2_fast(s[16 * half + 2 * i] - mx);       // masked keys: 2^-inf = 0
-              e1 = ex2_fast(s[16 * half + 2 * i + 1] - mx);
-            }
-            sum += e0 + e1;
-            ph[i] = pack_h2(e0, e1);
-            float a0, a1;
-            unpack_h2(ph[i], a0, a1);
-            pl[i] = pack_h2(e0 - a0, e1 - a1);
-          }
-          tmem_st8u(lane_addr + sc_col + (uint32_t)(quarter * 16 + half * 8), ph);
-          tmem_st8u(lane_addr + sc_col + (uint32_t)(64 + quarter * 16 + half * 8), pl);
-        }
-        red[1][quarter][row] = sum;
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-        tc_fence_before();
-        bt_sync();
-        const float l = (red[1][0][row] + red[1][1][row]) + (red[1][2][row] + red[1][3][row]);
-
-        // 4e. O = P_hi V_hi + P_lo V_hi + P_hi V_lo (N = 32, K = 128 keys) into TMEM [o_col, o_col + 32)
-        if (warp == 0) {
+        };
+        if (warp == 0) issue_s(k_t);
+        float mx = 0.f, l = 0.f;                // the last key block's row maximum and sum
+#pragma unroll 1
+        for (int kb = 0; kb < NB; ++kb) {
+          const int it = h * NB + kb;             // key blocks done: phase of bar_s / bar_o
+          mbar_wait(&bar_s, (uint32_t)(it & 1), failed);
           tc_fence_after();
-          const uint32_t idesc = make_idesc_f16(BT_DK);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) {         // 16 keys per step: 8 packed columns of P, 32 bytes of a V^T row
-            const int key = j * 16;
-            const uint8_t* vb = v_t + (key >> 6) * BT_VT_B;
-            const uint64_t ko = (uint64_t)(((key & 63) >> 4) * 2);
-            const uint64_t dv_hi = make_smem_desc(smem_u32(vb)) + ko, dv_lo = make_smem_desc(smem_u32(vb + BT_DK * ROW_B)) + ko;
-            const uint32_t a_hi = tmem + sc_col + (uint32_t)(j * 8), a_lo = tmem + sc_col + (uint32_t)(64 + j * 8);
-            umma_f16_ts_elect(tmem + o_col, a_hi, dv_hi, idesc, j == 0 ? 0u : 1u, leader);
-            umma_f16_ts_elect(tmem + o_col, a_lo, dv_hi, idesc, 1u, leader);
-            umma_f16_ts_elect(tmem + o_col, a_hi, dv_lo, idesc, 1u, leader);
-          }
-          umma_commit_elect(&bar_o, leader);
-        }
-        mbar_wait(&bar_o, (uint32_t)(h & 1), failed);
-        tc_fence_after();
+          if (tracing && it == 0) p.trace[4] = clock64();
 
-        // 4f. O / rowsum -> columns [h D, h D + D) of the attention gate's operand pair
+          // 4c. masked row maximum over this thread's 32 keys
+          float s[32];
+          mx = -INFINITY;
+          if (live) {
+            tmem_ld32(lane_addr + sc_col + (uint32_t)k0, s);
+#pragma unroll
+            for (int i = 0; i < 32; ++i) {
+              const int key = k0 + i;
+              if (!PAIR) s[i] = (key >= klo && key < khi) ? s[i] : -INFINITY;
+              mx = fmaxf(mx, s[i]);
+            }
+          }
+          red[0][quarter][row] = mx;
+          tc_fence_before();                      // every load of S is complete before anyone writes P over it
+          bt_sync();
+          tc_fence_after();
+          mx = fmaxf(fmaxf(red[0][0][row], red[0][1][row]), fmaxf(red[0][2][row], red[0][3][row]));
+
+          // 4d. p = 2^(s - max) (0 for other images' keys) as packed fp16 (hi, lo): keys (2i, 2i + 1) in column i of each half
+          float sum = 0.f;
+#pragma unroll
+          for (int half = 0; half < 2; ++half) {
+            uint32_t ph[8], pl[8];
+#pragma unroll
+            for (int i = 0; i < 8; ++i) {
+              float e0 = 0.f, e1 = 0.f;
+              if (live) {
+                e0 = ex2_fast(s[16 * half + 2 * i] - mx);       // masked keys: 2^-inf = 0
+                e1 = ex2_fast(s[16 * half + 2 * i + 1] - mx);
+              }
+              sum += e0 + e1;
+              ph[i] = pack_h2(e0, e1);
+              float a0, a1;
+              unpack_h2(ph[i], a0, a1);
+              pl[i] = pack_h2(e0 - a0, e1 - a1);
+            }
+            tmem_st8u(lane_addr + sc_col + (uint32_t)(quarter * 16 + half * 8), ph);
+            tmem_st8u(lane_addr + sc_col + (uint32_t)(64 + quarter * 16 + half * 8), pl);
+          }
+          red[1][quarter][row] = sum;
+          asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+          tc_fence_before();
+          bt_sync();
+          l = (red[1][0][row] + red[1][1][row]) + (red[1][2][row] + red[1][3][row]);
+
+          // 4e. O_kb = P_hi V_hi + P_lo V_hi + P_hi V_lo (N = 32, K = 128 keys) into TMEM [o_col + 32 kb, o_col + 32 kb + 32)
+          if (warp == 0) {
+            tc_fence_after();
+            const uint32_t idesc = make_idesc_f16(BT_DK), od = tmem + o_col + (uint32_t)(kb * BT_DK);
+            const uint8_t* vt = kb ? rem + 2 * BT_SLICE : v_t;
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {         // 16 keys per step: 8 packed columns of P, 32 bytes of a V^T row
+              const int key = j * 16;
+              const uint8_t* vb = vt + (key >> 6) * BT_VT_B;
+              const uint64_t ko = (uint64_t)(((key & 63) >> 4) * 2);
+              const uint64_t dv_hi = make_smem_desc(smem_u32(vb)) + ko, dv_lo = make_smem_desc(smem_u32(vb + BT_DK * ROW_B)) + ko;
+              const uint32_t a_hi = tmem + sc_col + (uint32_t)(j * 8), a_lo = tmem + sc_col + (uint32_t)(64 + j * 8);
+              umma_f16_ts_elect(od, a_hi, dv_hi, idesc, j == 0 ? 0u : 1u, leader);
+              umma_f16_ts_elect(od, a_lo, dv_hi, idesc, 1u, leader);
+              umma_f16_ts_elect(od, a_hi, dv_lo, idesc, 1u, leader);
+            }
+            umma_commit_elect(&bar_o, leader);
+            if (PAIR && kb == 0) {                // the peer's keys into the same S columns once P_0 has been read
+              mbar_wait(&bar_o, (uint32_t)(it & 1), failed);
+              mbar_wait(&bar_rfull, (uint32_t)(h & 1), failed);
+              issue_s(rem);
+            }
+            if (PAIR && kb == 1 && h == p.heads - 1) umma_commit_elect(&bar_rfree, leader);   // the remote buffer is read
+          }
+          if (PAIR && kb == 0 && quarter == 0) {  // read after the next block's barriers
+            own_ml[0][row] = mx;
+            own_ml[PAIR ? 1 : 0][row] = l;
+          }
+        }
+        mbar_wait(&bar_o, (uint32_t)((h * NB + NB - 1) & 1), failed);
+        tc_fence_after();
+        if (PAIR && h + 1 < p.heads && threadIdx.x == 0) mbar_arrive_cluster(mapa_rank(&bar_pempty, cluster_ctarank() ^ 1u));
+
+        // 4f. O / rowsum -> columns [h D, h D + D) of the attention gate's operand pair; PAIR: the exact combination of the
+        // two key blocks
+        float w0 = 1.0f / l, w1 = 0.f;
+        if (PAIR) {
+          const float m0 = own_ml[0][row], l0 = own_ml[PAIR ? 1 : 0][row], m = fmaxf(m0, mx);
+          w0 = ex2_fast(m0 - m);
+          w1 = ex2_fast(mx - m);
+          const float inv = 1.0f / (l0 * w0 + l * w1);
+          w0 *= inv;
+          w1 *= inv;
+        }
         if (quarter < chunks) {
           float o[8];
           tmem_ld8(lane_addr + o_col + (uint32_t)(quarter * 8), o);
-          const float inv = 1.0f / l;
+          if (PAIR) {
+            float o1[8];
+            tmem_ld8(lane_addr + o_col + (uint32_t)(BT_DK + quarter * 8), o1);
 #pragma unroll
-          for (int e = 0; e < 8; ++e) o[e] *= inv;
+            for (int e = 0; e < 8; ++e) o[e] = o[e] * w0 + o1[e] * w1;
+          } else {
+#pragma unroll
+            for (int e = 0; e < 8; ++e) o[e] *= w0;
+          }
           uint4 hi, lo;
           cvt8(o, hi, lo);
           const int c = h * D + quarter * 8, kb = c >> 5, ch = (c & 31) >> 3;
@@ -504,6 +571,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
   }
   tc_fence_before();
   __syncthreads();
+  if (PAIR) cluster_sync_all();                 // neither CTA retires while the peer may still signal or copy into it
   if (tracing) p.trace[7] = clock64();
   if (warp == 0) tmem_dealloc(tmem, 512u);
   if (threadIdx.x == 0 && failed_flag && p.status) *p.status = 1;
@@ -517,9 +585,11 @@ using namespace flowk::tc;
 
 namespace {
 // Shapes the kernel takes and its shared-memory carve: [in_proj operand pair | one head's Q, K, V^T] [attention output pair]
-// [weight ring: 2 stages] [x1 slab]; the c1 tile of the gate GEMM lies over the first two regions.
-bool block_tail_plan(long long M, int HW, int C, int heads, BlockTailParams& p, size_t& smem) {
-  if (HW < 1 || HW > 128 || 128 % HW || M % 128) return false;
+// [weight ring: 2 stages] [x1 slab]; the c1 tile of the gate GEMM lies over the first two regions.  PAIR (HW = 256, two
+// tiles per image): the remote K / V^T buffer lies over the ring stage of the attention gate's second weight slice when a
+// stage holds it (C = 96), else after the slab.
+bool block_tail_plan(long long M, int HW, int C, int heads, bool pair, BlockTailParams& p, size_t& smem) {
+  if (pair ? HW != 256 || M % 256 : HW < 1 || HW > 128 || 128 % HW || M % 128) return false;
   if (C < 32 || C % 32 || 5 * C > 512 || heads < 1 || C % heads) return false;  // TMEM: gate [0, 2C) + in_proj [2C, 5C)
   const int D = C / heads;
   if (D != 24 && D != 32) return false;
@@ -529,7 +599,8 @@ bool block_tail_plan(long long M, int HW, int C, int heads, BlockTailParams& p, 
   p.D = D;
   p.qscale = 1.4426950408889634f / sqrtf((float)D);
   p.n_ip = 3 * C <= 256 ? 3 * C : 3 * C / 2;
-  p.s_col = 5 * C + 160 <= 512 ? 5 * C : 0;      // S / P and O after in_proj, or over the drained gate accumulator
+  // S / P and O (PAIR: O_0, O_1) after in_proj, or over the drained gate accumulator
+  p.s_col = 5 * C + 128 + (pair ? 2 : 1) * BT_DK <= 512 ? 5 * C : 0;
   const int r1 = 2 * nkb * BT_SLICE > BT_QKV_B ? 2 * nkb * BT_SLICE : BT_QKV_B;
   p.qkv_off = 0;
   p.r2_off = r1;
@@ -537,33 +608,37 @@ bool block_tail_plan(long long M, int HW, int C, int heads, BlockTailParams& p, 
   if (p.ring_off < 2 * nkb * 2 * BT_SLICE) return false;   // the c1 tile must fit below the ring
   p.stage_b = 2 * 3 * C * V2_ROW_B;
   p.slab_off = p.ring_off + 2 * p.stage_b;
-  smem = (size_t)p.slab_off + (size_t)128 * (C + 4) * 4 + 1024;
+  const int slab_end = p.slab_off + 128 * (C + 4) * 4;
+  p.rem_alias = pair && p.stage_b >= BT_REM_B;
+  p.rem_off = 0;
+  if (p.rem_alias) p.rem_off = p.ring_off + ((3 * nkb + 1) & 1) * p.stage_b;   // the stage of weight slice 3 nkb + 1
+  else if (pair) p.rem_off = (slab_end + 1023) / 1024 * 1024;
+  smem = (size_t)(pair && !p.rem_alias ? p.rem_off + BT_REM_B : slab_end) + 1024;
   return smem + 8 * 1024 <= 227 * 1024;          // (+ the kernel's static shared memory)
 }
 
-template <int NKB>
+template <int NKB, bool PAIR>
 int block_tail_launch(const BlockTailParams& p, int tiles, size_t smem, const CUtensorMap* maps, cudaStream_t stream) {
   static size_t smem_set = 0;
   if (smem > smem_set) {
-    FLOWK_CUDA_OK(cudaFuncSetAttribute(block_tail_tc_kernel<NKB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    FLOWK_CUDA_OK(cudaFuncSetAttribute(block_tail_tc_kernel<NKB, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
     smem_set = smem;
   }
-  FLOWK_CUDA_OK(launch_pdl(block_tail_tc_kernel<NKB>, dim3(tiles), dim3(BT_THREADS), smem, stream, p, maps[0], maps[1],
-                           maps[2], maps[3], maps[4], maps[5], maps[6], maps[7]));
+  FLOWK_CUDA_OK(launch_pdl_cluster(block_tail_tc_kernel<NKB, PAIR>, dim3(tiles), dim3(BT_THREADS), smem, stream,
+                                   PAIR ? 2 : 1, p, maps[0], maps[1], maps[2], maps[3], maps[4], maps[5], maps[6], maps[7]));
   return launch_status();
 }
-}  // namespace
 
-extern "C" int flowk_block_tail_tc(const void* c1_hi, const void* c1_lo, const void* wg_hi, const void* wg_lo, float sc_g,
-                                   const float* bias_g, const float* x, const float* gamma1, const float* beta1,
-                                   const float* pos, const void* wi_hi, const void* wi_lo, float sc_i, const void* wa_hi,
-                                   const void* wa_lo, float sc_a, const float* bias_a, const float* gamma2,
-                                   const float* beta2, float* x2, void* out_hi, void* out_lo, int celu, int B, int HW, int C,
-                                   int heads, int* status, long long* trace, flowk_stream_t stream) {
+int block_tail_entry(bool pair, const void* c1_hi, const void* c1_lo, const void* wg_hi, const void* wg_lo, float sc_g,
+                     const float* bias_g, const float* x, const float* gamma1, const float* beta1, const float* pos,
+                     const void* wi_hi, const void* wi_lo, float sc_i, const void* wa_hi, const void* wa_lo, float sc_a,
+                     const float* bias_a, const float* gamma2, const float* beta2, float* x2, void* out_hi, void* out_lo,
+                     int celu, int B, int HW, int C, int heads, int* status, long long* trace, flowk_stream_t stream) {
   BlockTailParams p{};
   size_t smem = 0;
   const long long M = (long long)B * HW;
-  if (B < 0 || !block_tail_plan(M, HW, C, heads, p, smem)) return FLOWK_ERR_SHAPE;
+  if (B < 0 || !block_tail_plan(M, HW, C, heads, pair, p, smem)) return FLOWK_ERR_SHAPE;
   if (B == 0) return FLOWK_OK;
   if (M > 0x7fffffffLL) return FLOWK_ERR_SHAPE;
   const void* ptrs[] = {c1_hi, c1_lo, wg_hi, wg_lo, bias_g, x, gamma1, beta1, pos, wi_hi, wi_lo, wa_hi, wa_lo, bias_a,
@@ -598,9 +673,36 @@ extern "C" int flowk_block_tail_tc(const void* c1_hi, const void* c1_lo, const v
       !make_map_sw64(&maps[6], wa_hi, 2LL * C, k1, 2 * C) || !make_map_sw64(&maps[7], wa_lo, 2LL * C, k1, 2 * C))
     return FLOWK_ERR_ARG;
   const int tiles = (int)(M / 128);
-  switch (C / 32) {
-    case 1: return block_tail_launch<1>(p, tiles, smem, maps, stream);
-    case 2: return block_tail_launch<2>(p, tiles, smem, maps, stream);
-    default: return block_tail_launch<3>(p, tiles, smem, maps, stream);
+  switch (C / 32 + (pair ? 3 : 0)) {
+    case 1: return block_tail_launch<1, false>(p, tiles, smem, maps, stream);
+    case 2: return block_tail_launch<2, false>(p, tiles, smem, maps, stream);
+    case 3: return block_tail_launch<3, false>(p, tiles, smem, maps, stream);
+    case 4: return block_tail_launch<1, true>(p, tiles, smem, maps, stream);
+    case 5: return block_tail_launch<2, true>(p, tiles, smem, maps, stream);
+    default: return block_tail_launch<3, true>(p, tiles, smem, maps, stream);
   }
+}
+}  // namespace
+
+extern "C" int flowk_block_tail_tc(const void* c1_hi, const void* c1_lo, const void* wg_hi, const void* wg_lo, float sc_g,
+                                   const float* bias_g, const float* x, const float* gamma1, const float* beta1,
+                                   const float* pos, const void* wi_hi, const void* wi_lo, float sc_i, const void* wa_hi,
+                                   const void* wa_lo, float sc_a, const float* bias_a, const float* gamma2,
+                                   const float* beta2, float* x2, void* out_hi, void* out_lo, int celu, int B, int HW, int C,
+                                   int heads, int* status, long long* trace, flowk_stream_t stream) {
+  return block_tail_entry(false, c1_hi, c1_lo, wg_hi, wg_lo, sc_g, bias_g, x, gamma1, beta1, pos, wi_hi, wi_lo, sc_i, wa_hi,
+                          wa_lo, sc_a, bias_a, gamma2, beta2, x2, out_hi, out_lo, celu, B, HW, C, heads, status, trace,
+                          stream);
+}
+
+extern "C" int flowk_block_tail_pair_tc(const void* c1_hi, const void* c1_lo, const void* wg_hi, const void* wg_lo,
+                                        float sc_g, const float* bias_g, const float* x, const float* gamma1,
+                                        const float* beta1, const float* pos, const void* wi_hi, const void* wi_lo,
+                                        float sc_i, const void* wa_hi, const void* wa_lo, float sc_a, const float* bias_a,
+                                        const float* gamma2, const float* beta2, float* x2, void* out_hi, void* out_lo,
+                                        int celu, int B, int HW, int C, int heads, int* status, long long* trace,
+                                        flowk_stream_t stream) {
+  return block_tail_entry(true, c1_hi, c1_lo, wg_hi, wg_lo, sc_g, bias_g, x, gamma1, beta1, pos, wi_hi, wi_lo, sc_i, wa_hi,
+                          wa_lo, sc_a, bias_a, gamma2, beta2, x2, out_hi, out_lo, celu, B, HW, C, heads, status, trace,
+                          stream);
 }

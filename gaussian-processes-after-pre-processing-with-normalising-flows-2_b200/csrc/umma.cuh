@@ -183,6 +183,17 @@ __device__ __forceinline__ uint32_t mapa_rank(const void* bar, uint32_t rank) {
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(bar)), "r"(rank));
   return r;
 }
+// `bytes` (a multiple of 16) from this CTA's shared memory to the shared::cluster address `dst` of another CTA of the
+// cluster, completing as transaction bytes on the barrier at shared::cluster address `bar` (in the destination CTA)
+__device__ __forceinline__ void bulk_copy_to_peer(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
+  asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+               ::"r"(dst), "r"(smem_u32(src)), "r"(bytes), "r"(bar)
+               : "memory");
+}
+// one arrival on the barrier at shared::cluster address `bar` (possibly in another CTA of the cluster)
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t bar) {
+  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar) : "memory");
+}
 __device__ __forceinline__ void tma_load_4d_pair(void* smem, const CUtensorMap* map, uint32_t bar_cluster, int c0, int c1,
                                                  int c2, int c3) {
   asm volatile(

@@ -251,12 +251,27 @@ def block_tail_supported(HW, C, heads, M):
             and C // heads in (24, 32))
 
 
+# The same block tail at 16x16 (an image spans two 128-row tiles) as one launch of two-CTA clusters, one per image
+# (flowk_block_tail_pair_tc); FLOWK_BLOCK_TAIL_PAIR=0 keeps the gate GEMM + fused in_proj attention + gate launches (A/B runs).
+BLOCK_TAIL_PAIR = __import__("os").environ.get("FLOWK_BLOCK_TAIL_PAIR", "1") != "0"
+
+
+def block_tail_pair_supported(HW, C, heads, B):
+    """Shapes the conditioner routes to flowk_block_tail_pair_tc: 16x16 maps (HW = 256, two tiles per image), head dims 24 /
+    32, 5C <= 512 TMEM columns, and B >= 8.  The batch rule is a routing contract: smaller batches (B = 2 and 4 at level 1)
+    keep flowk_attention_inproj_tc, as the conditioner's route tests (tests/test_attention_inproj_fused.py,
+    tests/test_block_tail_tc.py) specify; the kernel itself takes any B >= 1."""
+    if not (BLOCK_TAIL_PAIR and heads >= 1 and C % heads == 0):
+        return False
+    return HW == 256 and B >= 8 and C % 32 == 0 and 5 * C <= 512 and C // heads in (24, 32)
+
+
 def block_tail(c1_hi, c1_lo, gate, bias_g, x, ln1, pos, in_proj, attn_gate, bias_a, ln2, B, HW, C, heads, celu,
-               status=None, trace=None):
+               status=None, trace=None, pair=False):
     """c1_hi / c1_lo [B*HW, 2C] fp16 rows the block's gate multiplies, x [B*HW, C] the block input; gate / in_proj /
     attn_gate = (w_hi, w_lo, acc_scale) fp16 weight operands (conv_weight_operand_f16), ln1 / ln2 = (gamma, beta), pos
     [HW, C] -> (x2 [B*HW, C] fp32, out_hi, out_lo): concat_elu(x2) as an fp16 pair [B*HW, 2C] when `celu`, else x2 as a
-    pair [B*HW, C]."""
+    pair [B*HW, C].  `pair` launches flowk_block_tail_pair_tc (HW = 256) instead of flowk_block_tail_tc."""
     M = B * HW
     # the kernel's tensor maps are built from B, HW and C: the tensors must have exactly these layouts
     assert c1_hi.dtype == c1_lo.dtype == torch.float16 and c1_hi.shape == c1_lo.shape == (M, 2 * C)
@@ -272,10 +287,17 @@ def block_tail(c1_hi, c1_lo, gate, bias_g, x, ln1, pos, in_proj, attn_gate, bias
     width = 2 * C if celu else C
     hi = torch.empty(M, width, device=x.device, dtype=torch.float16)
     lo = torch.empty_like(hi)
-    _lib.call("flowk_block_tail_tc", c1_hi.data_ptr(), c1_lo.data_ptr(), gate[0].data_ptr(), gate[1].data_ptr(),
+    _lib.call("flowk_block_tail_pair_tc" if pair else "flowk_block_tail_tc", c1_hi.data_ptr(), c1_lo.data_ptr(), gate[0].data_ptr(), gate[1].data_ptr(),
               float(gate[2]), bias_g.data_ptr(), x.data_ptr(), ln1[0].data_ptr(), ln1[1].data_ptr(), pos.data_ptr(),
               in_proj[0].data_ptr(), in_proj[1].data_ptr(), float(in_proj[2]), attn_gate[0].data_ptr(),
               attn_gate[1].data_ptr(), float(attn_gate[2]), bias_a.data_ptr(), ln2[0].data_ptr(), ln2[1].data_ptr(),
               x2.data_ptr(), hi.data_ptr(), lo.data_ptr(), int(bool(celu)), B, HW, C, heads, _p(status), _p(trace),
               _stream())
     return x2, hi, lo
+
+
+def block_tail_pair(c1_hi, c1_lo, gate, bias_g, x, ln1, pos, in_proj, attn_gate, bias_a, ln2, B, HW, C, heads, celu,
+                    status=None, trace=None):
+    """block_tail for 16x16 maps (HW = 256): one cluster of two CTAs per image (flowk_block_tail_pair_tc)."""
+    return block_tail(c1_hi, c1_lo, gate, bias_g, x, ln1, pos, in_proj, attn_gate, bias_a, ln2, B, HW, C, heads, celu,
+                      status=status, trace=trace, pair=True)

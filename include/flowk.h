@@ -493,6 +493,19 @@ int flowk_block_tail_tc(const void* c1_hi, const void* c1_lo, const void* wg_hi,
                         const float* bias_a, const float* gamma2, const float* beta2, float* x2, void* out_hi,
                         void* out_lo, int celu, int B, int HW, int C, int heads, int* status, long long* trace,
                         flowk_stream_t stream);
+/* The same block tail for 16x16 maps (HW = 256), where an image spans two 128-row tiles: one cluster of two CTAs per image,
+ * each CTA owning 128 of its rows, exchanging each head's K and V through distributed shared memory so that every row
+ * attends over all 256 keys of its image.  Same arguments, outputs, status and error codes as flowk_block_tail_tc; takes
+ * HW = 256, any B >= 0 (B = 0 returns FLOWK_OK), C a multiple of 32 with 5C <= 512 and C/heads in {24, 32}; FLOWK_ERR_SHAPE
+ * otherwise.  `trace` (device long long[8], NULL in production) receives clock64 stamps of the first CTA (rank 0 of image
+ * 0): 0 start, 1 gate accumulator, 2 in_proj operand written, 3 in_proj accumulator, 4 first head's S over its own keys,
+ * 5 attention done, 6 attention-gate accumulator, 7 end (after the cluster's closing barrier). */
+int flowk_block_tail_pair_tc(const void* c1_hi, const void* c1_lo, const void* wg_hi, const void* wg_lo, float sc_g,
+                             const float* bias_g, const float* x, const float* gamma1, const float* beta1, const float* pos,
+                             const void* wi_hi, const void* wi_lo, float sc_i, const void* wa_hi, const void* wa_lo,
+                             float sc_a, const float* bias_a, const float* gamma2, const float* beta2, float* x2,
+                             void* out_hi, void* out_lo, int celu, int B, int HW, int C, int heads, int* status,
+                             long long* trace, flowk_stream_t stream);
 
 #ifdef __cplusplus
 }
