@@ -29,15 +29,18 @@
 // encoding rows offset by 128 r, no mask: all 256 keys of the image are valid).  Phase 4, per head:
 //   * after its drain a CTA also sends the head's K pair and V^T (32 KB, one cp.async.bulk shared::cta -> shared::cluster)
 //     into the peer's "remote" buffer, completing on the peer's rfull barrier;
-//   * S and P V run over two 128-key blocks, the CTA's own keys first (the first S never waits for the peer), then the
-//     peer's from the remote buffer; each block keeps its row maximum m_b and sum l_b, and the epilogue combines them
-//     exactly: O = sum_b O_b 2^(m_b - m) / sum_b l_b 2^(m_b - m) (the one-wave attention kernel's split-key softmax);
+//   * S and P V run over four 64-key blocks, the CTA's own keys 0-63 and 64-127 first (the first S never waits for the
+//     peer), then the peer's from the remote buffer.  A dedicated MMA warp keeps two S / P buffers in flight: S_{b+2} is
+//     issued into block b's buffer as soon as P_b V has retired, so the softmax of block b runs under P_{b-1} V and
+//     S_{b+1}.  Each block has its own row maximum m_b; the compute threads fold O_b into registers as it retires with a
+//     running maximum, o = o 2^(m_old - m) + O_b 2^(m_b - m) (the split-key combination of the one-wave attention kernel,
+//     applied block by block), which frees O_b's TMEM for P_{b+2} V;
 //   * once the P V that read the remote buffer has retired, the CTA arrives on the peer's pempty barrier; a CTA waits
 //     there before its next drain (so its bulk copy of the previous head has been read) and before sending a head.
-//   TMEM: S [s, s + 128) and O_0, O_1 (32 columns each) after it, over the drained gate accumulator at C = 96.  Shared
-//   memory: the remote buffer lies over the ring stage the attention gate's second weight slice goes to; the producer
-//   loads that slice only after the last P V has retired (rfree barrier), the first slice goes to the other stage.
-//   All tcgen05 instructions stay cta_group::1.
+//   TMEM: two S / P buffers [s, s + 64), [s + 64, s + 128) and two O buffers of 32 columns after them, over the drained
+//   gate accumulator at C = 96.  Shared memory: the remote buffer lies over the ring stage the attention gate's second
+//   weight slice goes to; the producer loads that slice only after the last P V has retired (rfree barrier), the first
+//   slice goes to the other stage.  All tcgen05 instructions stay cta_group::1.
 #include <cuda.h>
 #include "common.cuh"
 #include "umma.cuh"
@@ -47,7 +50,8 @@ namespace flowk {
 namespace tc {
 
 constexpr int BT_WARPS = 16;                    // compute warps: 4 per TMEM lane group, a quarter of each row's columns each
-constexpr int BT_THREADS = 32 * BT_WARPS + 32;  // + one TMA producer warp
+// + one TMA producer warp, and (PAIR) one warp that issues the attention's MMAs
+constexpr int bt_threads(bool pair) { return 32 * BT_WARPS + (pair ? 64 : 32); }
 constexpr int BT_SLICE = 128 * V2_ROW_B;        // one 32-channel slice of a 128-row operand (hi or lo), SWIZZLE_64B: 8 KB
 constexpr int BT_DK = 32;                       // head dim padded to the MMA's K = 16 granule (one 64-byte row)
 constexpr int BT_VT_B = 2 * BT_DK * ROW_B;      // one 64-key block of V^T: [32 rows of hi | 32 rows of lo][128 B]
@@ -83,9 +87,11 @@ struct BlockTailParams {
 };
 
 __device__ __forceinline__ void bt_sync() { asm volatile("bar.sync 1, %0;" ::"n"(32 * BT_WARPS) : "memory"); }
+// PAIR: the compute warps and the attention MMA warp, once per head (its q, k and v are drained)
+__device__ __forceinline__ void bt_sync_mma() { asm volatile("bar.sync 2, %0;" ::"n"(32 * BT_WARPS + 32) : "memory"); }
 
 template <int NKB, bool PAIR>   // C = 32 NKB channels; PAIR: two-CTA clusters over 256-row images
-__global__ void __launch_bounds__(BT_THREADS, 1)
+__global__ void __launch_bounds__(bt_threads(PAIR), 1)
 block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMap map_c1_hi,
                      const __grid_constant__ CUtensorMap map_c1_lo, const __grid_constant__ CUtensorMap map_wg_hi,
                      const __grid_constant__ CUtensorMap map_wg_lo, const __grid_constant__ CUtensorMap map_wi_hi,
@@ -97,12 +103,12 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
   constexpr int PITCH = C + 4;                  // x1 slab row pitch (floats): 16-byte shift per row, conflict-free chunks
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  __shared__ uint64_t bar_a, bar_full[2], bar_empty[2], bar_g, bar_i, bar_s, bar_o, bar_ag;
+  __shared__ uint64_t bar_a, bar_full[2], bar_empty[2], bar_g, bar_i, bar_s[PAIR ? 2 : 1], bar_o[PAIR ? 2 : 1], bar_ag;
+  __shared__ uint64_t bar_p[2];                 // PAIR: P of the S / P buffer written (one arrival per compute warp)
   __shared__ uint64_t bar_rfull, bar_pempty, bar_rfree;   // PAIR: remote buffer filled / peer's buffer free / ring stage free
   __shared__ uint32_t tmem_slot;
   __shared__ int failed_flag;
-  __shared__ float red[2][4][128];              // per-row partials of the four threads that share a row
-  __shared__ float own_ml[PAIR ? 2 : 1][128];   // PAIR: the own key block's row maximum and sum, per row
+  __shared__ float red[PAIR ? 3 : 2][4][128];   // per-row partials of the four threads that share a row
   volatile int* failed = &failed_flag;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -116,8 +122,11 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
     }
     mbar_init(&bar_g, 1);
     mbar_init(&bar_i, 1);
-    mbar_init(&bar_s, 1);
-    mbar_init(&bar_o, 1);
+    for (int s = 0; s < (PAIR ? 2 : 1); ++s) {
+      mbar_init(&bar_s[s], 1);
+      mbar_init(&bar_o[s], 1);
+      if (PAIR) mbar_init(&bar_p[s], BT_WARPS);
+    }
     mbar_init(&bar_ag, 1);
     mbar_init(&bar_rfull, 1);
     mbar_init(&bar_pempty, 1);
@@ -174,8 +183,64 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
         }
       }
     }
+  } else if (PAIR && warp == BT_WARPS + 1) {
+    // ===================== PAIR: phase 4's MMAs, per head over four 64-key blocks b (own 0-63, 64-127, peer's 0-63, 64-127)
+    // S_b = Q K_b^T -> S / P buffer b & 1 at [s_col + 64 (b & 1), + 64); O_b = P_b V_b -> [s_col + 128 + 32 (b & 1), + 32)
+    const uint32_t leader = elect_one();
+    const uint8_t* q_t = smem + p.qkv_off;
+    const uint8_t* k_t = q_t + 2 * BT_SLICE;
+    const uint8_t* v_t = q_t + 4 * BT_SLICE;
+    const uint8_t* rem = smem + p.rem_off;
+    const uint32_t sc_col = (uint32_t)p.s_col, o_col = sc_col + 128u;
+    const uint64_t dq_hi = make_smem_desc_sw64(smem_u32(q_t)), dq_lo = make_smem_desc_sw64(smem_u32(q_t + BT_SLICE));
+    auto issue_s = [&](int b) {
+      tc_fence_after();
+      const uint32_t idesc = make_idesc_f16(64), d = tmem + sc_col + (uint32_t)(64 * (b & 1));
+      const uint8_t* kt = (b < 2 ? k_t : rem) + (b & 1) * 64 * V2_ROW_B;   // 64 rows of the SWIZZLE_64B K pair: 4 KB
+      const uint64_t dk_hi = make_smem_desc_sw64(smem_u32(kt)), dk_lo = make_smem_desc_sw64(smem_u32(kt + BT_SLICE));
+#pragma unroll
+      for (int ks = 0; ks < BT_DK / 16; ++ks) {
+        const uint64_t ko = (uint64_t)(ks * 2);
+        umma_elect<true>(d, dq_hi + ko, dk_hi + ko, idesc, ks == 0 ? 0u : 1u, leader);
+        umma_elect<true>(d, dq_lo + ko, dk_hi + ko, idesc, 1u, leader);
+        umma_elect<true>(d, dq_hi + ko, dk_lo + ko, idesc, 1u, leader);
+      }
+      umma_commit_elect(&bar_s[b & 1], leader);
+    };
+#pragma unroll 1
+    for (int h = 0; h < p.heads; ++h) {
+      bt_sync_mma();                            // Q, K, V^T of head h are in shared memory
+      issue_s(0);
+      issue_s(1);
+#pragma unroll 1
+      for (int b = 0; b < 4; ++b) {
+        const int it = h * 4 + b;               // blocks done: buffer it & 1, phase (it >> 1) & 1 of bar_p / bar_o / bar_s
+        mbar_wait(&bar_p[b & 1], (uint32_t)((it >> 1) & 1), failed);   // P_b written, O buffer b & 1 drained
+        tc_fence_after();
+        // O_b = P_hi V_hi + P_lo V_hi + P_hi V_lo (N = 32, K = 64 keys)
+        const uint32_t idesc = make_idesc_f16(BT_DK), od = tmem + o_col + (uint32_t)(BT_DK * (b & 1));
+        const uint32_t pc = tmem + sc_col + (uint32_t)(64 * (b & 1));
+        const uint8_t* vb = b < 2 ? v_t + b * BT_VT_B : rem + 2 * BT_SLICE + (b - 2) * BT_VT_B;
+        const uint64_t dv_hi = make_smem_desc(smem_u32(vb)), dv_lo = make_smem_desc(smem_u32(vb + BT_DK * ROW_B));
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {           // 16 keys per step: 8 packed columns of P, 32 bytes of a V^T row
+          const uint64_t ko = (uint64_t)(j * 2);
+          umma_f16_ts_elect(od, pc + (uint32_t)(j * 8), dv_hi + ko, idesc, j == 0 ? 0u : 1u, leader);
+          umma_f16_ts_elect(od, pc + (uint32_t)(32 + j * 8), dv_hi + ko, idesc, 1u, leader);
+          umma_f16_ts_elect(od, pc + (uint32_t)(j * 8), dv_lo + ko, idesc, 1u, leader);
+        }
+        umma_commit_elect(&bar_o[b & 1], leader);
+        if (b < 2) {                            // S_{b+2} overwrites the P_b that this P V reads: wait for it to retire
+          mbar_wait(&bar_o[b & 1], (uint32_t)((it >> 1) & 1), failed);
+          if (b == 0) mbar_wait(&bar_rfull, (uint32_t)(h & 1), failed);   // the peer's K / V^T of head h have landed
+          issue_s(b + 2);
+        }
+      }
+      if (h == p.heads - 1) umma_commit_elect(&bar_rfree, leader);   // the remote buffer is read
+    }
   } else {
-    // ===================== compute warps: MMA issue (warp 0, elected lane), epilogues and softmax (all) ================
+    // ===================== compute warps: MMA issue (warp 0, elected lane; PAIR: phase 4's from the MMA warp above),
+    // epilogues and softmax (all)
     const uint32_t leader = warp == 0 ? elect_one() : 0u;
     const int lane_grp = warp & 3, quarter = warp >> 2;
     const int row = lane_grp * 32 + lane;       // TMEM lane = tile row
@@ -316,20 +381,18 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
     if (tracing) p.trace[3] = clock64();
 
     // ---- 4. attention, one head at a time ----------------------------------------------------------------------------------
-    {
+    if constexpr (!PAIR) {   // deep levels: one 128-key block per head, MMAs from warp 0
       uint8_t* q_t = smem + p.qkv_off;          // [hi | lo][128 rows][64 B], SWIZZLE_64B (over the dead in_proj operand)
       uint8_t* k_t = q_t + 2 * BT_SLICE;
       uint8_t* v_t = q_t + 4 * BT_SLICE;        // 2 blocks of 64 keys, SWIZZLE_128B
       const int D = p.D, chunks = D >> 3;
-      const uint32_t ip = (uint32_t)(2 * C), sc_col = (uint32_t)p.s_col, o_col = sc_col + 128u;  // PAIR: O_1 at o_col + 32
-      const int klo = PAIR ? 0 : row / p.HW * p.HW, khi = PAIR ? 128 : klo + p.HW;  // the keys of this row's image
+      const uint32_t ip = (uint32_t)(2 * C), sc_col = (uint32_t)p.s_col, o_col = sc_col + 128u;
+      const int klo = row / p.HW * p.HW, khi = klo + p.HW;  // the keys of this row's image
       const int k0 = quarter * 32;
       const bool live = k0 < khi && k0 + 32 > klo;          // warp-uniform: a warp's 32 rows meet the same quarters
-      uint8_t* rem = smem + p.rem_off;          // PAIR: the peer's K pair and V^T of the head, laid out as k_t, v_t
-      constexpr int NB = PAIR ? 2 : 1;          // key blocks per head: own keys, then (PAIR) the peer's
+      constexpr int NB = 1;                     // key blocks per head
 #pragma unroll 1
       for (int h = 0; h < p.heads; ++h) {
-        if (PAIR) mbar_wait(&bar_pempty, (uint32_t)(h & 1), failed);   // the peer is done with our previous head's copy
         // 4a. drain: thread (row, quarter) takes dims [8 quarter, 8 quarter + 8) of the head's k, v and q; dims >= D are zero
         {
           const uint32_t col = lane_addr + ip + (uint32_t)(h * D + quarter * 8);
@@ -375,11 +438,6 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
         fence_proxy_async();
         tc_fence_before();
         bt_sync();
-        if (PAIR && warp == 1 && lane == 0) {   // K pair and V^T (contiguous from k_t) -> the peer's remote buffer
-          mbar_expect_tx(&bar_rfull, (uint32_t)BT_REM_B);   // ... and the peer's into ours
-          const uint32_t peer = cluster_ctarank() ^ 1u;
-          bulk_copy_to_peer(mapa_rank(rem, peer), k_t, (uint32_t)BT_REM_B, mapa_rank(&bar_rfull, peer));
-        }
 
         // 4b. S = Q K^T into TMEM [s_col, s_col + 128) (warp 0; `kt` = the key block's K pair)
         auto issue_s = [&](const uint8_t* kt) {
@@ -394,14 +452,14 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
             umma_elect<true>(tmem + sc_col, dq_lo + ko, dk_hi + ko, idesc, 1u, leader);
             umma_elect<true>(tmem + sc_col, dq_hi + ko, dk_lo + ko, idesc, 1u, leader);
           }
-          umma_commit_elect(&bar_s, leader);
+          umma_commit_elect(&bar_s[0], leader);
         };
         if (warp == 0) issue_s(k_t);
         float mx = 0.f, l = 0.f;                // the last key block's row maximum and sum
 #pragma unroll 1
         for (int kb = 0; kb < NB; ++kb) {
           const int it = h * NB + kb;             // key blocks done: phase of bar_s / bar_o
-          mbar_wait(&bar_s, (uint32_t)(it & 1), failed);
+          mbar_wait(&bar_s[0], (uint32_t)(it & 1), failed);
           tc_fence_after();
           if (tracing && it == 0) p.trace[4] = clock64();
 
@@ -413,7 +471,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
               const int key = k0 + i;
-              if (!PAIR) s[i] = (key >= klo && key < khi) ? s[i] : -INFINITY;
+              s[i] = (key >= klo && key < khi) ? s[i] : -INFINITY;
               mx = fmaxf(mx, s[i]);
             }
           }
@@ -454,7 +512,7 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
           if (warp == 0) {
             tc_fence_after();
             const uint32_t idesc = make_idesc_f16(BT_DK), od = tmem + o_col + (uint32_t)(kb * BT_DK);
-            const uint8_t* vt = kb ? rem + 2 * BT_SLICE : v_t;
+            const uint8_t* vt = v_t;
 #pragma unroll
             for (int j = 0; j < 8; ++j) {         // 16 keys per step: 8 packed columns of P, 32 bytes of a V^T row
               const int key = j * 16;
@@ -466,52 +524,170 @@ block_tail_tc_kernel(const BlockTailParams p, const __grid_constant__ CUtensorMa
               umma_f16_ts_elect(od, a_lo, dv_hi, idesc, 1u, leader);
               umma_f16_ts_elect(od, a_hi, dv_lo, idesc, 1u, leader);
             }
-            umma_commit_elect(&bar_o, leader);
-            if (PAIR && kb == 0) {                // the peer's keys into the same S columns once P_0 has been read
-              mbar_wait(&bar_o, (uint32_t)(it & 1), failed);
-              mbar_wait(&bar_rfull, (uint32_t)(h & 1), failed);
-              issue_s(rem);
-            }
-            if (PAIR && kb == 1 && h == p.heads - 1) umma_commit_elect(&bar_rfree, leader);   // the remote buffer is read
-          }
-          if (PAIR && kb == 0 && quarter == 0) {  // read after the next block's barriers
-            own_ml[0][row] = mx;
-            own_ml[PAIR ? 1 : 0][row] = l;
+            umma_commit_elect(&bar_o[0], leader);
           }
         }
-        mbar_wait(&bar_o, (uint32_t)((h * NB + NB - 1) & 1), failed);
+        mbar_wait(&bar_o[0], (uint32_t)((h * NB + NB - 1) & 1), failed);
         tc_fence_after();
-        if (PAIR && h + 1 < p.heads && threadIdx.x == 0) mbar_arrive_cluster(mapa_rank(&bar_pempty, cluster_ctarank() ^ 1u));
 
-        // 4f. O / rowsum -> columns [h D, h D + D) of the attention gate's operand pair; PAIR: the exact combination of the
-        // two key blocks
-        float w0 = 1.0f / l, w1 = 0.f;
-        if (PAIR) {
-          const float m0 = own_ml[0][row], l0 = own_ml[PAIR ? 1 : 0][row], m = fmaxf(m0, mx);
-          w0 = ex2_fast(m0 - m);
-          w1 = ex2_fast(mx - m);
-          const float inv = 1.0f / (l0 * w0 + l * w1);
-          w0 *= inv;
-          w1 *= inv;
-        }
+        // 4f. O / rowsum -> columns [h D, h D + D) of the attention gate's operand pair
+        const float w0 = 1.0f / l;
         if (quarter < chunks) {
           float o[8];
           tmem_ld8(lane_addr + o_col + (uint32_t)(quarter * 8), o);
-          if (PAIR) {
-            float o1[8];
-            tmem_ld8(lane_addr + o_col + (uint32_t)(BT_DK + quarter * 8), o1);
 #pragma unroll
-            for (int e = 0; e < 8; ++e) o[e] = o[e] * w0 + o1[e] * w1;
-          } else {
-#pragma unroll
-            for (int e = 0; e < 8; ++e) o[e] *= w0;
-          }
+          for (int e = 0; e < 8; ++e) o[e] *= w0;
           uint4 hi, lo;
           cvt8(o, hi, lo);
           const int c = h * D + quarter * 8, kb = c >> 5, ch = (c & 31) >> 3;
           *reinterpret_cast<uint4*>(r2 + kb * 2 * BT_SLICE + sw64_off(row, ch)) = hi;
           *reinterpret_cast<uint4*>(r2 + kb * 2 * BT_SLICE + BT_SLICE + sw64_off(row, ch)) = lo;
         }
+        // (the next head's drain barrier orders these TMEM loads before its MMAs overwrite S and O)
+      }
+    } else {                 // PAIR: four 64-key blocks per head, MMAs from the MMA warp
+      uint8_t* q_t = smem + p.qkv_off;          // [hi | lo][128 rows][64 B], SWIZZLE_64B (over the dead in_proj operand)
+      uint8_t* k_t = q_t + 2 * BT_SLICE;
+      uint8_t* v_t = q_t + 4 * BT_SLICE;        // 2 blocks of 64 keys, SWIZZLE_128B
+      const int D = p.D, chunks = D >> 3;
+      const uint32_t ip = (uint32_t)(2 * C), sc_col = (uint32_t)p.s_col, o_col = sc_col + 128u;
+
+      // 4a. drain: thread (row, quarter) takes dims [8 quarter, 8 quarter + 8) of the head's k, v and q; dims >= D are zero
+      auto drain = [&](int h) {
+        const uint32_t col = lane_addr + ip + (uint32_t)(h * D + quarter * 8);
+        float v[8];
+        uint4 hi, lo;
+        const bool has = quarter < chunks;
+        if (has) {
+          tmem_ld8(col, v);
+#pragma unroll
+          for (int e = 0; e < 8; ++e) v[e] *= p.sc_i;
+        } else {
+#pragma unroll
+          for (int e = 0; e < 8; ++e) v[e] = 0.f;
+        }
+        cvt8(v, hi, lo);
+        *reinterpret_cast<uint4*>(k_t + sw64_off(row, quarter)) = hi;
+        *reinterpret_cast<uint4*>(k_t + BT_SLICE + sw64_off(row, quarter)) = lo;
+        if (has) {
+          tmem_ld8(col + 2 * C, v);
+#pragma unroll
+          for (int e = 0; e < 8; ++e) v[e] = v[e] * p.sc_i * p.qscale;
+        }
+        cvt8(v, hi, lo);
+        *reinterpret_cast<uint4*>(q_t + sw64_off(row, quarter)) = hi;
+        *reinterpret_cast<uint4*>(q_t + BT_SLICE + sw64_off(row, quarter)) = lo;
+        if (has) {
+          tmem_ld8(col + C, v);
+#pragma unroll
+          for (int e = 0; e < 8; ++e) v[e] *= p.sc_i;
+        }
+        // V^T: rows = head dims, contraction (keys) along the 128-byte rows; hi rows then lo rows per 64-key block
+        uint8_t* blk = v_t + (row >> 6) * BT_VT_B;
+        const int kk = row & 63;
+#pragma unroll
+        for (int e = 0; e < 8; ++e) {
+          const int dim = quarter * 8 + e;
+          unsigned short hh, ll;
+          split_f16(v[e], hh, ll);
+          *reinterpret_cast<unsigned short*>(blk + sw_off(dim, kk >> 3) + ((kk & 7) << 1)) = hh;
+          *reinterpret_cast<unsigned short*>(blk + sw_off(BT_DK + dim, kk >> 3) + ((kk & 7) << 1)) = ll;
+        }
+        fence_proxy_async();
+        tc_fence_before();
+      };
+      // 4f. O / rowsum -> columns [h D, h D + D) of the attention gate's operand pair
+      auto store_o = [&](int h, const float (&o)[8], float w) {
+        float t[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) t[e] = o[e] * w;
+        uint4 hi, lo;
+        cvt8(t, hi, lo);
+        const int c = h * D + quarter * 8, kb = c >> 5, ch = (c & 31) >> 3;
+        *reinterpret_cast<uint4*>(r2 + kb * 2 * BT_SLICE + sw64_off(row, ch)) = hi;
+        *reinterpret_cast<uint4*>(r2 + kb * 2 * BT_SLICE + BT_SLICE + sw64_off(row, ch)) = lo;
+      };
+
+      // Per head, four 64-key blocks b: own keys 0-63, 64-127, then the peer's 0-63, 64-127 from the remote buffer.  The
+      // MMA warp keeps two S / P buffers in flight, so the softmax of block b runs while the tensor pipe does P_{b-1} V
+      // and S_{b+1}.  A thread owns 16 keys of a row per block.  Each block has its own row maximum m_b; the thread
+      // folds O_b into registers as it retires, m = max(m, m_b), o = o 2^(m_old - m) + O_b 2^(m_b - m), and likewise
+      // its share of the row sum (the exact split-key combination, applied block by block).
+      uint8_t* rem = smem + p.rem_off;        // the peer's K pair and V^T of the head, laid out as k_t, v_t
+#pragma unroll 1
+      for (int h = 0; h < p.heads; ++h) {
+        mbar_wait(&bar_pempty, (uint32_t)(h & 1), failed);   // the peer is done with our previous head's copy
+        drain(h);
+        bt_sync_mma();
+        if (warp == 1 && lane == 0) {         // K pair and V^T (contiguous from k_t) -> the peer's remote buffer
+          mbar_expect_tx(&bar_rfull, (uint32_t)BT_REM_B);   // ... and the peer's into ours
+          const uint32_t peer = cluster_ctarank() ^ 1u;
+          bulk_copy_to_peer(mapa_rank(rem, peer), k_t, (uint32_t)BT_REM_B, mapa_rank(&bar_rfull, peer));
+        }
+        float m = -INFINITY, l = 0.f, o[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        // fold O_b (its P V committed on bar_o[b & 1]) with block maximum mb and this thread's block sum lb
+        auto fold = [&](int b, float mb, float lb) {
+          const int it = h * 4 + b;
+          mbar_wait(&bar_o[b & 1], (uint32_t)((it >> 1) & 1), failed);
+          tc_fence_after();
+          const float mn = fmaxf(m, mb), a = ex2_fast(m - mn), c = ex2_fast(mb - mn);
+          l = l * a + lb * c;
+          m = mn;
+          if (quarter < chunks) {
+            float ob[8];
+            tmem_ld8(lane_addr + o_col + (uint32_t)(BT_DK * (b & 1) + quarter * 8), ob);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) o[e] = o[e] * a + ob[e] * c;
+          }
+        };
+        float mp = 0.f, lp = 0.f;             // the previous block's maximum and sum, folded one block later
+#pragma unroll 1
+        for (int b = 0; b < 4; ++b) {
+          const int it = h * 4 + b;
+          const uint32_t sb = lane_addr + sc_col + (uint32_t)(64 * (b & 1));
+          mbar_wait(&bar_s[b & 1], (uint32_t)((it >> 1) & 1), failed);
+          tc_fence_after();
+          if (tracing && it == 0) p.trace[4] = clock64();
+          float s[16];
+          tmem_ld16(sb + (uint32_t)(quarter * 16), s);
+          float mb = s[0];
+#pragma unroll
+          for (int i = 1; i < 16; ++i) mb = fmaxf(mb, s[i]);
+          red[b & 1][quarter][row] = mb;
+          tc_fence_before();                  // every load of S_b is complete before anyone writes P_b over it
+          bt_sync();
+          tc_fence_after();
+          mb = fmaxf(fmaxf(red[b & 1][0][row], red[b & 1][1][row]), fmaxf(red[b & 1][2][row], red[b & 1][3][row]));
+          // p = 2^(s - m_b) as packed fp16 (hi, lo): keys (2i, 2i + 1) of the block in column i of each 32-column half
+          uint32_t ph[8], pl[8];
+          float lb = 0.f;
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            const float e0 = ex2_fast(s[2 * i] - mb), e1 = ex2_fast(s[2 * i + 1] - mb);
+            lb += e0 + e1;
+            ph[i] = pack_h2(e0, e1);
+            float a0, a1;
+            unpack_h2(ph[i], a0, a1);
+            pl[i] = pack_h2(e0 - a0, e1 - a1);
+          }
+          tmem_st8u(sb + (uint32_t)(quarter * 8), ph);
+          tmem_st8u(sb + (uint32_t)(32 + quarter * 8), pl);
+          asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+          tc_fence_before();
+          __syncwarp();
+          if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&bar_p[b & 1])) : "memory");
+          // O_{b-1} is drained before this warp's next arrival lets P_{b+1} V overwrite its buffer
+          if (b > 0) fold(b - 1, mp, lp);
+          mp = mb;
+          lp = lb;
+        }
+        fold(3, mp, lp);
+        // P_3 V has retired, and with it every MMA of the head that read the remote buffer
+        if (h + 1 < p.heads && threadIdx.x == 0) mbar_arrive_cluster(mapa_rank(&bar_pempty, cluster_ctarank() ^ 1u));
+        red[2][quarter][row] = l;
+        bt_sync();
+        l = (red[2][0][row] + red[2][1][row]) + (red[2][2][row] + red[2][3][row]);
+        if (quarter < chunks) store_o(h, o, 1.0f / l);
         // (the next head's drain barrier orders these TMEM loads before its MMAs overwrite S and O)
       }
     }
@@ -625,7 +801,7 @@ int block_tail_launch(const BlockTailParams& p, int tiles, size_t smem, const CU
                                        (int)smem));
     smem_set = smem;
   }
-  FLOWK_CUDA_OK(launch_pdl_cluster(block_tail_tc_kernel<NKB, PAIR>, dim3(tiles), dim3(BT_THREADS), smem, stream,
+  FLOWK_CUDA_OK(launch_pdl_cluster(block_tail_tc_kernel<NKB, PAIR>, dim3(tiles), dim3(bt_threads(PAIR)), smem, stream,
                                    PAIR ? 2 : 1, p, maps[0], maps[1], maps[2], maps[3], maps[4], maps[5], maps[6], maps[7]));
   return launch_status();
 }
