@@ -84,6 +84,8 @@ SIGNATURES = {
     "flowk_attention_train_fwd": ([_fp, _fp, _fp, _fp, ctypes.c_uint, ctypes.c_float, _i, _i, _i, _i, _st], _i),
     "flowk_attention_train_bwd": ([_i, _fp, _fp, _fp, _fp, _fp, _fp, ctypes.c_uint, ctypes.c_float, _i, _i, _i, _i, _st], _i),
     "flowk_attention_dropout_mask": ([_fp, ctypes.c_uint, ctypes.c_float, _i, _i, _fp, _st], _i),
+    "flowk_attention_train_tc_fwd": ([_fp, _fp, _fp, _fp, ctypes.c_uint, ctypes.c_float, _i, _i, _i, _i, _st], _i),
+    "flowk_attention_train_tc_bwd": ([_i, _fp, _fp, _fp, _fp, _fp, _fp, ctypes.c_uint, ctypes.c_float, _i, _i, _i, _i, _st], _i),
     "flowk_adamax_step": ([_fp, _i, _fp, ctypes.c_float, ctypes.c_float, ctypes.c_float, _st], _i),
     "flowk_glu_bwd": ([_fp, _fp, _fp, ctypes.c_longlong, _i, ctypes.c_longlong, _st], _i),
     "flowk_mar_step": ([ctypes.c_void_p, _st], _i),

@@ -9,6 +9,7 @@
 // intermediate (each computes delta itself), so they may run concurrently on two streams.
 // Rows of qkv [M, 3C] are (k | v | q) (:136-139); dqkv has the same layout.
 #include "common.cuh"
+#include "attention_dropout.cuh"
 
 namespace flowk {
 namespace attn_train {
@@ -28,19 +29,6 @@ __device__ __forceinline__ void mma3(float (&c)[4], const uint32_t (&ah)[4], con
   mma_tf32(c, ah, bh0, bh1);
   mma_tf32(c, al, bh0, bh1);
   mma_tf32(c, ah, bl0, bl1);
-}
-
-// dropout multiplier of attention weight (query q, key k) of pair `pair`: 0 with probability thresh / 2^32, else 1/(1-p)
-__device__ __forceinline__ float drop_scale(uint32_t seed, uint32_t pair, uint32_t q, uint32_t k, uint32_t S, uint32_t thresh,
-                                            float inv_keep) {
-  uint32_t x = ((pair * S + q) * S + k) ^ seed;
-  x *= 0x9E3779B1u; x ^= x >> 16;
-  x *= 0x85EBCA6Bu; x ^= x >> 13;
-  x *= 0xC2B2AE35u; x ^= x >> 16;
-  return x >= thresh ? inv_keep : 0.f;
-}
-__device__ __forceinline__ uint32_t layer_seed(const unsigned* seed_dev, unsigned salt) {
-  return (seed_dev ? *seed_dev : 0u) * 0x01000193u ^ (salt * 0x9E3779B9u + 0x7F4A7C15u);
 }
 
 // stage `tile_rows` rows of D floats (row j at src + j*row_stride, rows >= `rows` are zero) as (hi, lo), pitch D + 4
@@ -412,6 +400,7 @@ extern "C" int flowk_attention_train_fwd(const float* qkv, float* out, float* ls
     case 24: return run_fwd<24>(qkv, out, lse, seed_device, salt, p_drop, B, HW, C, heads, stream);
     case 32: return run_fwd<32>(qkv, out, lse, seed_device, salt, p_drop, B, HW, C, heads, stream);
     case 40: return run_fwd<40>(qkv, out, lse, seed_device, salt, p_drop, B, HW, C, heads, stream);
+    case 64: return run_fwd<64>(qkv, out, lse, seed_device, salt, p_drop, B, HW, C, heads, stream);
     default: return FLOWK_ERR_SHAPE;
   }
 }
@@ -430,6 +419,7 @@ extern "C" int flowk_attention_train_bwd(int which, const float* qkv, const floa
     case 24: return run_bwd<24>(which, qkv, out, dout, lse, dqkv, seed_device, salt, p_drop, B, HW, C, heads, stream);
     case 32: return run_bwd<32>(which, qkv, out, dout, lse, dqkv, seed_device, salt, p_drop, B, HW, C, heads, stream);
     case 40: return run_bwd<40>(which, qkv, out, dout, lse, dqkv, seed_device, salt, p_drop, B, HW, C, heads, stream);
+    case 64: return run_bwd<64>(which, qkv, out, dout, lse, dqkv, seed_device, salt, p_drop, B, HW, C, heads, stream);
     default: return FLOWK_ERR_SHAPE;
   }
 }

@@ -623,7 +623,7 @@ def attention_train_supported(qkv, heads):
         return False
     b, s, c3 = qkv.shape
     c = c3 // 3
-    return c3 % 3 == 0 and c % heads == 0 and c // heads in (8, 16, 24, 32, 40) and s % 8 == 0 and \
+    return c3 % 3 == 0 and c % heads == 0 and c // heads in (8, 16, 24, 32, 40, 64) and s % 8 == 0 and \
         b * heads * s * s < 2 ** 32 - 1
 
 
@@ -632,6 +632,12 @@ def attention_train_supported(qkv, heads):
 ATTENTION_BWD_FORK = __import__("os").environ.get("FLOWK_ATTN_FORK", "0") == "1"
 FOLD_DROPOUT = __import__("os").environ.get("FLOWK_FOLD_DROPOUT", "1") != "0"   # Dropout2d folded into concat_elu
 ATTENTION_TC = True      # training attention core (softmax(q k^T) v with dropout, forward + backward) on the flowk kernels
+
+
+def _attention_train_entry(seq, head_dim):
+    """Head dim 64 at 128 / 256 tokens runs on the tcgen05 kernels (csrc/attention_train_tc.cu); every other admitted shape,
+    head dim 64 at the shorter sequences of the deep levels included, on the mma.sync kernels (csrc/attention_train.cu)."""
+    return "flowk_attention_train_tc" if head_dim == 64 and seq in (128, 256) else "flowk_attention_train"
 
 
 class _AttentionCore(torch.autograd.Function):
@@ -645,8 +651,8 @@ class _AttentionCore(torch.autograd.Function):
         out = torch.empty(b, s, c, device=qkv.device, dtype=torch.float32)
         lse = torch.empty(b * heads, s, device=qkv.device, dtype=torch.float32)
         seed = dropout_seed(qkv.device)
-        _lib.call("flowk_attention_train_fwd", qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), seed.data_ptr(), salt,
-                  float(p_drop), b, s, c, heads, tc._stream())
+        _lib.call(_attention_train_entry(s, c // heads) + "_fwd", qkv.data_ptr(), out.data_ptr(), lse.data_ptr(),
+                  seed.data_ptr(), salt, float(p_drop), b, s, c, heads, tc._stream())
         ctx.save_for_backward(qkv, out, lse)
         ctx.cfg = (heads, float(p_drop), salt)
         return out
@@ -661,11 +667,12 @@ class _AttentionCore(torch.autograd.Function):
         seed = dropout_seed(qkv.device)
         args = (qkv.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(), dqkv.data_ptr(), seed.data_ptr(), salt, p_drop,
                 b, s, c3 // 3, heads)
+        bwd = _attention_train_entry(s, c3 // 3 // heads) + "_bwd"
         fork = _fork_wgrad(qkv.device)
         fork.on = fork.on and ATTENTION_BWD_FORK
         with fork:                                  # side stream: key side (dk, dv columns)
-            _lib.call("flowk_attention_train_bwd", 2, *args, tc._stream())
-        _lib.call("flowk_attention_train_bwd", 1, *args, tc._stream())       # main stream: query side (dq columns)
+            _lib.call(bwd, 2, *args, tc._stream())
+        _lib.call(bwd, 1, *args, tc._stream())       # main stream: query side (dq columns)
         fork.join()
         return dqkv, None, None, None
 

@@ -389,7 +389,7 @@ int flowk_weight_norm_bwd_partials(const float* v, const float* g, const float* 
  * (writes the q columns of dqkv), 2 = key side (k and v columns), 3 = both; 1 and 2 may run on different streams.  The dropout mask is a counter-based hash of
  * (*seed_device, salt, image*head, query, key): the backward regenerates it, nothing of size HW x HW touches HBM.
  * seed_device: device scalar the caller advances once per training step (so a captured graph draws fresh masks on each
- * replay); salt: per-layer constant.  HW % 8 == 0, C / heads in {8, 16, 24, 32, 40}, B*heads*HW*HW < 2^32.
+ * replay); salt: per-layer constant.  HW % 8 == 0, C / heads in {8, 16, 24, 32, 40, 64}, B*heads*HW*HW < 2^32.
  * flowk_attention_dropout_mask materialises the multipliers (0 or 1/(1-p)) [B*heads, HW, HW] - for tests. */
 int flowk_attention_train_fwd(const float* qkv, float* out, float* lse, const unsigned* seed_device, unsigned salt,
                               float p_drop, int B, int HW, int C, int heads, flowk_stream_t stream);
@@ -398,6 +398,18 @@ int flowk_attention_train_bwd(int which, const float* qkv, const float* out, con
                               int heads, flowk_stream_t stream);
 int flowk_attention_dropout_mask(const unsigned* seed_device, unsigned salt, float p_drop, int pairs, int HW, float* mask,
                                  flowk_stream_t stream);
+
+/* The same training attention core (reference flow_modules/mixlogcdf_nn.py:139-147: q k^T / sqrt(d), softmax, dropout,
+ * weight v) on tcgen05 (csrc/attention_train_tc.cu) for head dim C / heads == 64 and HW in {128, 256}: kind::tf32 MMAs on
+ * (hi, lo) operand pairs (fp32 accuracy), TMEM accumulators, the dropout mask of flowk_attention_dropout_mask.  Same
+ * arguments, layouts, lse and `which` as flowk_attention_train_fwd / _bwd; the two backward kernels use no atomics, so
+ * results are bit-identical from call to call.  FLOWK_ERR_ARG on a NULL pointer or `which` outside 1..3; FLOWK_ERR_SHAPE
+ * for C / heads != 64, HW not in {128, 256}, p_drop outside [0, 1) or B*heads*HW*HW >= 2^32 - 1. */
+int flowk_attention_train_tc_fwd(const float* qkv, float* out, float* lse, const unsigned* seed_device, unsigned salt,
+                                 float p_drop, int B, int HW, int C, int heads, flowk_stream_t stream);
+int flowk_attention_train_tc_bwd(int which, const float* qkv, const float* out, const float* dout, const float* lse,
+                                 float* dqkv, const unsigned* seed_device, unsigned salt, float p_drop, int B, int HW, int C,
+                                 int heads, flowk_stream_t stream);
 
 /* Adamax step (torch.optim.Adamax semantics, weight_decay = 0; the reference's optimizer, marscf_main.py:302) over every
  * parameter tensor of a model in one launch / one HBM pass.  `chunks_device`: DEVICE array, each tensor cut into pieces
