@@ -54,6 +54,7 @@ SIGNATURES = {
     "flowk_patch_attention_bwd": ([_fp] * 8 + [_i] * 5 + [_st], _i),
     "flowk_attention_tc": ([_fp, _fp, _fp, _i, _i, _i, _i, _i, _fp, _fp, _st], _i),
     "flowk_attention_tc_v2": ([_fp, _fp, _fp, _i, _i, _i, _i, _i, _fp, _fp, _st], _i),
+    "flowk_attention_long_tc": ([_fp, _fp, _fp, _i, _i, _i, _i, _i, _fp, _fp, _st], _i),
     "flowk_attention_tc_v2_occupancy": ([_i, _i, _i, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)], _i),
     "flowk_attention_inproj_tc": ([_fp, _fp, _fp, _fp, _f, _fp, _fp, _i, _i, _i, _i, _fp, _fp, _st], _i),
     "flowk_attention_inproj_tc_occupancy": ([_i, _i, _i, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)], _i),
@@ -145,6 +146,7 @@ DIMS = {
     "flowk_nchw_to_nhwc_hilo": slice(2, 6), "flowk_split_hilo": slice(3, 4), "flowk_attention": slice(3, 7),
     "flowk_nchw_to_nhwc_hilo_f16": slice(2, 6), "flowk_split_hilo_f16": slice(3, 4), "flowk_attention_f16": slice(3, 7),
     "flowk_attention_tc": slice(4, 8), "flowk_attention_tc_v2": slice(4, 8), "flowk_attention_inproj_tc": slice(7, 11),
+    "flowk_attention_long_tc": slice(4, 8),
     "flowk_block_tail_tc": slice(23, 27), "flowk_block_tail_pair_tc": slice(23, 27),
     "flowk_patch_attention": slice(6, 10),
     "flowk_patch_attention_train_fwd": slice(7, 11), "flowk_patch_attention_bwd": slice(8, 12),

@@ -186,9 +186,22 @@ def attention(qkv, B, HW, C, heads, f16=False, status=None, trace=None):
         _lib.call("flowk_attention_tc", qkv.data_ptr(), hi.data_ptr(), lo.data_ptr(), int(f16), B, HW, C, heads,
                   _p(status), _p(trace), _stream())
         return hi, lo
+    if not _attention_mma_supported(HW, C, heads) and attention_long_tc_supported(HW, C, heads):
+        _lib.call("flowk_attention_long_tc", qkv.data_ptr(), hi.data_ptr(), lo.data_ptr(), int(f16), B, HW, C, heads,
+                  _p(status), _p(trace), _stream())
+        return hi, lo
     _lib.call("flowk_attention_f16" if f16 else "flowk_attention", qkv.data_ptr(), hi.data_ptr(), lo.data_ptr(), B, HW, C,
               heads, _stream())
     return hi, lo
+
+
+def attention_long_tc_supported(HW, C, heads):
+    """Shapes the long-sequence tcgen05 attention kernel (csrc/attention_long_tc.cu) takes: seq a multiple of 128 and at least
+    512, head dim 24, 32, 40 or 64.  `attention` sends it only the shapes no other kernel takes (d > 24 at 1024 tokens: the
+    level-1 maps of 64x64 images at widths 128, 160 and 256); the shapes the mma.sync kernel runs keep it."""
+    if not (heads >= 1 and C % heads == 0):
+        return False
+    return HW >= 512 and HW % 128 == 0 and C // heads in (24, 32, 40, 64)
 
 
 # q, k, v computed inside the one-wave kernel from the gate GEMM's normalised rows (flowk_attention_inproj_tc) instead of
@@ -218,11 +231,15 @@ def attention_inproj(p_hi, p_lo, w_hi, w_lo, acc_scale, B, HW, C, heads, status=
     return hi, lo
 
 
-def attention_supported(HW, C, heads):
-    if attention_tc_supported(HW, C, heads):
-        return True
+def _attention_mma_supported(HW, C, heads):
+    """Shapes the mma.sync attention kernel (csrc/attention.cu) takes within its shared-memory budget."""
     return C % heads == 0 and (C // heads) in (8, 16, 24, 32, 40, 64) and (HW <= 256 or HW % 256 == 0) and HW % 4 == 0 \
         and 2 * min(HW, 1 << 30) * (C // heads) * 4 * max(1, 256 // max(HW, 1)) <= 220 * 1024
+
+
+def attention_supported(HW, C, heads):
+    return (attention_tc_supported(HW, C, heads) or _attention_mma_supported(HW, C, heads)
+            or attention_long_tc_supported(HW, C, heads))
 
 
 def chain_supported(C, n2, f16=False):

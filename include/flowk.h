@@ -474,6 +474,15 @@ int flowk_attention_tc(const float* qkv, void* out_hi, void* out_lo, int out_f16
 int flowk_attention_tc_v2(const float* qkv, void* out_hi, void* out_lo, int out_f16, int B, int HW, int C, int heads,
                           int* status, long long* trace, flowk_stream_t stream);
 int flowk_attention_tc_v2_occupancy(int HW, int C, int heads, int* blocks_per_sm, int* smem_bytes);
+/* The tcgen05 attention core for long sequences (csrc/attention_long_tc.cu): one CTA per (image, head, 128-query tile), keys
+ * streamed through shared memory in 128-key blocks, per-block softmax folded into a running output (online softmax), P kept
+ * in tensor memory; nothing of size HW x HW leaves the SM.  Same arguments and outputs as flowk_attention_tc.  Takes HW a
+ * multiple of 128 with HW >= 512 and C/heads in {24, 32, 40, 64}, any B >= 0 (B = 0: FLOWK_OK, no launch);
+ * FLOWK_ERR_SHAPE otherwise, FLOWK_ERR_ARG for a NULL qkv / out_hi / out_lo.  `status` as for flowk_attention_tc;
+ * `trace` (device long long[3], NULL in production): clock64 stamps of CTA 0 at start, after the key loop and at the end.
+ * Deterministic: no atomics, key blocks folded in order. */
+int flowk_attention_long_tc(const float* qkv, void* out_hi, void* out_lo, int out_f16, int B, int HW, int C, int heads,
+                            int* status, long long* trace, flowk_stream_t stream);
 /* The one-wave kernel with the in_proj GEMM fused in front: instead of the fp32 in_proj rows it takes the rows that GEMM
  * would multiply, p_hi / p_lo [B*HW, C] fp16 (the normalised rows + positional encoding, as flowk_conv_gemm's
  * OUT_HILO_POS writes them), and the in_proj weight operand w_hi / w_lo [3C, ceil64(C)] fp16 with (k | v | q) rows as
